@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the squigly-trace B200 backend (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload config1..config5] [--spp S] [--no-cpu-baseline] [--no-other-configs]
+                    [--workload config1..config5] [--spp S] [--no-cpu-baseline] [--no-other-configs] [--dump-outputs DIR]
 
 Default workload (BASELINE.json configs[1]): data/scene.obj + scene.sq + camera at 1920x1080, 1024 spp, max 8 bounces.
 A step = one full render of that frame through the hot path.  Metric = Mrays/s, where a ray is one closest-hit
@@ -17,6 +17,12 @@ at surfaces with surfColor = 0; both are exact (bit-identical image), and only e
       rays/sample, a 40 k-ray bit-exact spot check against the oracle, and a roofline on its binding resource
   intersect_batch (1 GPU only): the batched Scene.intersect entry point on 8 M incoherent rays and a 1080p pinhole fan
   frame_sha256 / per_rank : identity of rank 0's RGB8 frame and every rank's phase times (outside the timed region)
+
+`--dump-outputs DIR` writes the frame of the last timed step as a caller of the timed path receives it (sqt_download_image):
+DIR/accum.npy (per-pixel radiance sums) and DIR/rgb8.npy (the tone-mapped frame), both float32 of shape (rows, cols, 3).
+When the two together would exceed 64 MB, the same seeded sample of pixels is taken from both, (n, 3) each, and its
+row-major pixel indices go to DIR/pixel_index.npy (float64).  Inputs are fixed by the arguments (seeded scenes, SEED), so
+two builds of the project can be compared output for output.
 
 `--impl reference` times that oracle alone (the Haskell reference cannot be built: no GHC in the image).
 Multi-GPU: launched by torchrun, one rank per GPU; pixel groups are partitioned over ranks and the accumulation
@@ -39,6 +45,7 @@ for p in (ROOT, PKG):
 
 SEED = 0
 DATA = os.path.join(ROOT, "data")
+DUMP_BYTES = 64_000_000
 KERNEL_VERSION = "r02-v17"         # key into profiles/r02_traffic.json (ncu DRAM bytes per k_paths_pool launch)
 
 
@@ -105,6 +112,22 @@ def _traffic():
         return t.get(KERNEL_VERSION)
     except Exception:
         return None
+
+
+def dump_outputs(directory, arrays):
+    """arrays: name -> (rows, cols, 3) frame.  Saved as float32, whole or as one seeded pixel sample (see the module docstring)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    out = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    npix = out["rgb8"].shape[0] * out["rgb8"].shape[1]
+    per_pixel = 3 * 4 * len(out)
+    if npix * per_pixel > DUMP_BYTES:
+        n = (DUMP_BYTES - 4096) // (per_pixel + 8)
+        idx = np.sort(np.random.default_rng(SEED).choice(npix, n, replace=False))
+        out = {k: v.reshape(npix, 3)[idx] for k, v in out.items()}
+        out["pixel_index"] = idx.astype(np.float64)
+    for k, v in out.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
 
 
 def workload_cfg(name):
@@ -388,8 +411,10 @@ def run_ours(args, rank, world, local_rank):
     # identity of the frame and where every rank spent its time (outside the timed region)
     frame_sha = None
     if rank == 0:
-        rgb8, _ = ctx.download(p.rows, p.cols, want_accum=False)
+        rgb8, accum = ctx.download(p.rows, p.cols, want_accum=bool(args.dump_outputs))
         frame_sha = hashlib.sha256(rgb8.tobytes()).hexdigest()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"accum": accum, "rgb8": rgb8})
     per_rank = [dict(rank=rank, **{k: round(v, 3) for k, v in phase.items()})]
     if dist is not None:
         gathered = [None] * world
@@ -500,7 +525,13 @@ def main():
     ap.add_argument("--spp", type=int, default=0, help="override the workload's samples per pixel (a reduced run; stated in config.spp)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step to DIR as .npy files (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm sizes its sample by timing)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -512,7 +543,8 @@ def main():
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(args.gpus), "--master-addr",
                "127.0.0.1", "--master-port", "29517", os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps),
                "--warmup", str(args.warmup), "--workload", args.workload, "--spp", str(args.spp)] \
-            + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + (["--no-other-configs"] if args.no_other_configs else [])
+            + (["--no-cpu-baseline"] if args.no_cpu_baseline else []) + (["--no-other-configs"] if args.no_other_configs else []) \
+            + (["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
         raise SystemExit(subprocess.call(cmd))
     run_ours(args, rank, world, local_rank)
 
