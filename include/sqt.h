@@ -190,6 +190,40 @@ int sqt_comm_init_all(sqt_ctx **ctxs, int n);
 int sqt_render_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const sqt_render_params *params,
                      uint8_t *rgb8_out, float *accum_out, sqt_stats *stats_or_null);
 
+/* progressive frames: one sqt_render_params job (the target spp and everything else) advanced in chunks of samples per
+ * pixel, so that a host can show previews, bound the time a frame takes and stop once the image is good enough ---------
+ *
+ * Seeds stay keyed to the target spp: sample k of pixel (y, x) uses generator seed spp*(x + y*seed_stride) + k as in
+ * sqt_render.  After k < spp samples the image is the k-sample PREFIX of the spp frame, not an spp = k render.
+ *
+ * sqt_render_begin     does the checks and the pre-pass of sqt_render, makes every allocation the frame needs, zero-fills
+ *                      and traces the primary hits -- no paths.  Stats: what that cost.  Cast mode (mode 1) and
+ *                      SQT_F_SPLIT_SAMPLES are SQT_E_UNSUPPORTED.
+ * sqt_render_advance   traces samples [k, min(k + n_samples, spp)), then reduces (groups), tone-maps the preview
+ *                      (rgbFloatToPixelRGB of sum * (1.0f/(float)k)) and computes the noise estimate; it allocates
+ *                      nothing.  n_samples < 1 is SQT_E_INVALID; at k = spp it returns SQT_OK and launches nothing.
+ *                      Summed over begin and every advance, the stats' rays / samples / counters equal sqt_render's.
+ * After all spp samples, with any chunking, the sums and RGB8 equal sqt_render's for the same job bit for bit.
+ * Every progressive frame also keeps the per-pixel second moment s2 = s2 + x*x over the sample radiances x (binary32,
+ * sample order, from +0); sqt_download_moments reads it, sqt_download_image reads the sums and the preview (both
+ * SQT_E_INVALID before the first advance / outside a frame).
+ * noise (rank 0; NaN on other ranks), fp64 over all N = rows*cols*3 values after n = k samples:
+ *   mu = s1/n, var = max(0, (s2 - s1*mu)/(n-1)), e2 = var/n, noise = sqrt(sum(e2)/N) / (sum(mu)/N);
+ *   0 when sum(mu) = 0, +inf when k < 2.  The reduction order is fixed: the same buffers give the same bits.
+ * A frame ends with sqt_render[_resident|_group], sqt_tone_map, sqt_upload_scene[_group], sqt_upload_spheres or a new
+ * begin; sqt_render_advance then returns SQT_E_INVALID.  sqt_intersect_batch does not end a frame.
+ * In a group every rank must make the same calls: ranks that disagree on k, the target spp or the chunk fail on every
+ * rank before anything is traced. */
+typedef struct sqt_progress {
+    int32_t samples_done, samples_total;
+    double noise;
+} sqt_progress;                          /* 16 B */
+int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *params, sqt_stats *stats_or_null);
+int sqt_render_advance(sqt_ctx *ctx, int32_t n_samples, sqt_progress *progress_or_null, sqt_stats *stats_or_null);
+int sqt_render_begin_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const sqt_render_params *params, sqt_stats *stats_or_null);
+int sqt_render_advance_group(sqt_ctx **ctxs, int n, int32_t n_samples, sqt_progress *progress_or_null, sqt_stats *stats_or_null);
+int sqt_download_moments(sqt_ctx *ctx, float *m2_out);   /* rows*cols*3 floats: s2 of the frame in progress (rank 0) */
+
 /* measured roofline denominators on this device (microbenchmarks; see DESIGN.md) ------------- */
 int sqt_measure_fp32_peak(sqt_ctx *ctx, double *gops_per_s);     /* non-fused FADD/FMUL issue rate, Gop/s */
 int sqt_measure_l2_bandwidth(sqt_ctx *ctx, double *gb_per_s);    /* L2-resident 128-bit read bandwidth */

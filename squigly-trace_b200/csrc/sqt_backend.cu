@@ -7,6 +7,7 @@
 // There is no CPU fallback in this file: every entry point needs a compute-capability-10.x device.
 #include <cuda_runtime.h>
 #include <stdarg.h>
+#include <stddef.h>
 #include <stdio.h>
 #include <string.h>
 #include <atomic>
@@ -21,6 +22,9 @@
 #include "sqt_nccl.hpp"
 
 // ============================================================================== context
+// launch shape of a frame's sample rounds (prepare_render): work items, this rank's sample range, S = 1 << log2_s
+struct RenderPlan { long long nwork = 0; int k0 = 0, k1 = 0, log2_s = 0; long long sbytes = 0; };
+
 struct sqt_ctx {
     int device = 0, sm_count = 0, cc_major = 0, cc_minor = 0;
     char name[128] = {0};
@@ -67,10 +71,22 @@ struct sqt_ctx {
     int pool_carveout = 0;              // shared-memory carve-out of k_paths_pool in percent of 228 KB (0 = the driver's choice)
     float4 *d_gstack = nullptr; uint16_t *d_gpm = nullptr; uint4 *d_gpath = nullptr; long long cap_pool_slots = 0, cap_stack_entries = 0;
     bool comm_broken = false;           // the communicator was aborted after a rank failed
+    // progressive frame (sqt_render_begin / sqt_render_advance): what the frame needs between two calls
+    bool prog = false;                  // a progressive frame is in progress
+    int prog_k = 0;                     // samples [0, prog_k) are in the sums
+    bool prog_count = false;
+    RenderParams prog_d = {};
+    RenderPlan prog_pl;
+    float *d_m2 = nullptr; long long cap_m2 = 0;                 // per-pixel second moment (npix * 3 floats)
+    float *d_red1 = nullptr, *d_red2 = nullptr; long long cap_red = 0;   // rank 0 of a group: sums and moments of all ranks
+    double *d_noise = nullptr, *h_noise = nullptr;               // partial sums of k_frame_noise_part + the result (pinned copy)
     // group
     int rank = 0, world = 1;
     ncclComm_t comm = nullptr;
 };
+
+// d_flag: word 0 the material check of an upload, words 1.. the group agreement (flag + up to three keys as (v, -v))
+constexpr int kFlagWords = 8;
 
 static thread_local std::string g_create_err;
 
@@ -136,7 +152,7 @@ extern "C" int sqt_create(int device, sqt_ctx **out) {
         CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
         for (auto &ev : c->ev) CU(cudaEventCreate(&ev));
         CU(cudaMalloc(&c->d_stats, sizeof(DeviceStats)));
-        CU(cudaMalloc(&c->d_flag, 2 * sizeof(uint32_t)));
+        CU(cudaMalloc(&c->d_flag, kFlagWords * sizeof(uint32_t)));
         CU(cudaMallocHost(&c->h_stats, sizeof(DeviceStats)));
         return SQT_OK;
     };
@@ -161,6 +177,8 @@ extern "C" int sqt_destroy(sqt_ctx *c) {
     free_scene(c);
     cudaFree(c->d_prim); cudaFree(c->d_accum); cudaFree(c->d_rgb8); cudaFree(c->d_stats); cudaFree(c->d_flag); cudaFree(c->d_pixel_list); cudaFree(c->d_sbuf); cudaFree(c->d_gstack); cudaFree(c->d_gpm); cudaFree(c->d_gpath);
     cudaFree(c->d_org); cudaFree(c->d_dir); cudaFree(c->d_dist); cudaFree(c->d_point); cudaFree(c->d_tri);
+    cudaFree(c->d_m2); cudaFree(c->d_red1); cudaFree(c->d_red2); cudaFree(c->d_noise);
+    if (c->h_noise) cudaFreeHost(c->h_noise);
     if (c->h_stats) cudaFreeHost(c->h_stats);
     if (c->h_rgb8) cudaFreeHost(c->h_rgb8);
     if (c->h_accum) cudaFreeHost(c->h_accum);
@@ -254,6 +272,7 @@ static void stream_tris(sqt_ctx **ctxs, int n, const sqt_tri *tris, size_t n_tri
 static int upload_scene_to(sqt_ctx **ctxs, int n, const sqt_scene_desc *s) {
     sqt_ctx *ctx = ctxs[0];
     const double t0 = now_ms();
+    for (int g = 0; g < n; ++g) ctxs[g]->prog = false;          // a new scene ends a progressive frame
     if (!s->nodes || s->n_nodes == 0) return fail(ctx, SQT_E_INVALID, "scene has no BIH nodes");
     if (s->n_tris && !s->tris) return fail(ctx, SQT_E_INVALID, "tris is NULL");
     if (s->n_tris >= (1u << 27) || s->n_nodes >= (1u << 27)) return fail(ctx, SQT_E_UNSUPPORTED, "scene too large for the 27-bit indices");
@@ -369,6 +388,7 @@ extern "C" int sqt_last_upload(const sqt_ctx *ctx, uint64_t *h2d_bytes, double *
 // extension: analytic spheres (include/sqt.h)
 extern "C" int sqt_upload_spheres(sqt_ctx *ctx, const sqt_sphere *sp, uint32_t n) {
     if (!ctx) return SQT_E_INVALID;
+    ctx->prog = false;
     if (!ctx->has_scene) return fail(ctx, SQT_E_NO_SCENE, "sqt_upload_spheres before sqt_upload_scene");
     if (n && !sp) return fail(ctx, SQT_E_INVALID, "spheres is NULL");
     if ((uint64_t)ctx->sc.n_tris + n >= (1u << 27)) return fail(ctx, SQT_E_UNSUPPORTED, "too many surfaces");
@@ -527,7 +547,8 @@ extern "C" int sqt_intersect_batch(sqt_ctx *ctx, const float *org, const float *
     CU(cudaEventRecord(ctx->ev[0], st));
     CU(cudaMemcpyAsync(ctx->d_org, org, (size_t)n * 12, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(ctx->d_dir, dir, (size_t)n * 12, cudaMemcpyHostToDevice, st));
-    CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), st));
+    // the counters only: n_hit is the pixel list of a progressive frame's primary pass, which this call does not end
+    CU(cudaMemsetAsync(ctx->d_stats, 0, offsetof(DeviceStats, n_hit), st));
     CU(cudaEventRecord(ctx->ev[1], st));
     if (stats)      // instrumented variant: fills the visit/test counters
         k_intersect_batch<true><<<persistent_grid(ctx, k_intersect_batch<true>, n), 128, 0, st>>>(
@@ -585,7 +606,6 @@ static RenderParams to_device_params(const sqt_ctx *ctx, const sqt_camera *cam, 
 
 // Everything of a render that can fail for lack of memory or because of its arguments, done BEFORE any kernel or
 // collective is enqueued: image buffers, the sample buffer of a round, the pool slots' global state.
-struct RenderPlan { long long nwork = 0; int k0 = 0, k1 = 0, log2_s = 0; long long sbytes = 0; };
 static int prepare_render(sqt_ctx *ctx, const RenderParams &d, bool count, bool host_image, RenderPlan &pl) {
     const long long npix = (long long)d.rows * d.cols;
     int rc = ensure_image(ctx, npix); if (rc) return rc;
@@ -609,25 +629,31 @@ static int prepare_render(sqt_ctx *ctx, const RenderParams &d, bool count, bool 
 // Multi-rank contexts: all ranks learn whether every rank got through check_params + prepare_render, with a one-word
 // ncclAllReduce(max) -- a collective every rank reaches whatever happened to it locally.  Only if all agree is the
 // frame (and its ncclReduce) enqueued; otherwise every rank returns an error and nobody waits in a collective.
-static int group_agree(sqt_ctx *ctx, int rc_local) {
+// `keys` (progressive frames: samples done, target spp, end of the chunk) must be equal on every rank: each travels as
+// (v, -v) in the same all-reduce, so max(v) == -max(-v) holds exactly when all ranks agree.
+static int group_agree(sqt_ctx *ctx, int rc_local, const int32_t *keys = nullptr, int n_keys = 0) {
     if (ctx->world <= 1 || !ctx->comm) return rc_local;
     if (ctx->comm_broken) return fail(ctx, SQT_E_NCCL, "the communicator of this group was aborted after an earlier failure");
     NcclApi *na = nccl_api();
     const std::string local_err = ctx->err;
     cudaSetDevice(ctx->device);
     uint32_t *flag = ctx->d_flag + 1;
-    const uint32_t v = rc_local ? 1u : 0u;
-    uint32_t out = 1u;
-    cudaError_t e = cudaMemcpyAsync(flag, &v, 4, cudaMemcpyHostToDevice, ctx->stream);
-    ncclResult_t r = e == cudaSuccess ? na->AllReduce(flag, flag, 1, kNcclInt32, kNcclMax, ctx->comm, ctx->stream) : 1;
-    if (r == 0) e = cudaMemcpyAsync(&out, flag, 4, cudaMemcpyDeviceToHost, ctx->stream);
+    const int nw = 1 + 2 * n_keys;
+    uint32_t v[kFlagWords - 1] = {rc_local ? 1u : 0u}, out[kFlagWords - 1] = {1u};
+    for (int i = 0; i < n_keys; ++i) { v[1 + 2 * i] = (uint32_t)keys[i]; v[2 + 2 * i] = (uint32_t)(-keys[i]); }
+    cudaError_t e = cudaMemcpyAsync(flag, v, nw * 4, cudaMemcpyHostToDevice, ctx->stream);
+    ncclResult_t r = e == cudaSuccess ? na->AllReduce(flag, flag, nw, kNcclInt32, kNcclMax, ctx->comm, ctx->stream) : 1;
+    if (r == 0) e = cudaMemcpyAsync(out, flag, nw * 4, cudaMemcpyDeviceToHost, ctx->stream);
     if (r == 0 && e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (r != 0 || e != cudaSuccess) {
         na->CommAbort(ctx->comm); ctx->comm_broken = true;
         return fail(ctx, SQT_E_NCCL, "group agreement failed (%s); communicator aborted", r ? na->GetErrorString(r) : cudaGetErrorString(e));
     }
     if (rc_local) { ctx->err = local_err; return rc_local; }
-    if (out) return fail(ctx, SQT_E_NCCL, "another rank of the group could not start this render; nothing was enqueued");
+    if (out[0]) return fail(ctx, SQT_E_NCCL, "another rank of the group could not start this render; nothing was enqueued");
+    for (int i = 0; i < n_keys; ++i)
+        if ((int32_t)out[1 + 2 * i] != -(int32_t)out[2 + 2 * i])
+            return fail(ctx, SQT_E_INVALID, "the ranks of the group disagree on the progressive frame (samples done / target spp / chunk); nothing was enqueued");
     return SQT_OK;
 }
 // a failure after the agreement (a launch error) would leave the other ranks waiting in ncclReduce: abort the communicator
@@ -636,68 +662,102 @@ static int group_abort(sqt_ctx *ctx, int rc) {
     return rc;
 }
 
-// Enqueue all kernels of one render on ctx->stream (no host sync, no allocation).  Events: 0 start, 1 after primary,
-// 2 after paths, 3 after reduce, 4 after tonemap.
-static int enqueue_render(sqt_ctx *ctx, const RenderParams &d, bool count, const RenderPlan &pl, uint32_t *launches) {
+// Enqueue the kernels of a render on ctx->stream (no host sync, no allocation), in three stages: frame start, sample
+// rounds, finish.  A one-shot frame is start + rounds [k0, k1) + finish; a progressive frame runs the start once and
+// rounds + finish once per chunk.  Events: 0 start, 1 after primary, 2 after paths, 3 after reduce, 4 after tonemap.
+
+// frame start: zero the stats and the sums, the primary pass
+static int enqueue_start(sqt_ctx *ctx, const RenderParams &d, bool count, const RenderPlan &pl, uint32_t &nl) {
     const long long npix = (long long)d.rows * d.cols;
-    int rc = SQT_OK;
     cudaStream_t st = ctx->stream;
     CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), st));
     CU(cudaMemsetAsync(ctx->d_accum, 0, (size_t)npix * 3 * sizeof(float), st));
     CU(cudaEventRecord(ctx->ev[0], st));
+    if (d.mode == 0 && d.primary_reuse) {
+        if (count) k_primary<true><<<persistent_grid(ctx, k_primary<true>, pl.nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_prim, ctx->d_pixel_list, ctx->d_stats, ctx->tune);
+        else k_primary<false><<<persistent_grid(ctx, k_primary<false>, pl.nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_prim, ctx->d_pixel_list, ctx->d_stats, ctx->tune);
+        CU(cudaGetLastError()); nl++;
+    }
+    CU(cudaEventRecord(ctx->ev[1], st));
+    return SQT_OK;
+}
+
+// samples [ka, kb) in rounds of S samples per pixel: trace (persistent lanes, one work counter per round, numbered from
+// 0 in every call), then add in sample order -- onto the sums alone (m2 == nullptr) or the sums and the second moments
+static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, const RenderPlan &pl, int ka, int kb, float *m2, uint32_t &nl) {
+    int rc = SQT_OK;
+    cudaStream_t st = ctx->stream;
     const long long nwork = pl.nwork;
-    uint32_t nl = 0;
     if (d.mode == 1) {
-        CU(cudaEventRecord(ctx->ev[1], st));
         if (count) k_raycast<true><<<persistent_grid(ctx, k_raycast<true>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_accum, ctx->d_stats, ctx->tune);
         else k_raycast<false><<<persistent_grid(ctx, k_raycast<false>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_accum, ctx->d_stats, ctx->tune);
         CU(cudaGetLastError()); nl++;
-    } else {
-        if (d.primary_reuse) {
-            if (count) k_primary<true><<<persistent_grid(ctx, k_primary<true>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_prim, ctx->d_pixel_list, ctx->d_stats, ctx->tune);
-            else k_primary<false><<<persistent_grid(ctx, k_primary<false>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_prim, ctx->d_pixel_list, ctx->d_stats, ctx->tune);
-            CU(cudaGetLastError()); nl++;
-        }
-        CU(cudaEventRecord(ctx->ev[1], st));
-        // rounds of S samples per pixel: trace (persistent lanes, one counter per round), then add in sample order
-        const int k0 = pl.k0, k1 = pl.k1;
-        RoundInfo rd = {};
-        rd.pixel_list = d.primary_reuse ? ctx->d_pixel_list : nullptr;
-        rd.prim = d.primary_reuse ? ctx->d_prim : nullptr;
-        rd.n_slots = nwork; rd.slot_stride = nwork;
-        rd.log2_s = pl.log2_s;
-        const int S = 1 << rd.log2_s;
-        rd.sbuf = ctx->d_sbuf;
-        const int agrid = (int)((nwork + 255) / 256 < (long long)ctx->sm_count * 8 ? (nwork + 255) / 256 : (long long)ctx->sm_count * 8);
-        int round = 0;
-        for (int kb = k0; kb < k1; kb += S, ++round) {
-            rd.k0 = kb; rd.k1 = kb + S < k1 ? kb + S : k1;
-            CU(cudaMemsetAsync(ctx->d_sbuf, 0, (size_t)(nwork * (long long)(rd.k1 - rd.k0) * 12ll), st));
-            if (ctx->pool_k > 0) {
-                rc = count ? pool_step_k<true>(ctx, d, rd, round, nwork << rd.log2_s, true) : pool_step_k<false>(ctx, d, rd, round, nwork << rd.log2_s, true);
-                if (rc) return rc;
-            } else if (count) k_paths<true><<<persistent_grid(ctx, k_paths<true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
-            else k_paths<false><<<persistent_grid(ctx, k_paths<false>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
-            CU(cudaGetLastError()); nl++;
-            k_accumulate<<<agrid > 0 ? agrid : 1, 256, 0, st>>>(d, rd, ctx->d_accum, ctx->d_stats);
-            CU(cudaGetLastError()); nl++;
-        }
+        return SQT_OK;
     }
+    RoundInfo rd = {};
+    rd.pixel_list = d.primary_reuse ? ctx->d_pixel_list : nullptr;
+    rd.prim = d.primary_reuse ? ctx->d_prim : nullptr;
+    rd.n_slots = nwork; rd.slot_stride = nwork;
+    rd.log2_s = pl.log2_s;
+    const int S = 1 << rd.log2_s;
+    rd.sbuf = ctx->d_sbuf;
+    const int agrid = (int)((nwork + 255) / 256 < (long long)ctx->sm_count * 8 ? (nwork + 255) / 256 : (long long)ctx->sm_count * 8);
+    int round = 0;
+    for (int k = ka; k < kb; k += S, ++round) {
+        rd.k0 = k; rd.k1 = k + S < kb ? k + S : kb;
+        CU(cudaMemsetAsync(ctx->d_sbuf, 0, (size_t)(nwork * (long long)(rd.k1 - rd.k0) * 12ll), st));
+        if (ctx->pool_k > 0) {
+            rc = count ? pool_step_k<true>(ctx, d, rd, round, nwork << rd.log2_s, true) : pool_step_k<false>(ctx, d, rd, round, nwork << rd.log2_s, true);
+            if (rc) return rc;
+        } else if (count) k_paths<true><<<persistent_grid(ctx, k_paths<true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
+        else k_paths<false><<<persistent_grid(ctx, k_paths<false>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
+        CU(cudaGetLastError()); nl++;
+        if (m2) k_accumulate_m2<<<agrid > 0 ? agrid : 1, 256, 0, st>>>(d, rd, ctx->d_accum, m2, ctx->d_stats);
+        else k_accumulate<<<agrid > 0 ? agrid : 1, 256, 0, st>>>(d, rd, ctx->d_accum, ctx->d_stats);
+        CU(cudaGetLastError()); nl++;
+    }
+    return SQT_OK;
+}
+
+// finish: the sums of all ranks onto rank 0 -- in place for a one-shot frame (sum1 == d_accum, no moments), into
+// rank 0's separate buffers for a progressive one (the ranks' running sums must survive the next reduce) -- then the
+// tone map with `inv` and, for a progressive frame after k samples, the noise estimate, both on rank 0
+static int enqueue_finish(sqt_ctx *ctx, long long npix, float inv, float *sum1, float *sum2, int k, uint32_t &nl) {
+    cudaStream_t st = ctx->stream;
     CU(cudaEventRecord(ctx->ev[2], st));
     if (ctx->world > 1 && ctx->comm) {
         NcclApi *na = nccl_api();
-        ncclResult_t r = na->Reduce(ctx->d_accum, ctx->d_accum, (size_t)npix * 3, kNcclFloat32, kNcclSum, 0, ctx->comm, st);
+        ncclResult_t r = na->Reduce(ctx->d_accum, sum1, (size_t)npix * 3, kNcclFloat32, kNcclSum, 0, ctx->comm, st);
         if (r != 0) return fail(ctx, SQT_E_NCCL, "ncclReduce failed: %s", na->GetErrorString(r));
         nl++;
+        if (sum2) {
+            r = na->Reduce(ctx->d_m2, sum2, (size_t)npix * 3, kNcclFloat32, kNcclSum, 0, ctx->comm, st);
+            if (r != 0) return fail(ctx, SQT_E_NCCL, "ncclReduce failed: %s", na->GetErrorString(r));
+            nl++;
+        }
     }
     CU(cudaEventRecord(ctx->ev[3], st));
     if (ctx->rank == 0) {
-        const float inv = 1.0f / (float)d.spp;
-        k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(ctx->d_accum, npix, inv, ctx->d_rgb8);
+        k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(sum1, npix, inv, ctx->d_rgb8);
         CU(cudaGetLastError()); nl++;
+        if (sum2) {
+            k_frame_noise_part<<<kNoiseBlocks, 256, 0, st>>>(sum1, sum2, npix * 3, k, ctx->d_noise);
+            k_frame_noise<<<1, kNoiseBlocks, 0, st>>>(ctx->d_noise, npix * 3, k, ctx->d_noise + 2 * kNoiseBlocks);
+            CU(cudaGetLastError()); nl += 2;
+            CU(cudaMemcpyAsync(ctx->h_noise, ctx->d_noise + 2 * kNoiseBlocks, sizeof(double), cudaMemcpyDeviceToHost, st));
+        }
     }
     CU(cudaEventRecord(ctx->ev[4], st));
     CU(cudaMemcpyAsync(ctx->h_stats, ctx->d_stats, sizeof(DeviceStats), cudaMemcpyDeviceToHost, st));
+    return SQT_OK;
+}
+
+static int enqueue_render(sqt_ctx *ctx, const RenderParams &d, bool count, const RenderPlan &pl, uint32_t *launches) {
+    const long long npix = (long long)d.rows * d.cols;
+    uint32_t nl = 0;
+    int rc = enqueue_start(ctx, d, count, pl, nl); if (rc) return rc;
+    rc = enqueue_rounds(ctx, d, count, pl, pl.k0, pl.k1, nullptr, nl); if (rc) return rc;
+    rc = enqueue_finish(ctx, npix, 1.0f / (float)d.spp, ctx->d_accum, nullptr, d.spp, nl); if (rc) return rc;
     ctx->img_pixels = npix; ctx->img_spp = d.spp;
     *launches = nl;
     return SQT_OK;
@@ -731,6 +791,7 @@ static void fill_stats(sqt_ctx *ctx, sqt_stats *s, uint32_t launches) {
 
 extern "C" int sqt_render_resident(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
     if (!ctx) return SQT_E_INVALID;
+    ctx->prog = false;
     if (stats) memset(stats, 0, sizeof *stats);
     cudaSetDevice(ctx->device);
     RenderParams d = {};
@@ -745,6 +806,14 @@ extern "C" int sqt_render_resident(sqt_ctx *ctx, const sqt_camera *cam, const sq
     return SQT_OK;
 }
 
+// the sums (moments = false) or second moments of the frame: on rank 0 of a progressive group frame the reduced
+// copies, everywhere else the context's own buffers
+static float *frame_sums(sqt_ctx *ctx, bool moments) {
+    const bool reduced = ctx->prog && ctx->world > 1 && ctx->comm && ctx->rank == 0;
+    if (moments) return reduced ? ctx->d_red2 : ctx->d_m2;
+    return reduced ? ctx->d_red1 : ctx->d_accum;
+}
+
 extern "C" int sqt_download_image(sqt_ctx *ctx, uint8_t *rgb8_out, float *accum_out) {
     if (!ctx) return SQT_E_INVALID;
     if (ctx->img_pixels <= 0) return fail(ctx, SQT_E_INVALID, "no rendered image to download");
@@ -752,7 +821,7 @@ extern "C" int sqt_download_image(sqt_ctx *ctx, uint8_t *rgb8_out, float *accum_
     const long long npix = ctx->img_pixels;
     int rc = ensure_host_image(ctx, npix); if (rc) return rc;
     if (rgb8_out) CU(cudaMemcpyAsync(ctx->h_rgb8, ctx->d_rgb8, (size_t)npix * 3, cudaMemcpyDeviceToHost, ctx->stream));
-    if (accum_out) CU(cudaMemcpyAsync(ctx->h_accum, ctx->d_accum, (size_t)npix * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    if (accum_out) CU(cudaMemcpyAsync(ctx->h_accum, frame_sums(ctx, false), (size_t)npix * 12, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     if (rgb8_out) memcpy(rgb8_out, ctx->h_rgb8, (size_t)npix * 3);
     if (accum_out) memcpy(accum_out, ctx->h_accum, (size_t)npix * 12);
@@ -762,6 +831,7 @@ extern "C" int sqt_download_image(sqt_ctx *ctx, uint8_t *rgb8_out, float *accum_
 extern "C" int sqt_render(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, uint8_t *rgb8_out,
                           float *accum_out, sqt_stats *stats) {
     if (!ctx) return SQT_E_INVALID;
+    ctx->prog = false;
     if (stats) memset(stats, 0, sizeof *stats);
     cudaSetDevice(ctx->device);
     RenderParams d = {};
@@ -792,6 +862,7 @@ extern "C" int sqt_render(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_
 
 extern "C" int sqt_tone_map(sqt_ctx *ctx, const float *mean_rgb, int64_t npix, uint8_t *rgb8_out) {
     if (!ctx) return SQT_E_INVALID;
+    ctx->prog = false;                  // d_accum is its scratch
     if (npix < 0 || (npix > 0 && (!mean_rgb || !rgb8_out))) return fail(ctx, SQT_E_INVALID, "bad tone_map arguments");
     if (npix == 0) return SQT_OK;
     CU(cudaSetDevice(ctx->device));
@@ -803,6 +874,111 @@ extern "C" int sqt_tone_map(sqt_ctx *ctx, const float *mean_rgb, int64_t npix, u
     CU(cudaMemcpyAsync(rgb8_out, ctx->d_rgb8, (size_t)npix * 3, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     ctx->img_pixels = 0;
+    return SQT_OK;
+}
+
+// ------------------------------------------------------------------------------ progressive frames
+// Every buffer a progressive frame needs beyond those of a one-shot render (prepare_render): the second moments, the
+// noise reduction's partial sums and, on rank 0 of a group, the reduced sums and moments.
+static int ensure_progressive(sqt_ctx *ctx, long long npix) {
+    if (!ctx->d_noise) CU(cudaMalloc(&ctx->d_noise, (2 * kNoiseBlocks + 1) * sizeof(double)));
+    if (!ctx->h_noise) CU(cudaMallocHost(&ctx->h_noise, sizeof(double)));
+    if (npix > ctx->cap_m2) {
+        cudaFree(ctx->d_m2); ctx->d_m2 = nullptr; ctx->cap_m2 = 0;
+        CU(cudaMalloc(&ctx->d_m2, (size_t)npix * 12));
+        ctx->cap_m2 = npix;
+    }
+    if (ctx->world > 1 && ctx->comm && ctx->rank == 0 && npix > ctx->cap_red) {
+        cudaFree(ctx->d_red1); cudaFree(ctx->d_red2); ctx->d_red1 = ctx->d_red2 = nullptr; ctx->cap_red = 0;
+        CU(cudaMalloc(&ctx->d_red1, (size_t)npix * 12));
+        CU(cudaMalloc(&ctx->d_red2, (size_t)npix * 12));
+        ctx->cap_red = npix;
+    }
+    return SQT_OK;
+}
+
+extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
+    if (!ctx) return SQT_E_INVALID;
+    if (stats) memset(stats, 0, sizeof *stats);
+    cudaSetDevice(ctx->device);
+    ctx->prog = false; ctx->img_pixels = 0;
+    RenderParams d = {};
+    RenderPlan pl;
+    int rc = check_params(ctx, cam, p);
+    if (!rc && p->mode != 0) rc = fail(ctx, SQT_E_UNSUPPORTED, "progressive frames trace paths (mode 0) only");
+    if (!rc && (p->flags & SQT_F_SPLIT_SAMPLES)) rc = fail(ctx, SQT_E_UNSUPPORTED, "progressive frames use the pixel-group partition, not SQT_F_SPLIT_SAMPLES");
+    const bool count = !rc && (p->flags & SQT_F_COUNT_WORK) != 0;
+    if (!rc) { d = to_device_params(ctx, cam, p); rc = prepare_render(ctx, d, count, false, pl); }
+    const long long npix = (long long)d.rows * d.cols;
+    if (!rc) rc = ensure_progressive(ctx, npix);
+    const int32_t keys[3] = {0, rc ? 0 : p->spp, 0};
+    rc = group_agree(ctx, rc, keys, 3); if (rc) return rc;
+    cudaStream_t st = ctx->stream;
+    uint32_t nl = 0;
+    auto enqueue = [&]() -> int {
+        CU(cudaMemsetAsync(ctx->d_m2, 0, (size_t)npix * 12, st));
+        int r = enqueue_start(ctx, d, count, pl, nl); if (r) return r;
+        for (int e = 2; e <= 4; ++e) CU(cudaEventRecord(ctx->ev[e], st));
+        CU(cudaMemcpyAsync(ctx->h_stats, ctx->d_stats, sizeof(DeviceStats), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        return SQT_OK;
+    };
+    rc = enqueue(); if (rc) return group_abort(ctx, rc);
+    fill_stats(ctx, stats, nl);
+    ctx->prog = true; ctx->prog_k = 0; ctx->prog_count = count; ctx->prog_d = d; ctx->prog_pl = pl;
+    return SQT_OK;
+}
+
+extern "C" int sqt_render_advance(sqt_ctx *ctx, int32_t n_samples, sqt_progress *progress, sqt_stats *stats) {
+    if (!ctx) return SQT_E_INVALID;
+    if (stats) memset(stats, 0, sizeof *stats);
+    cudaSetDevice(ctx->device);
+    int rc = SQT_OK;
+    if (!ctx->prog) rc = fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    else if (n_samples < 1) rc = fail(ctx, SQT_E_INVALID, "n_samples must be at least 1");
+    const RenderParams &d = ctx->prog_d;
+    const int k = ctx->prog_k, spp = d.spp;
+    const int kb = rc ? 0 : (n_samples >= spp - k ? spp : k + n_samples);
+    const int32_t keys[3] = {rc ? 0 : k, rc ? 0 : spp, kb};
+    rc = group_agree(ctx, rc, keys, 3); if (rc) return rc;
+    const bool root = ctx->rank == 0;
+    if (k < spp) {
+        const long long npix = (long long)d.rows * d.cols;
+        cudaStream_t st = ctx->stream;
+        uint32_t nl = 0;
+        auto enqueue = [&]() -> int {
+            // the counters of this call only; n_hit (the primary pass's pixel list) stays
+            CU(cudaMemsetAsync(ctx->d_stats, 0, offsetof(DeviceStats, n_hit), st));
+            CU(cudaMemsetAsync((char *)ctx->d_stats + offsetof(DeviceStats, work_next), 0, sizeof(DeviceStats) - offsetof(DeviceStats, work_next), st));
+            CU(cudaEventRecord(ctx->ev[0], st));
+            CU(cudaEventRecord(ctx->ev[1], st));
+            int r = enqueue_rounds(ctx, d, ctx->prog_count, ctx->prog_pl, k, kb, ctx->d_m2, nl); if (r) return r;
+            r = enqueue_finish(ctx, npix, 1.0f / (float)kb, frame_sums(ctx, false), frame_sums(ctx, true), kb, nl); if (r) return r;
+            CU(cudaStreamSynchronize(st));
+            return SQT_OK;
+        };
+        rc = enqueue();
+        if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+        fill_stats(ctx, stats, nl);
+        ctx->prog_k = kb; ctx->img_pixels = npix; ctx->img_spp = kb;
+    }
+    if (progress) {
+        progress->samples_done = ctx->prog_k; progress->samples_total = spp;
+        progress->noise = root ? *ctx->h_noise : __builtin_nan("");
+    }
+    return SQT_OK;
+}
+
+extern "C" int sqt_download_moments(sqt_ctx *ctx, float *m2_out) {
+    if (!ctx) return SQT_E_INVALID;
+    if (!ctx->prog) return fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    if (!m2_out) return fail(ctx, SQT_E_INVALID, "m2_out is NULL");
+    CU(cudaSetDevice(ctx->device));
+    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    int rc = ensure_host_image(ctx, npix); if (rc) return rc;
+    CU(cudaMemcpyAsync(ctx->h_accum, frame_sums(ctx, true), (size_t)npix * 12, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    memcpy(m2_out, ctx->h_accum, (size_t)npix * 12);
     return SQT_OK;
 }
 
@@ -854,6 +1030,34 @@ extern "C" int sqt_render_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, co
     for (int i = 1; i < n; ++i)
         th.emplace_back([&, i]() { rcs[i] = sqt_render(ctxs[i], cam, p, nullptr, nullptr, nullptr); });
     rcs[0] = sqt_render(ctxs[0], cam, p, rgb8_out, accum_out, stats);
+    for (auto &t : th) t.join();
+    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
+    return SQT_OK;
+}
+
+// progressive frames on every context of a single-process group, one host thread per device like sqt_render_group
+// (rank 0 gets the progress and the stats)
+extern "C" int sqt_render_begin_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
+    if (!ctxs || n < 1) return SQT_E_INVALID;
+    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
+    if (n == 1) return sqt_render_begin(ctxs[0], cam, p, stats);
+    std::vector<int> rcs(n, 0);
+    std::vector<std::thread> th;
+    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_begin(ctxs[i], cam, p, nullptr); });
+    rcs[0] = sqt_render_begin(ctxs[0], cam, p, stats);
+    for (auto &t : th) t.join();
+    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
+    return SQT_OK;
+}
+
+extern "C" int sqt_render_advance_group(sqt_ctx **ctxs, int n, int32_t n_samples, sqt_progress *progress, sqt_stats *stats) {
+    if (!ctxs || n < 1) return SQT_E_INVALID;
+    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
+    if (n == 1) return sqt_render_advance(ctxs[0], n_samples, progress, stats);
+    std::vector<int> rcs(n, 0);
+    std::vector<std::thread> th;
+    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_advance(ctxs[i], n_samples, nullptr, nullptr); });
+    rcs[0] = sqt_render_advance(ctxs[0], n_samples, progress, stats);
     for (auto &t : th) t.join();
     for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
     return SQT_OK;

@@ -6,6 +6,8 @@
 //                        queues by the kind of step they need and serves one queue per round with all lanes (default)
 //   k_paths            : the integrator with one ray per lane and warp-synchronous phases (SQT_POOL=0)
 //   k_accumulate       : adds a round's samples to the per-pixel sums in sample order (Lib.hs:88)
+//   k_accumulate_m2    : the same plus the per-pixel second moment (progressive frames)
+//   k_frame_noise_part, k_frame_noise : deterministic fp64 noise estimate of a progressive frame
 //   k_raycast          : --cast mode (Lib.hs:141-151)
 //   k_tonemap          : mean + rgbFloatToPixelRGB (Lib.hs:88-104)
 //   k_leaf_records, k_check_materials, k_branch_tight, k_child_slabs, k_flag_slabs : scene upload (leaf records from the triangles; material
@@ -613,6 +615,58 @@ __global__ void __launch_bounds__(256) k_accumulate(RenderParams p, RoundInfo rd
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long slot = (long long)blockIdx.x * blockDim.x + threadIdx.x; slot < rd.n_slots; slot += stride)
         accumulate_slot(p, rd, slot, accum);
+}
+// the same for a progressive frame: running sums and second moments (accumulate_m2_slot)
+__global__ void __launch_bounds__(256) k_accumulate_m2(RenderParams p, RoundInfo rd, float *__restrict__ accum, float *__restrict__ m2,
+                                                       const DeviceStats *ds) {
+    if (rd.pixel_list) rd.n_slots = (long long)ds->n_hit;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long slot = (long long)blockIdx.x * blockDim.x + threadIdx.x; slot < rd.n_slots; slot += stride)
+        accumulate_m2_slot(p, rd, slot, accum, m2);
+}
+
+// Noise estimate of a progressive frame after n samples, over all N = 3*npix values (s1 = sum, s2 = second moment):
+//   mu = s1/n, var = max(0, (s2 - s1*mu)/(n-1)), e2 = var/n, noise = sqrt(sum(e2)/N) / (sum(mu)/N)
+// in fp64.  Two stages with a fixed shape (kNoiseBlocks x 256 threads, then one block), so the order of every addition
+// depends on N alone -- never on the SM count -- and the same buffers always give the same bits.
+constexpr int kNoiseBlocks = 512;
+__device__ __forceinline__ void block_sum2(double &a, double &b, double *sh) {      // fixed-order tree over the block
+    const int t = threadIdx.x;
+    sh[t] = a; sh[blockDim.x + t] = b;
+    __syncthreads();
+    for (int h = blockDim.x / 2; h > 0; h >>= 1) {
+        if (t < h) { sh[t] += sh[t + h]; sh[blockDim.x + t] += sh[blockDim.x + t + h]; }
+        __syncthreads();
+    }
+    a = sh[0]; b = sh[blockDim.x];
+}
+__global__ void __launch_bounds__(256) k_frame_noise_part(const float *__restrict__ s1, const float *__restrict__ s2, long long nval, int n,
+                                                          double *__restrict__ part) {
+    __shared__ double sh[512];
+    const double dn = (double)n;
+    double se2 = 0.0, smu = 0.0;
+    const long long stride = (long long)kNoiseBlocks * 256;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < nval; i += stride) {
+        const double a = (double)s1[i], q = (double)s2[i];
+        const double mu = a / dn;
+        const double v = (q - a * mu) / (dn - 1.0);
+        se2 += (v > 0.0 ? v : 0.0) / dn;
+        smu += mu;
+    }
+    block_sum2(se2, smu, sh);
+    if (threadIdx.x == 0) { part[2 * blockIdx.x] = se2; part[2 * blockIdx.x + 1] = smu; }
+}
+__global__ void __launch_bounds__(kNoiseBlocks) k_frame_noise(const double *__restrict__ part, long long nval, int n, double *__restrict__ noise) {
+    __shared__ double sh[2 * kNoiseBlocks];
+    double se2 = part[2 * threadIdx.x], smu = part[2 * threadIdx.x + 1];
+    block_sum2(se2, smu, sh);
+    if (threadIdx.x == 0) {
+        double r;
+        if (n < 2) r = __longlong_as_double(0x7ff0000000000000ll);          // +inf: no variance from one sample
+        else if (smu == 0.0) r = 0.0;
+        else r = sqrt(se2 / (double)nval) / (smu / (double)nval);
+        *noise = r;
+    }
 }
 
 template <bool COUNT>

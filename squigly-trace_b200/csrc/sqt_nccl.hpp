@@ -1,6 +1,6 @@
 // sqt_nccl.hpp -- NCCL reached through dlopen, so that the single-GPU path has no NCCL dependency at all.
-// Only the handful of entry points the render path uses (one ncclReduce of the accumulation buffers per frame,
-// a one-word ncclAllReduce with which the ranks agree that all of them can enter it, ncclCommAbort for the case
+// Only the handful of entry points the render path uses (ncclReduce of the accumulation buffers -- and moments --,
+// a few-word ncclAllReduce with which the ranks agree that all of them can enter it, ncclCommAbort for the case
 // they cannot).
 #pragma once
 #include <cuda_runtime.h>

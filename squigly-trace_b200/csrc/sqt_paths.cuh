@@ -270,6 +270,23 @@ SQT_HD void accumulate_slot(const RenderParams &p, const RoundInfo &rd, long lon
     }
     accum[3 * pixel] = sr; accum[3 * pixel + 1] = sg; accum[3 * pixel + 2] = sb;
 }
+// the same for a progressive frame, which also keeps the per-pixel second moment: s2 = s2 + x*x over the sample
+// radiances x, every operation rounded to binary32, in sample order
+SQT_HD void accumulate_m2_slot(const RenderParams &p, const RoundInfo &rd, long long slot, float *accum, float *m2) {
+    const long long pixel = rd.pixel_list ? (long long)rd.pixel_list[slot] : work_to_pixel(p, slot);
+    if (pixel < 0) return;
+    float sr = accum[3 * pixel], sg = accum[3 * pixel + 1], sb = accum[3 * pixel + 2];
+    float qr = m2[3 * pixel], qg = m2[3 * pixel + 1], qb = m2[3 * pixel + 2];
+    const int n = rd.k1 - rd.k0;
+    for (int ks = 0; ks < n; ++ks) {
+        const long long i = 3 * ((long long)ks * rd.slot_stride + slot);
+        const float xr = rd.sbuf[i], xg = rd.sbuf[i + 1], xb = rd.sbuf[i + 2];
+        sr = XADD(sr, xr); sg = XADD(sg, xg); sb = XADD(sb, xb);
+        qr = XADD(qr, XMUL(xr, xr)); qg = XADD(qg, XMUL(xg, xg)); qb = XADD(qb, XMUL(xb, xb));
+    }
+    accum[3 * pixel] = sr; accum[3 * pixel + 1] = sg; accum[3 * pixel + 2] = sb;
+    m2[3 * pixel] = qr; m2[3 * pixel + 1] = qg; m2[3 * pixel + 2] = qb;
+}
 
 // samples per pixel per round: the largest power of two <= spp whose sample buffer (slots * S * 12 B) fits the budget
 SQT_HD int round_log2_s(long long slots, int n_samples, long long budget_bytes) {

@@ -1,6 +1,6 @@
 // main.cpp -- the squigly-trace command line (app/Main.hs:13-75) driving the B200 backend.
 // Flags follow the cmdargs record of the reference: -s/--samples, -d/--dimensions W,H, -p/--savepath,
-// --objpath, -c/--camerapath, --debug, --debugpath, --cast ; plus --bounces, --gpus, --corrected, --seed.
+// --objpath, -c/--camerapath, --debug, --debugpath, --cast ; plus --bounces, --gpus, --corrected, --seed, --progress.
 #include <chrono>
 #include <cstdlib>
 #include <cstring>
@@ -26,6 +26,7 @@ static void usage() {
                  "     --gpus=INT          Number of B200s to use\n"
                  "     --corrected         Width x height image with per-axis offsets (default: Lib.hs index convention)\n"
                  "     --seed=INT          RNG key\n"
+                 "     --progress=INT      Render in chunks of INT samples, saving a preview after each\n"
                  "  -? --help              Display help message\n";
 }
 
@@ -64,6 +65,7 @@ int main(int argc, char **argv) {
             else if (a == "--gpus") st.gpus = std::stoi(need());
             else if (a == "--corrected") st.corrected = true;
             else if (a == "--seed") st.seed = std::stoull(need());
+            else if (a == "--progress") { st.progress = std::stoi(need()); if (st.progress < 1) throw std::runtime_error("--progress must be at least 1"); }
             else if (a == "-?" || a == "--help") { usage(); return 0; }
             else throw std::runtime_error("Unknown flag: " + a);
         }

@@ -1,4 +1,6 @@
 // render.cpp -- `render` (Lib.hs:68-75) and the Scene plug-in (Geometry.hs:62-65) on top of the C ABI.
+#include <chrono>
+#include <cstdio>
 #include <cstring>
 #include <iostream>
 
@@ -91,7 +93,36 @@ RenderReport renderToBuffer(const SceneBIH &scene, const Camera &cam, const Sett
     return rep;
 }
 
+// --progress=N: the same frame as a progressive one (include/sqt.h) in chunks of N samples; after every chunk the preview
+// overwrites the save path and one line reports samples done, the noise estimate and the elapsed time.  The last image
+// is the one-shot frame bit for bit.
+static RenderReport renderProgressive(const SceneBIH &scene, const Camera &cam, const Settings &settings) {
+    const sqt_render_params p = paramsFromSettings(settings);
+    if (p.mode != 0) throw std::runtime_error("--progress needs path tracing (not --cast)");
+    sqt_camera c;
+    c.position[0] = cam.position.x; c.position[1] = cam.position.y; c.position[2] = cam.position.z;
+    std::memcpy(c.rotation, cam.rotation, sizeof c.rotation);
+    RenderReport rep; rep.rows = p.rows; rep.cols = p.cols;
+    std::vector<uint8_t> img((size_t)p.rows * p.cols * 3, 0);
+    const DeviceBIH &g = *scene.geometry;
+    const auto t0 = std::chrono::steady_clock::now();
+    g.check(0, sqt_render_begin_group(g.ctxs(), g.gpus(), &c, &p, &rep.stats), "sqt_render_begin");
+    sqt_progress pr{0, p.spp, 0.0};
+    while (pr.samples_done < pr.samples_total) {
+        sqt_stats st;
+        g.check(0, sqt_render_advance_group(g.ctxs(), g.gpus(), settings.progress, &pr, &st), "sqt_render_advance");
+        rep.stats.device_ms += st.device_ms; rep.stats.rays_traced += st.rays_traced; rep.stats.samples += st.samples;
+        g.check(0, sqt_download_image(g.ctx(0), img.data(), nullptr), "sqt_download_image");
+        writeImage(settings.savePath, img.data(), rep.rows, rep.cols);
+        const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        std::printf("%d/%d samples  noise %.6g  %.3fs\n", pr.samples_done, pr.samples_total, pr.noise, sec);
+        std::fflush(stdout);
+    }
+    return rep;
+}
+
 RenderReport render(const SceneBIH &scene, const Camera &cam, const Settings &settings) {
+    if (settings.progress > 0) return renderProgressive(scene, cam, settings);
     std::vector<uint8_t> img;
     RenderReport rep = renderToBuffer(scene, cam, settings, img, nullptr);
     writeImage(settings.savePath, img.data(), rep.rows, rep.cols);        // img `seq` writeImage savePath img

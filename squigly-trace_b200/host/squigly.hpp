@@ -102,6 +102,7 @@ struct Settings {
     int gpus = 1;
     bool corrected = false;     // false = Lib.hs:69-85 index convention verbatim (SURVEY A.5)
     uint64_t seed = 0;
+    int progress = 0;           // > 0: render in chunks of this many samples, writing a preview after each
 };
 struct RenderReport { sqt_stats stats{}; int rows = 0, cols = 0; };
 // render :: Scene a -> Camera -> Settings -> IO ()   (Lib.hs:68-75): computes the image on the device(s) and writes it

@@ -28,7 +28,8 @@ ABI_SYMBOLS = [
     "sqt_abi_version", "sqt_create", "sqt_destroy", "sqt_last_error", "sqt_upload_scene", "sqt_intersect_batch",
     "sqt_render", "sqt_render_resident", "sqt_download_image", "sqt_tone_map", "sqt_comm_unique_id", "sqt_comm_init",
     "sqt_comm_init_all", "sqt_render_group", "sqt_measure_fp32_peak", "sqt_measure_l2_bandwidth", "sqt_device_info", "sqt_set_option", "sqt_upload_spheres",
-    "sqt_upload_scene_group", "sqt_last_upload",
+    "sqt_upload_scene_group", "sqt_last_upload", "sqt_render_begin", "sqt_render_advance", "sqt_render_begin_group",
+    "sqt_render_advance_group", "sqt_download_moments",
 ]
 
 
@@ -76,6 +77,10 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
 
 
+class Progress(C.Structure):
+    _fields_ = [("samples_done", C.c_int32), ("samples_total", C.c_int32), ("noise", C.c_double)]
+
+
 NODE_DT = np.dtype([("lmax", "<f4"), ("rmin", "<f4"), ("a", "<u4"), ("b", "<u4")])
 TRI_DT = np.dtype([("v0", "<f4", 3), ("e1", "<f4", 3), ("e2", "<f4", 3), ("material", "<u4"), ("orig_index", "<u4"), ("pad", "<u4")])
 SPHERE_DT = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4"), ("pad", "<u4", 3)])
@@ -119,6 +124,11 @@ def b200():
         L.sqt_upload_spheres.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
         L.sqt_upload_scene_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.sqt_last_upload.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_double), C.POINTER(C.c_double)]
+        L.sqt_render_begin.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sqt_render_advance.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+        L.sqt_render_begin_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sqt_render_advance_group.argtypes = [C.c_void_p, C.c_int, C.c_int32, C.c_void_p, C.c_void_p]
+        L.sqt_download_moments.argtypes = [C.c_void_p, C.c_void_p]
         L.sqt_device_info.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p]
         for name in ABI_SYMBOLS:
             if name not in ("sqt_last_error",):
@@ -316,6 +326,24 @@ class Context:
         self._ck(self.L.sqt_download_image(self.h, _p(rgb8), _p(accum)), "sqt_download_image")
         return rgb8, accum
 
+    def render_begin(self, cam12, params):
+        """Start a progressive frame (include/sqt.h): checks, allocations and the primary pass; returns the stats."""
+        cam = camera_struct(cam12)
+        st = Stats()
+        self._ck(self.L.sqt_render_begin(self.h, C.byref(cam), C.byref(params), C.byref(st)), "sqt_render_begin")
+        return st.as_dict()
+
+    def render_advance(self, n_samples):
+        """Trace the next n_samples samples per pixel of the progressive frame."""
+        pr, st = Progress(), Stats()
+        self._ck(self.L.sqt_render_advance(self.h, n_samples, C.byref(pr), C.byref(st)), "sqt_render_advance")
+        return dict(samples_done=pr.samples_done, samples_total=pr.samples_total, noise=pr.noise, stats=st.as_dict())
+
+    def download_moments(self, rows, cols):
+        m2 = np.zeros((rows, cols, 3), np.float32)
+        self._ck(self.L.sqt_download_moments(self.h, _p(m2)), "sqt_download_moments")
+        return m2
+
     def tone_map(self, mean_rgb):
         mean_rgb = np.ascontiguousarray(mean_rgb, np.float32)
         out = np.zeros(mean_rgb.shape, np.uint8)
@@ -375,6 +403,21 @@ class Group:
         if rc:
             raise SqtError("sqt_render_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
         return dict(rgb8=rgb8, accum=accum, stats=st.as_dict())
+
+    def render_begin(self, cam12, params):
+        cam = camera_struct(cam12)
+        st = Stats()
+        rc = self.L.sqt_render_begin_group(self.arr, len(self.ctxs), C.byref(cam), C.byref(params), C.byref(st))
+        if rc:
+            raise SqtError("sqt_render_begin_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        return st.as_dict()
+
+    def render_advance(self, n_samples):
+        pr, st = Progress(), Stats()
+        rc = self.L.sqt_render_advance_group(self.arr, len(self.ctxs), n_samples, C.byref(pr), C.byref(st))
+        if rc:
+            raise SqtError("sqt_render_advance_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        return dict(samples_done=pr.samples_done, samples_total=pr.samples_total, noise=pr.noise, stats=st.as_dict())
 
     def close(self):
         for c in self.ctxs:

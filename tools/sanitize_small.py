@@ -1,5 +1,5 @@
 """Smallest end-to-end exercise of every kernel, for compute-sanitizer (one tool per gpurun call):
-intersect batch, render with both path schedulers, cast mode, spheres, tone map, multi-round accumulation."""
+intersect batch, render with both path schedulers, cast mode, spheres, tone map, multi-round accumulation, a progressive frame."""
 import os
 import sys
 
@@ -26,5 +26,9 @@ for pool in ("2", "0"):
     out3 = ctx.render(cam, pysqt.make_params(64, 48, 2, max_depth=4, seed=1))
     out4 = ctx.render(cam, pysqt.make_params(64, 48, 2, mode=1))
     ctx.tone_map(np.abs(rng.normal(size=(100, 3))).astype(np.float32))
+    ctx.render_begin(cam, pysqt.make_params(64, 48, 6, max_depth=5, seed=1))      # progressive: k_accumulate_m2, k_frame_noise*
+    for n in (1, 2, 3):
+        ctx.render_advance(n)
+    ctx.download_moments(48, 64)
     print("pool", pool, "ok", int((tri >= 0).sum()), out["stats"]["rays_traced"], out3["stats"]["rays_traced"])
     ctx.close()
