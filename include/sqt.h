@@ -224,6 +224,41 @@ int sqt_render_begin_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const s
 int sqt_render_advance_group(sqt_ctx **ctxs, int n, int32_t n_samples, sqt_progress *progress_or_null, sqt_stats *stats_or_null);
 int sqt_download_moments(sqt_ctx *ctx, float *m2_out);   /* rows*cols*3 floats: s2 of the frame in progress (rank 0) */
 
+/* adaptive sampling in a progressive frame: between two advances, stop tracing the pixels that have converged -------
+ *
+ * sqt_render_retire    looks at every active pixel after k = samples_done samples and retires it when k >= min_samples
+ *                      and, in fp64 and in this order (n = k: every active pixel has exactly k samples):
+ *                        for c in r,g,b:  mu_c = s1_c / n ;  v_c = (s2_c - s1_c*mu_c) / (n-1) ;  v_c = v_c > 0 ? v_c : 0
+ *                        e2 = (v_r + v_g + v_b) / n ;  m = mu_r + mu_g + mu_b ;  t = max(rel_tol * m, abs_tol)
+ *                        retire iff e2 < t*t
+ *                      (the per-value terms of the noise estimate).  The comparison is strict, so zero tolerances retire
+ *                      nothing, and an all-black pixel (m = 0, e2 = 0) only retires when abs_tol > 0.  A NaN in the sums,
+ *                      the moments or any of these terms means the pixel is never retired.  A retired pixel's sums and
+ *                      moments are frozen and it is never traced again in this frame.  *active_out: the pixels still
+ *                      active in the whole frame (all ranks).  At k = spp or k < min_samples it changes nothing.
+ *                      Stopping where the data says the estimate is good enough is a known source of bias: the expected
+ *                      value of an adaptive frame is not that of the spp frame.  Each pixel's VALUE is still exactly the
+ *                      n_p-sample prefix of the spp frame (seeds stay keyed to the target spp).
+ * sample count n_p     the samples in a pixel's sums: the k at which it retired, else samples_done (pixels without a
+ *                      primary hit included).  Previews and the final image are rgbFloatToPixelRGB(sum * (1.0f/(float)n_p))
+ *                      per pixel, the reciprocal correctly rounded, so a pixel with n_p = spp has sqt_render's bytes; the
+ *                      noise estimate uses n = n_p in each pixel's terms.  A frame that never retires is unchanged.
+ * sqt_render_advance   traces the active pixels only: stats.samples = active pixels * samples in the chunk.  With no
+ *                      active pixel left it launches nothing (samples_done still moves on).
+ * Errors: SQT_E_INVALID outside a frame, before k >= 2, for min_samples < 2, negative or NaN tolerances or non-zero
+ * reserved; SQT_E_UNSUPPORTED for a frame begun with SQT_F_NO_PRIMARY_REUSE.  Whatever ends a frame ends its adaptive
+ * state.  In a group every rank retires its own pixels from its own sums; ranks that disagree on k, the target spp or
+ * any of the three criteria fail on every rank before anything runs.  The counts reach rank 0 by a sum over ranks, and
+ * a group frame is bit-identical to one GPU's. */
+typedef struct sqt_retire_params {
+    float rel_tol, abs_tol;              /* error target: sqrt(e2) < max(rel_tol * m, abs_tol) */
+    int32_t min_samples;                 /* >= 2 */
+    uint32_t reserved;                   /* 0 */
+} sqt_retire_params;                     /* 16 B */
+int sqt_render_retire(sqt_ctx *ctx, const sqt_retire_params *rp, int64_t *active_out_or_null);
+int sqt_render_retire_group(sqt_ctx **ctxs, int n, const sqt_retire_params *rp, int64_t *active_out_or_null);
+int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out);   /* rows*cols n_p of the frame in progress (rank 0) */
+
 /* measured roofline denominators on this device (microbenchmarks; see DESIGN.md) ------------- */
 int sqt_measure_fp32_peak(sqt_ctx *ctx, double *gops_per_s);     /* non-fused FADD/FMUL issue rate, Gop/s */
 int sqt_measure_l2_bandwidth(sqt_ctx *ctx, double *gb_per_s);    /* L2-resident 128-bit read bandwidth */

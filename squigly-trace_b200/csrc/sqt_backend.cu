@@ -80,13 +80,19 @@ struct sqt_ctx {
     float *d_m2 = nullptr; long long cap_m2 = 0;                 // per-pixel second moment (npix * 3 floats)
     float *d_red1 = nullptr, *d_red2 = nullptr; long long cap_red = 0;   // rank 0 of a group: sums and moments of all ranks
     double *d_noise = nullptr, *h_noise = nullptr;               // partial sums of k_frame_noise_part + the result (pinned copy)
+    // adaptive frame (sqt_render_retire): per-pixel sample counts (0 = active) and the scratch of the list compaction
+    bool prog_adaptive = false;         // retire has run in this frame: d_pixel_list / n_hit hold the active pixels
+    long long prog_n = 0;               // this rank's active slots (the primary pass's hit count until the first retire)
+    long long prog_total = 0;           // active pixels of the whole frame after the last retire
+    int *d_counts = nullptr, *d_redc = nullptr, *d_list2 = nullptr; uint8_t *d_keep = nullptr; long long *d_tile = nullptr;
+    long long *d_active = nullptr, *h_active = nullptr;          // all-reduced active total; pinned (local, total)
     // group
     int rank = 0, world = 1;
     ncclComm_t comm = nullptr;
 };
 
-// d_flag: word 0 the material check of an upload, words 1.. the group agreement (flag + up to three keys as (v, -v))
-constexpr int kFlagWords = 8;
+// d_flag: word 0 the material check of an upload, words 1.. the group agreement (flag + up to seven keys as (v, -v))
+constexpr int kFlagWords = 16;
 
 static thread_local std::string g_create_err;
 
@@ -178,7 +184,9 @@ extern "C" int sqt_destroy(sqt_ctx *c) {
     cudaFree(c->d_prim); cudaFree(c->d_accum); cudaFree(c->d_rgb8); cudaFree(c->d_stats); cudaFree(c->d_flag); cudaFree(c->d_pixel_list); cudaFree(c->d_sbuf); cudaFree(c->d_gstack); cudaFree(c->d_gpm); cudaFree(c->d_gpath);
     cudaFree(c->d_org); cudaFree(c->d_dir); cudaFree(c->d_dist); cudaFree(c->d_point); cudaFree(c->d_tri);
     cudaFree(c->d_m2); cudaFree(c->d_red1); cudaFree(c->d_red2); cudaFree(c->d_noise);
+    cudaFree(c->d_counts); cudaFree(c->d_redc); cudaFree(c->d_list2); cudaFree(c->d_keep); cudaFree(c->d_tile); cudaFree(c->d_active);
     if (c->h_noise) cudaFreeHost(c->h_noise);
+    if (c->h_active) cudaFreeHost(c->h_active);
     if (c->h_stats) cudaFreeHost(c->h_stats);
     if (c->h_rgb8) cudaFreeHost(c->h_rgb8);
     if (c->h_accum) cudaFreeHost(c->h_accum);
@@ -682,12 +690,12 @@ static int enqueue_start(sqt_ctx *ctx, const RenderParams &d, bool count, const 
     return SQT_OK;
 }
 
-// samples [ka, kb) in rounds of S samples per pixel: trace (persistent lanes, one work counter per round, numbered from
-// 0 in every call), then add in sample order -- onto the sums alone (m2 == nullptr) or the sums and the second moments
-static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, const RenderPlan &pl, int ka, int kb, float *m2, uint32_t &nl) {
+// samples [ka, kb) of `nwork` slots in rounds of S = 1 << log2_s samples per pixel: trace (persistent lanes, one work
+// counter per round, numbered from 0 in every call), then add in sample order -- onto the sums alone (m2 == nullptr) or
+// the sums and the second moments.  nwork, log2_s: the plan's, or an adaptive frame's active slots (sqt_render_advance).
+static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, long long nwork, int log2_s, int ka, int kb, float *m2, uint32_t &nl) {
     int rc = SQT_OK;
     cudaStream_t st = ctx->stream;
-    const long long nwork = pl.nwork;
     if (d.mode == 1) {
         if (count) k_raycast<true><<<persistent_grid(ctx, k_raycast<true>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_accum, ctx->d_stats, ctx->tune);
         else k_raycast<false><<<persistent_grid(ctx, k_raycast<false>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_accum, ctx->d_stats, ctx->tune);
@@ -698,7 +706,7 @@ static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, const
     rd.pixel_list = d.primary_reuse ? ctx->d_pixel_list : nullptr;
     rd.prim = d.primary_reuse ? ctx->d_prim : nullptr;
     rd.n_slots = nwork; rd.slot_stride = nwork;
-    rd.log2_s = pl.log2_s;
+    rd.log2_s = log2_s;
     const int S = 1 << rd.log2_s;
     rd.sbuf = ctx->d_sbuf;
     const int agrid = (int)((nwork + 255) / 256 < (long long)ctx->sm_count * 8 ? (nwork + 255) / 256 : (long long)ctx->sm_count * 8);
@@ -721,8 +729,9 @@ static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, const
 
 // finish: the sums of all ranks onto rank 0 -- in place for a one-shot frame (sum1 == d_accum, no moments), into
 // rank 0's separate buffers for a progressive one (the ranks' running sums must survive the next reduce) -- then the
-// tone map with `inv` and, for a progressive frame after k samples, the noise estimate, both on rank 0
-static int enqueue_finish(sqt_ctx *ctx, long long npix, float inv, float *sum1, float *sum2, int k, uint32_t &nl) {
+// tone map with `inv` and, for a progressive frame after k samples, the noise estimate, both on rank 0; counts: the
+// per-pixel sample counts of an adaptive frame (nullptr: every pixel has k samples)
+static int enqueue_finish(sqt_ctx *ctx, long long npix, float inv, float *sum1, float *sum2, int k, const int *counts, uint32_t &nl) {
     cudaStream_t st = ctx->stream;
     CU(cudaEventRecord(ctx->ev[2], st));
     if (ctx->world > 1 && ctx->comm) {
@@ -738,10 +747,10 @@ static int enqueue_finish(sqt_ctx *ctx, long long npix, float inv, float *sum1, 
     }
     CU(cudaEventRecord(ctx->ev[3], st));
     if (ctx->rank == 0) {
-        k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(sum1, npix, inv, ctx->d_rgb8);
+        k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(sum1, npix, inv, ctx->d_rgb8, counts);
         CU(cudaGetLastError()); nl++;
         if (sum2) {
-            k_frame_noise_part<<<kNoiseBlocks, 256, 0, st>>>(sum1, sum2, npix * 3, k, ctx->d_noise);
+            k_frame_noise_part<<<kNoiseBlocks, 256, 0, st>>>(sum1, sum2, npix * 3, k, counts, ctx->d_noise);
             k_frame_noise<<<1, kNoiseBlocks, 0, st>>>(ctx->d_noise, npix * 3, k, ctx->d_noise + 2 * kNoiseBlocks);
             CU(cudaGetLastError()); nl += 2;
             CU(cudaMemcpyAsync(ctx->h_noise, ctx->d_noise + 2 * kNoiseBlocks, sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -756,8 +765,8 @@ static int enqueue_render(sqt_ctx *ctx, const RenderParams &d, bool count, const
     const long long npix = (long long)d.rows * d.cols;
     uint32_t nl = 0;
     int rc = enqueue_start(ctx, d, count, pl, nl); if (rc) return rc;
-    rc = enqueue_rounds(ctx, d, count, pl, pl.k0, pl.k1, nullptr, nl); if (rc) return rc;
-    rc = enqueue_finish(ctx, npix, 1.0f / (float)d.spp, ctx->d_accum, nullptr, d.spp, nl); if (rc) return rc;
+    rc = enqueue_rounds(ctx, d, count, pl.nwork, pl.log2_s, pl.k0, pl.k1, nullptr, nl); if (rc) return rc;
+    rc = enqueue_finish(ctx, npix, 1.0f / (float)d.spp, ctx->d_accum, nullptr, d.spp, nullptr, nl); if (rc) return rc;
     ctx->img_pixels = npix; ctx->img_spp = d.spp;
     *launches = nl;
     return SQT_OK;
@@ -869,7 +878,7 @@ extern "C" int sqt_tone_map(sqt_ctx *ctx, const float *mean_rgb, int64_t npix, u
     int rc = ensure_image(ctx, npix); if (rc) return rc;
     cudaStream_t st = ctx->stream;
     CU(cudaMemcpyAsync(ctx->d_accum, mean_rgb, (size_t)npix * 12, cudaMemcpyHostToDevice, st));
-    k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(ctx->d_accum, npix, 1.0f, ctx->d_rgb8);
+    k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(ctx->d_accum, npix, 1.0f, ctx->d_rgb8, nullptr);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(rgb8_out, ctx->d_rgb8, (size_t)npix * 3, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -879,22 +888,36 @@ extern "C" int sqt_tone_map(sqt_ctx *ctx, const float *mean_rgb, int64_t npix, u
 
 // ------------------------------------------------------------------------------ progressive frames
 // Every buffer a progressive frame needs beyond those of a one-shot render (prepare_render): the second moments, the
-// noise reduction's partial sums and, on rank 0 of a group, the reduced sums and moments.
+// noise reduction's partial sums, what sqt_render_retire needs (sample counts, the compaction's scratch) and, on rank 0
+// of a group, the reduced sums, moments and counts.  Neither sqt_render_advance nor sqt_render_retire allocates.
 static int ensure_progressive(sqt_ctx *ctx, long long npix) {
     if (!ctx->d_noise) CU(cudaMalloc(&ctx->d_noise, (2 * kNoiseBlocks + 1) * sizeof(double)));
     if (!ctx->h_noise) CU(cudaMallocHost(&ctx->h_noise, sizeof(double)));
+    if (!ctx->d_active) CU(cudaMalloc(&ctx->d_active, sizeof(long long)));
+    if (!ctx->h_active) CU(cudaMallocHost(&ctx->h_active, 2 * sizeof(long long)));
     if (npix > ctx->cap_m2) {
-        cudaFree(ctx->d_m2); ctx->d_m2 = nullptr; ctx->cap_m2 = 0;
+        cudaFree(ctx->d_m2); cudaFree(ctx->d_counts); cudaFree(ctx->d_list2); cudaFree(ctx->d_keep); cudaFree(ctx->d_tile);
+        ctx->d_m2 = nullptr; ctx->d_counts = nullptr; ctx->d_list2 = nullptr; ctx->d_keep = nullptr; ctx->d_tile = nullptr; ctx->cap_m2 = 0;
         CU(cudaMalloc(&ctx->d_m2, (size_t)npix * 12));
+        CU(cudaMalloc(&ctx->d_counts, (size_t)npix * sizeof(int)));
+        CU(cudaMalloc(&ctx->d_list2, (size_t)npix * sizeof(int)));
+        CU(cudaMalloc(&ctx->d_keep, (size_t)npix));
+        CU(cudaMalloc(&ctx->d_tile, (size_t)(npix / kRetireTile + 1) * sizeof(long long)));
         ctx->cap_m2 = npix;
     }
     if (ctx->world > 1 && ctx->comm && ctx->rank == 0 && npix > ctx->cap_red) {
-        cudaFree(ctx->d_red1); cudaFree(ctx->d_red2); ctx->d_red1 = ctx->d_red2 = nullptr; ctx->cap_red = 0;
+        cudaFree(ctx->d_red1); cudaFree(ctx->d_red2); cudaFree(ctx->d_redc); ctx->d_red1 = ctx->d_red2 = nullptr; ctx->d_redc = nullptr; ctx->cap_red = 0;
         CU(cudaMalloc(&ctx->d_red1, (size_t)npix * 12));
         CU(cudaMalloc(&ctx->d_red2, (size_t)npix * 12));
+        CU(cudaMalloc(&ctx->d_redc, (size_t)npix * sizeof(int)));
         ctx->cap_red = npix;
     }
     return SQT_OK;
+}
+// the sample counts of an adaptive frame (0 = samples_done): rank 0 of a group reads the sum over ranks
+static const int *frame_counts(sqt_ctx *ctx) {
+    if (!ctx->prog_adaptive) return nullptr;
+    return ctx->world > 1 && ctx->comm && ctx->rank == 0 ? ctx->d_redc : ctx->d_counts;
 }
 
 extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
@@ -926,6 +949,7 @@ extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_r
     rc = enqueue(); if (rc) return group_abort(ctx, rc);
     fill_stats(ctx, stats, nl);
     ctx->prog = true; ctx->prog_k = 0; ctx->prog_count = count; ctx->prog_d = d; ctx->prog_pl = pl;
+    ctx->prog_adaptive = false; ctx->prog_n = (long long)ctx->h_stats->n_hit; ctx->prog_total = 0;
     return SQT_OK;
 }
 
@@ -942,8 +966,14 @@ extern "C" int sqt_render_advance(sqt_ctx *ctx, int32_t n_samples, sqt_progress 
     const int32_t keys[3] = {rc ? 0 : k, rc ? 0 : spp, kb};
     rc = group_agree(ctx, rc, keys, 3); if (rc) return rc;
     const bool root = ctx->rank == 0;
-    if (k < spp) {
+    if (k < spp && ctx->prog_adaptive && ctx->prog_total == 0) {
+        ctx->prog_k = kb; ctx->img_spp = kb;            // every pixel has retired: nothing to trace, the image stays
+    } else if (k < spp) {
         const long long npix = (long long)d.rows * d.cols;
+        // an adaptive frame traces its active slots only, in rounds as wide as the sample buffer allows for them (at
+        // most the chunk: wider rounds would only skip items); results never depend on the round width
+        const long long nslots = ctx->prog_adaptive ? ctx->prog_n : ctx->prog_pl.nwork;
+        const int log2_s = ctx->prog_adaptive ? round_log2_s(nslots, kb - k, ctx->prog_pl.sbytes) : ctx->prog_pl.log2_s;
         cudaStream_t st = ctx->stream;
         uint32_t nl = 0;
         auto enqueue = [&]() -> int {
@@ -952,8 +982,9 @@ extern "C" int sqt_render_advance(sqt_ctx *ctx, int32_t n_samples, sqt_progress 
             CU(cudaMemsetAsync((char *)ctx->d_stats + offsetof(DeviceStats, work_next), 0, sizeof(DeviceStats) - offsetof(DeviceStats, work_next), st));
             CU(cudaEventRecord(ctx->ev[0], st));
             CU(cudaEventRecord(ctx->ev[1], st));
-            int r = enqueue_rounds(ctx, d, ctx->prog_count, ctx->prog_pl, k, kb, ctx->d_m2, nl); if (r) return r;
-            r = enqueue_finish(ctx, npix, 1.0f / (float)kb, frame_sums(ctx, false), frame_sums(ctx, true), kb, nl); if (r) return r;
+            int r = enqueue_rounds(ctx, d, ctx->prog_count, nslots, log2_s, k, kb, ctx->d_m2, nl); if (r) return r;
+            r = enqueue_finish(ctx, npix, 1.0f / (float)kb, frame_sums(ctx, false), frame_sums(ctx, true), kb, frame_counts(ctx), nl);
+            if (r) return r;
             CU(cudaStreamSynchronize(st));
             return SQT_OK;
         };
@@ -979,6 +1010,87 @@ extern "C" int sqt_download_moments(sqt_ctx *ctx, float *m2_out) {
     CU(cudaMemcpyAsync(ctx->h_accum, frame_sums(ctx, true), (size_t)npix * 12, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
     memcpy(m2_out, ctx->h_accum, (size_t)npix * 12);
+    return SQT_OK;
+}
+
+// ------------------------------------------------------------------------------ adaptive frames
+static uint32_t float_bits(float f) { uint32_t u; memcpy(&u, &f, 4); return u; }
+
+extern "C" int sqt_render_retire(sqt_ctx *ctx, const sqt_retire_params *rp, int64_t *active_out) {
+    if (!ctx) return SQT_E_INVALID;
+    cudaSetDevice(ctx->device);
+    int rc = SQT_OK;
+    if (!ctx->prog) rc = fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    else if (!rp) rc = fail(ctx, SQT_E_INVALID, "retire params are NULL");
+    else if (!ctx->prog_d.primary_reuse) rc = fail(ctx, SQT_E_UNSUPPORTED, "adaptive frames need primary reuse (not SQT_F_NO_PRIMARY_REUSE)");
+    else if (ctx->prog_k < 2) rc = fail(ctx, SQT_E_INVALID, "retire needs at least 2 samples per pixel (samples done: %d)", ctx->prog_k);
+    else if (rp->min_samples < 2) rc = fail(ctx, SQT_E_INVALID, "min_samples must be at least 2");
+    else if (!(rp->rel_tol >= 0.0f) || !(rp->abs_tol >= 0.0f)) rc = fail(ctx, SQT_E_INVALID, "tolerances must be non-negative numbers");
+    else if (rp->reserved) rc = fail(ctx, SQT_E_INVALID, "reserved must be 0");
+    const int k = ctx->prog_k, spp = ctx->prog_d.spp;
+    const int32_t keys[5] = {rc ? 0 : k, rc ? 0 : spp, rc ? 0 : (int32_t)float_bits(rp->rel_tol), rc ? 0 : (int32_t)float_bits(rp->abs_tol),
+                             rc ? 0 : rp->min_samples};
+    rc = group_agree(ctx, rc, keys, 5); if (rc) return rc;
+    const bool group = ctx->world > 1 && ctx->comm;
+    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    cudaStream_t st = ctx->stream;
+    // at k = spp, and before min_samples, nothing can retire: only the active total is reported
+    const bool test = k < spp && k >= rp->min_samples;
+    auto enqueue = [&]() -> int {
+        const long long n = ctx->prog_n;
+        if (test) {
+            if (!ctx->prog_adaptive) CU(cudaMemsetAsync(ctx->d_counts, 0, (size_t)npix * sizeof(int), st));
+            if (n > 0) {
+                const long long tiles = (n + kRetireTile - 1) / kRetireTile;
+                k_retire_mark<<<(int)tiles, 256, 0, st>>>(ctx->d_pixel_list, n, ctx->d_accum, ctx->d_m2, k,
+                                                          (double)rp->rel_tol, (double)rp->abs_tol, ctx->d_counts, ctx->d_keep, ctx->d_tile);
+                k_retire_scan<<<1, 1024, 0, st>>>(ctx->d_tile, tiles, &ctx->d_stats->n_hit);
+                k_retire_compact<<<(int)tiles, 256, 0, st>>>(ctx->d_pixel_list, n, ctx->d_keep, ctx->d_tile, ctx->d_list2);
+                CU(cudaGetLastError());
+                CU(cudaMemcpyAsync(ctx->d_pixel_list, ctx->d_list2, (size_t)n * sizeof(int), cudaMemcpyDeviceToDevice, st));
+            }
+            if (group) {
+                NcclApi *na = nccl_api();
+                // a pixel's count is non-zero on its owner only, so the sum is exact
+                ncclResult_t r = na->Reduce(ctx->d_counts, ctx->d_redc, (size_t)npix, kNcclInt32, kNcclSum, 0, ctx->comm, st);
+                if (r != 0) return fail(ctx, SQT_E_NCCL, "ncclReduce failed: %s", na->GetErrorString(r));
+            }
+        }
+        CU(cudaMemcpyAsync(&ctx->h_active[0], &ctx->d_stats->n_hit, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        if (group) {
+            NcclApi *na = nccl_api();
+            ncclResult_t r = na->AllReduce(&ctx->d_stats->n_hit, ctx->d_active, 1, kNcclInt64, kNcclSum, ctx->comm, st);
+            if (r != 0) return fail(ctx, SQT_E_NCCL, "ncclAllReduce failed: %s", na->GetErrorString(r));
+            CU(cudaMemcpyAsync(&ctx->h_active[1], ctx->d_active, sizeof(long long), cudaMemcpyDeviceToHost, st));
+        }
+        CU(cudaStreamSynchronize(st));
+        return SQT_OK;
+    };
+    rc = enqueue();
+    if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+    ctx->prog_n = ctx->h_active[0];
+    ctx->prog_total = group ? ctx->h_active[1] : ctx->h_active[0];
+    if (test) ctx->prog_adaptive = true;
+    if (active_out) *active_out = ctx->prog_total;
+    return SQT_OK;
+}
+
+extern "C" int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out) {
+    if (!ctx) return SQT_E_INVALID;
+    if (!ctx->prog) return fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    if (!counts_out) return fail(ctx, SQT_E_INVALID, "counts_out is NULL");
+    CU(cudaSetDevice(ctx->device));
+    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    const int k = ctx->prog_k;
+    if (const int *c = frame_counts(ctx)) {
+        int rc = ensure_host_image(ctx, npix); if (rc) return rc;
+        CU(cudaMemcpyAsync(ctx->h_accum, c, (size_t)npix * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        memcpy(counts_out, ctx->h_accum, (size_t)npix * sizeof(int));
+    } else {
+        memset(counts_out, 0, (size_t)npix * sizeof(int));
+    }
+    for (long long i = 0; i < npix; ++i) if (!counts_out[i]) counts_out[i] = k;
     return SQT_OK;
 }
 
@@ -1058,6 +1170,19 @@ extern "C" int sqt_render_advance_group(sqt_ctx **ctxs, int n, int32_t n_samples
     std::vector<std::thread> th;
     for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_advance(ctxs[i], n_samples, nullptr, nullptr); });
     rcs[0] = sqt_render_advance(ctxs[0], n_samples, progress, stats);
+    for (auto &t : th) t.join();
+    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
+    return SQT_OK;
+}
+
+extern "C" int sqt_render_retire_group(sqt_ctx **ctxs, int n, const sqt_retire_params *rp, int64_t *active_out) {
+    if (!ctxs || n < 1) return SQT_E_INVALID;
+    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
+    if (n == 1) return sqt_render_retire(ctxs[0], rp, active_out);
+    std::vector<int> rcs(n, 0);
+    std::vector<std::thread> th;
+    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_retire(ctxs[i], rp, nullptr); });
+    rcs[0] = sqt_render_retire(ctxs[0], rp, active_out);
     for (auto &t : th) t.join();
     for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
     return SQT_OK;

@@ -8,6 +8,7 @@
 //   k_accumulate       : adds a round's samples to the per-pixel sums in sample order (Lib.hs:88)
 //   k_accumulate_m2    : the same plus the per-pixel second moment (progressive frames)
 //   k_frame_noise_part, k_frame_noise : deterministic fp64 noise estimate of a progressive frame
+//   k_retire_mark, k_retire_scan, k_retire_compact : adaptive frames: convergence test + stable compaction of the pixel list
 //   k_raycast          : --cast mode (Lib.hs:141-151)
 //   k_tonemap          : mean + rgbFloatToPixelRGB (Lib.hs:88-104)
 //   k_leaf_records, k_check_materials, k_branch_tight, k_child_slabs, k_flag_slabs : scene upload (leaf records from the triangles; material
@@ -640,13 +641,16 @@ __device__ __forceinline__ void block_sum2(double &a, double &b, double *sh) {  
     }
     a = sh[0]; b = sh[blockDim.x];
 }
+// counts (adaptive frames): per-pixel sample counts n_p, 0 = n; nullptr = every value has n samples
 __global__ void __launch_bounds__(256) k_frame_noise_part(const float *__restrict__ s1, const float *__restrict__ s2, long long nval, int n,
-                                                          double *__restrict__ part) {
+                                                          const int *__restrict__ counts, double *__restrict__ part) {
     __shared__ double sh[512];
-    const double dn = (double)n;
+    const double dk = (double)n;
     double se2 = 0.0, smu = 0.0;
     const long long stride = (long long)kNoiseBlocks * 256;
     for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < nval; i += stride) {
+        const int c = counts ? counts[i / 3] : 0;
+        const double dn = c ? (double)c : dk;
         const double a = (double)s1[i], q = (double)s2[i];
         const double mu = a / dn;
         const double v = (q - a * mu) / (dn - 1.0);
@@ -669,6 +673,75 @@ __global__ void __launch_bounds__(kNoiseBlocks) k_frame_noise(const double *__re
     }
 }
 
+// Adaptive frames (sqt_render_retire): the convergence test over the active pixel list and its STABLE compaction, in
+// three steps of a fixed shape -- mark (the test per slot, the kept slots per tile), scan (tile offsets, one block),
+// compact -- so that the new list keeps the old order (neighbouring pixels stay in one warp, which keeps primary hits
+// coherent) and never depends on the SM count.
+constexpr int kRetireTile = 1024;                      // slots per block: 256 threads x 4 consecutive slots
+// exclusive prefix sum of v over the block (in thread order); *total gets the block's sum.  sh: 32 ints.
+template <class T>
+__device__ __forceinline__ T block_excl_scan(T v, T *sh, T &total) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    T x = v;
+    for (int o = 1; o < 32; o <<= 1) { const T y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+    if (lane == 31) sh[w] = x;
+    __syncthreads();
+    if (w == 0) {
+        T s = lane < nw ? sh[lane] : (T)0;
+        for (int o = 1; o < 32; o <<= 1) { const T y = __shfl_up_sync(0xffffffffu, s, o); if (lane >= o) s += y; }
+        if (lane < nw) sh[lane] = s;
+    }
+    __syncthreads();
+    const T r = (w ? sh[w - 1] : (T)0) + x - v;
+    total = sh[nw - 1];
+    __syncthreads();
+    return r;
+}
+// retire (counts[pixel] = k) the slots that pass retire_test; keep[slot] = 1 for the rest
+__global__ void __launch_bounds__(256) k_retire_mark(const int *__restrict__ list, long long n, const float *__restrict__ s1,
+                                                     const float *__restrict__ s2, int k, double rel_tol, double abs_tol,
+                                                     int *__restrict__ counts, uint8_t *__restrict__ keep, long long *__restrict__ tile_kept) {
+    __shared__ long long sh[32];
+    const long long base = (long long)blockIdx.x * kRetireTile + 4 * threadIdx.x;
+    long long kept = 0;
+    for (int j = 0; j < 4 && base + j < n; ++j) {
+        const long long pix = list[base + j];
+        const bool ret = retire_test(s1 + 3 * pix, s2 + 3 * pix, k, rel_tol, abs_tol);
+        if (ret) counts[pix] = k;
+        keep[base + j] = ret ? 0 : 1;
+        kept += ret ? 0 : 1;
+    }
+    long long total;
+    block_excl_scan(kept, sh, total);
+    if (threadIdx.x == 0) tile_kept[blockIdx.x] = total;
+}
+// tile_kept -> exclusive tile offsets (in place) and the new list length
+__global__ void __launch_bounds__(1024) k_retire_scan(long long *__restrict__ tile, long long ntiles, unsigned long long *__restrict__ n_out) {
+    __shared__ long long sh[32];
+    long long carry = 0;
+    for (long long b0 = 0; b0 < ntiles; b0 += blockDim.x) {
+        const long long i = b0 + threadIdx.x;
+        const long long v = i < ntiles ? tile[i] : 0;
+        long long total;
+        const long long ex = block_excl_scan(v, sh, total);
+        if (i < ntiles) tile[i] = carry + ex;
+        carry += total;
+    }
+    if (threadIdx.x == 0) *n_out = (unsigned long long)carry;
+}
+__global__ void __launch_bounds__(256) k_retire_compact(const int *__restrict__ list, long long n, const uint8_t *__restrict__ keep,
+                                                        const long long *__restrict__ tile_off, int *__restrict__ out) {
+    __shared__ long long sh[32];
+    const long long base = (long long)blockIdx.x * kRetireTile + 4 * threadIdx.x;
+    bool f[4];
+    long long kept = 0;
+    for (int j = 0; j < 4; ++j) { f[j] = base + j < n && keep[base + j]; kept += f[j] ? 1 : 0; }
+    long long total;
+    long long o = tile_off[blockIdx.x] + block_excl_scan(kept, sh, total);
+    for (int j = 0; j < 4; ++j)
+        if (f[j]) out[o++] = list[base + j];
+}
+
 template <bool COUNT>
 __global__ void __launch_bounds__(128) k_raycast(SceneView sc, RenderParams p, float *__restrict__ accum, DeviceStats *ds, Tune tn) {
     Counters cn = {};
@@ -679,12 +752,16 @@ __global__ void __launch_bounds__(128) k_raycast(SceneView sc, RenderParams p, f
 }
 
 // avg = (1 / fromIntegral sampleCount) *^ sum outcomes ; rgbFloatToPixelRGB avg   (Lib.hs:88-89)
+// counts (adaptive frames): a pixel with a non-zero count n_p uses 1.0f / (float)n_p (correctly rounded, -prec-div=true)
+// in place of inv_spp; nullptr = every pixel uses inv_spp
 __global__ void __launch_bounds__(256) k_tonemap(const float *__restrict__ accum, long long npix, float inv_spp,
-                                                 uint8_t *__restrict__ rgb8) {
+                                                 uint8_t *__restrict__ rgb8, const int *__restrict__ counts) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= npix) return;
+    const int c = counts ? counts[i] : 0;
+    const float inv = c ? 1.0f / (float)c : inv_spp;
     uint8_t o[3];
-    tone_map(XMUL(inv_spp, accum[3 * i]), XMUL(inv_spp, accum[3 * i + 1]), XMUL(inv_spp, accum[3 * i + 2]), o);
+    tone_map(XMUL(inv, accum[3 * i]), XMUL(inv, accum[3 * i + 1]), XMUL(inv, accum[3 * i + 2]), o);
     rgb8[3 * i] = o[0]; rgb8[3 * i + 1] = o[1]; rgb8[3 * i + 2] = o[2];
 }
 

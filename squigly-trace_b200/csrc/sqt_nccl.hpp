@@ -1,7 +1,7 @@
 // sqt_nccl.hpp -- NCCL reached through dlopen, so that the single-GPU path has no NCCL dependency at all.
-// Only the handful of entry points the render path uses (ncclReduce of the accumulation buffers -- and moments --,
-// a few-word ncclAllReduce with which the ranks agree that all of them can enter it, ncclCommAbort for the case
-// they cannot).
+// Only the handful of entry points the render path uses (ncclReduce of the accumulation buffers -- and moments and
+// sample counts --, a few-word ncclAllReduce with which the ranks agree that all of them can enter it or sum their
+// active pixels, ncclCommAbort for the case they cannot).
 #pragma once
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -39,4 +39,4 @@ inline NcclApi *nccl_api() {
 #undef SQT_SYM
     return &api;
 }
-static const int kNcclInt32 = 2, kNcclFloat32 = 7, kNcclSum = 0, kNcclMax = 2;
+static const int kNcclInt32 = 2, kNcclInt64 = 4, kNcclFloat32 = 7, kNcclSum = 0, kNcclMax = 2;

@@ -287,6 +287,25 @@ SQT_HD void accumulate_m2_slot(const RenderParams &p, const RoundInfo &rd, long 
     accum[3 * pixel] = sr; accum[3 * pixel + 1] = sg; accum[3 * pixel + 2] = sb;
     m2[3 * pixel] = qr; m2[3 * pixel + 1] = qg; m2[3 * pixel + 2] = qb;
 }
+// the convergence test of an adaptive frame (sqt_render_retire, include/sqt.h) for one pixel with sums s1 and second
+// moments s2 after n >= 2 samples, in fp64 and in the header's order; false whenever a NaN turns up on the way
+SQT_HD bool retire_test(const float *s1, const float *s2, int n, double rel_tol, double abs_tol) {
+    const double dn = (double)n;
+    double mu[3], v[3];
+    bool nan = false;
+    for (int c = 0; c < 3; ++c) {
+        const double a = (double)s1[c], q = (double)s2[c];
+        mu[c] = a / dn;
+        const double vc = (q - a * mu[c]) / (dn - 1.0);
+        nan = nan || vc != vc;
+        v[c] = vc > 0.0 ? vc : 0.0;
+    }
+    const double e2 = (v[0] + v[1] + v[2]) / dn, m = mu[0] + mu[1] + mu[2];
+    const double tr = rel_tol * m;
+    const double t = tr > abs_tol ? tr : abs_tol;
+    nan = nan || m != m || tr != tr;
+    return !nan && e2 < t * t;
+}
 
 // samples per pixel per round: the largest power of two <= spp whose sample buffer (slots * S * 12 B) fits the budget
 SQT_HD int round_log2_s(long long slots, int n_samples, long long budget_bytes) {

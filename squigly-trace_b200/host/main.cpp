@@ -1,11 +1,16 @@
 // main.cpp -- the squigly-trace command line (app/Main.hs:13-75) driving the B200 backend.
 // Flags follow the cmdargs record of the reference: -s/--samples, -d/--dimensions W,H, -p/--savepath,
-// --objpath, -c/--camerapath, --debug, --debugpath, --cast ; plus --bounces, --gpus, --corrected, --seed, --progress.
+// --objpath, -c/--camerapath, --debug, --debugpath, --cast ; plus --bounces, --gpus, --corrected, --seed, --progress,
+// --adaptive.
+#include <cctype>
 #include <chrono>
+#include <climits>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <ctime>
 #include <iostream>
+#include <vector>
 
 #include "squigly.hpp"
 
@@ -27,6 +32,8 @@ static void usage() {
                  "     --corrected         Width x height image with per-axis offsets (default: Lib.hs index convention)\n"
                  "     --seed=INT          RNG key\n"
                  "     --progress=INT      Render in chunks of INT samples, saving a preview after each\n"
+                 "     --adaptive=REL[,ABS[,MIN]]  With --progress: after each chunk stop sampling the pixels whose\n"
+                 "                         standard error is below max(REL * mean, ABS) (after at least MIN samples, default 16)\n"
                  "  -? --help              Display help message\n";
 }
 
@@ -35,6 +42,36 @@ static std::string showTime() {      // formatTime defaultTimeLocale "%T%P UTC"
     char buf[64];
     std::strftime(buf, sizeof buf, "%T%P UTC", std::gmtime(&t));
     return buf;
+}
+
+// --adaptive=REL[,ABS[,MIN]]: finite non-negative tolerances, MIN an integer >= 2
+static void parseAdaptive(const std::string &v, Settings &st) {
+    const std::runtime_error bad("Could not parse --adaptive=" + v + ", expected REL[,ABS[,MIN]] with non-negative numbers REL, ABS and an integer MIN >= 2");
+    std::vector<std::string> f;
+    for (size_t b = 0;;) {
+        const size_t c = v.find(',', b);
+        f.push_back(v.substr(b, c == std::string::npos ? std::string::npos : c - b));
+        if (c == std::string::npos) break;
+        b = c + 1;
+    }
+    if (f.size() > 3) throw bad;
+    for (const std::string &s : f)
+        if (s.empty() || !(std::isdigit((unsigned char)s[0]) || s[0] == '.')) throw bad;
+    auto tol = [&](const std::string &s) {
+        char *e = nullptr;
+        const double d = std::strtod(s.c_str(), &e);
+        if (*e || !std::isfinite(d) || d < 0.0 || !std::isfinite((float)d)) throw bad;
+        return (float)d;
+    };
+    st.adaptiveRel = tol(f[0]);
+    if (f.size() > 1) st.adaptiveAbs = tol(f[1]);
+    if (f.size() > 2) {
+        char *e = nullptr;
+        const long long m = std::strtoll(f[2].c_str(), &e, 10);
+        if (*e || m < 2 || m > INT_MAX) throw bad;
+        st.adaptiveMin = (int)m;
+    }
+    st.adaptive = true;
 }
 
 int main(int argc, char **argv) {
@@ -66,9 +103,11 @@ int main(int argc, char **argv) {
             else if (a == "--corrected") st.corrected = true;
             else if (a == "--seed") st.seed = std::stoull(need());
             else if (a == "--progress") { st.progress = std::stoi(need()); if (st.progress < 1) throw std::runtime_error("--progress must be at least 1"); }
+            else if (a == "--adaptive") parseAdaptive(need(), st);
             else if (a == "-?" || a == "--help") { usage(); return 0; }
             else throw std::runtime_error("Unknown flag: " + a);
         }
+        if (st.adaptive && st.progress < 1) throw std::runtime_error("--adaptive needs --progress=N");
         // main (Main.hs:35-47)
         const Camera cam = loadCamera(st.cameraPath);
         // loadBIH (Main.hs:63-75)

@@ -95,7 +95,9 @@ RenderReport renderToBuffer(const SceneBIH &scene, const Camera &cam, const Sett
 
 // --progress=N: the same frame as a progressive one (include/sqt.h) in chunks of N samples; after every chunk the preview
 // overwrites the save path and one line reports samples done, the noise estimate and the elapsed time.  The last image
-// is the one-shot frame bit for bit.
+// is the one-shot frame bit for bit.  --adaptive: after every chunk of at least 2 samples the converged pixels retire
+// (sqt_render_retire) and the line also reports the pixels still active; with zero tolerances nothing retires and the
+// image is the one-shot frame as well.
 static RenderReport renderProgressive(const SceneBIH &scene, const Camera &cam, const Settings &settings) {
     const sqt_render_params p = paramsFromSettings(settings);
     if (p.mode != 0) throw std::runtime_error("--progress needs path tracing (not --cast)");
@@ -108,14 +110,21 @@ static RenderReport renderProgressive(const SceneBIH &scene, const Camera &cam, 
     const auto t0 = std::chrono::steady_clock::now();
     g.check(0, sqt_render_begin_group(g.ctxs(), g.gpus(), &c, &p, &rep.stats), "sqt_render_begin");
     sqt_progress pr{0, p.spp, 0.0};
+    const sqt_retire_params rp{settings.adaptiveRel, settings.adaptiveAbs, settings.adaptiveMin, 0u};
+    int64_t active = -1;
     while (pr.samples_done < pr.samples_total) {
         sqt_stats st;
         g.check(0, sqt_render_advance_group(g.ctxs(), g.gpus(), settings.progress, &pr, &st), "sqt_render_advance");
         rep.stats.device_ms += st.device_ms; rep.stats.rays_traced += st.rays_traced; rep.stats.samples += st.samples;
+        if (settings.adaptive && pr.samples_done >= 2)
+            g.check(0, sqt_render_retire_group(g.ctxs(), g.gpus(), &rp, &active), "sqt_render_retire");
         g.check(0, sqt_download_image(g.ctx(0), img.data(), nullptr), "sqt_download_image");
         writeImage(settings.savePath, img.data(), rep.rows, rep.cols);
         const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-        std::printf("%d/%d samples  noise %.6g  %.3fs\n", pr.samples_done, pr.samples_total, pr.noise, sec);
+        if (settings.adaptive && active >= 0)
+            std::printf("%d/%d samples  noise %.6g  active %lld  %.3fs\n", pr.samples_done, pr.samples_total, pr.noise, (long long)active, sec);
+        else
+            std::printf("%d/%d samples  noise %.6g  %.3fs\n", pr.samples_done, pr.samples_total, pr.noise, sec);
         std::fflush(stdout);
     }
     return rep;

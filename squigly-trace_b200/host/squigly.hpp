@@ -103,6 +103,9 @@ struct Settings {
     bool corrected = false;     // false = Lib.hs:69-85 index convention verbatim (SURVEY A.5)
     uint64_t seed = 0;
     int progress = 0;           // > 0: render in chunks of this many samples, writing a preview after each
+    bool adaptive = false;      // with progress: retire converged pixels after every chunk (sqt_render_retire)
+    float adaptiveRel = 0.0f, adaptiveAbs = 0.0f;
+    int adaptiveMin = 16;
 };
 struct RenderReport { sqt_stats stats{}; int rows = 0, cols = 0; };
 // render :: Scene a -> Camera -> Settings -> IO ()   (Lib.hs:68-75): computes the image on the device(s) and writes it

@@ -29,7 +29,8 @@ ABI_SYMBOLS = [
     "sqt_render", "sqt_render_resident", "sqt_download_image", "sqt_tone_map", "sqt_comm_unique_id", "sqt_comm_init",
     "sqt_comm_init_all", "sqt_render_group", "sqt_measure_fp32_peak", "sqt_measure_l2_bandwidth", "sqt_device_info", "sqt_set_option", "sqt_upload_spheres",
     "sqt_upload_scene_group", "sqt_last_upload", "sqt_render_begin", "sqt_render_advance", "sqt_render_begin_group",
-    "sqt_render_advance_group", "sqt_download_moments",
+    "sqt_render_advance_group", "sqt_download_moments", "sqt_render_retire", "sqt_render_retire_group",
+    "sqt_download_sample_counts",
 ]
 
 
@@ -81,6 +82,13 @@ class Progress(C.Structure):
     _fields_ = [("samples_done", C.c_int32), ("samples_total", C.c_int32), ("noise", C.c_double)]
 
 
+class RetireParams(C.Structure):
+    _fields_ = [("rel_tol", C.c_float), ("abs_tol", C.c_float), ("min_samples", C.c_int32), ("reserved", C.c_uint32)]
+
+
+MIN_SAMPLES = 16       # default min_samples of render_retire and of the CLI's --adaptive
+
+
 NODE_DT = np.dtype([("lmax", "<f4"), ("rmin", "<f4"), ("a", "<u4"), ("b", "<u4")])
 TRI_DT = np.dtype([("v0", "<f4", 3), ("e1", "<f4", 3), ("e2", "<f4", 3), ("material", "<u4"), ("orig_index", "<u4"), ("pad", "<u4")])
 SPHERE_DT = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4"), ("pad", "<u4", 3)])
@@ -129,6 +137,9 @@ def b200():
         L.sqt_render_begin_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqt_render_advance_group.argtypes = [C.c_void_p, C.c_int, C.c_int32, C.c_void_p, C.c_void_p]
         L.sqt_download_moments.argtypes = [C.c_void_p, C.c_void_p]
+        L.sqt_render_retire.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sqt_render_retire_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+        L.sqt_download_sample_counts.argtypes = [C.c_void_p, C.c_void_p]
         L.sqt_device_info.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p]
         for name in ABI_SYMBOLS:
             if name not in ("sqt_last_error",):
@@ -344,6 +355,18 @@ class Context:
         self._ck(self.L.sqt_download_moments(self.h, _p(m2)), "sqt_download_moments")
         return m2
 
+    def render_retire(self, rel_tol, abs_tol=0.0, min_samples=MIN_SAMPLES):
+        """Retire the converged pixels of the progressive frame (include/sqt.h); returns the pixels still active."""
+        rp, act = RetireParams(rel_tol, abs_tol, min_samples, 0), C.c_int64()
+        self._ck(self.L.sqt_render_retire(self.h, C.byref(rp), C.byref(act)), "sqt_render_retire")
+        return act.value
+
+    def download_sample_counts(self, rows, cols):
+        """Samples in each pixel's sums: the k at which it retired, else samples_done."""
+        n = np.zeros((rows, cols), np.int32)
+        self._ck(self.L.sqt_download_sample_counts(self.h, _p(n)), "sqt_download_sample_counts")
+        return n
+
     def tone_map(self, mean_rgb):
         mean_rgb = np.ascontiguousarray(mean_rgb, np.float32)
         out = np.zeros(mean_rgb.shape, np.uint8)
@@ -418,6 +441,16 @@ class Group:
         if rc:
             raise SqtError("sqt_render_advance_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
         return dict(samples_done=pr.samples_done, samples_total=pr.samples_total, noise=pr.noise, stats=st.as_dict())
+
+    def render_retire(self, rel_tol, abs_tol=0.0, min_samples=MIN_SAMPLES):
+        rp, act = RetireParams(rel_tol, abs_tol, min_samples, 0), C.c_int64()
+        rc = self.L.sqt_render_retire_group(self.arr, len(self.ctxs), C.byref(rp), C.byref(act))
+        if rc:
+            raise SqtError("sqt_render_retire_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        return act.value
+
+    def download_sample_counts(self, rows, cols):
+        return self.ctxs[0].download_sample_counts(rows, cols)
 
     def close(self):
         for c in self.ctxs:
