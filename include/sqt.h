@@ -259,6 +259,55 @@ int sqt_render_retire(sqt_ctx *ctx, const sqt_retire_params *rp, int64_t *active
 int sqt_render_retire_group(sqt_ctx **ctxs, int n, const sqt_retire_params *rp, int64_t *active_out_or_null);
 int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out);   /* rows*cols n_p of the frame in progress (rank 0) */
 
+/* denoised previews of a progressive frame: an edge-aware a-trous wavelet filter guided by the primary hits and the
+ * per-pixel variance (the spatial part of SVGF: Dammertz et al. 2010, Schied et al. 2017) -------------------------------
+ *
+ * Valid inside a progressive frame after k = samples_done >= 2 samples.  These calls read the frame and change nothing
+ * of it: a later advance, retire, download or denoise behaves exactly as if they had not been made, and they never end
+ * the frame.  The filter is biased, as every denoiser is.  It does not demodulate albedo: the scenes have no textures,
+ * albedo is constant per material and no two materials are ever blended.
+ * All arithmetic is binary32, one explicit rounding per operation, no contraction, only + - * / sqrt min max (so a host
+ * build gives the device's bits); e2 is fp64 as in sqt_render_retire.
+ * Inputs per pixel p (rank 0, after k samples):
+ *   n_p    the pixel's sample count (sqt_download_sample_counts);  c_p = s1_p * (1.0f/(float)n_p) per channel, the values
+ *          the preview tone-maps;  v_p = (float)e2 with e2 of sqt_render_retire's test at n = n_p;  l_p = (c_r + c_g) + c_b
+ *   valid  the pixel has a primary hit; an invalid pixel's output is its input and it is never a neighbour
+ *   mat_p  material of the primary hit;  z_p = its t;  N_p its unit geometric normal: e1 x e2 (triangle) or hit - centre
+ *          (sphere, hit = o + t*d), divided by its length sqrt(N.N), negated when N.d > 0 (facing the camera ray)
+ *   mirror reflective >= 1: this integrator's perfect mirror; the primary features say nothing about what it shows, so
+ *          the pixel is passed through unfiltered
+ * Level i = 0 .. levels-1, step s = 2^i, for every valid non-mirror p, reading the previous level's (c, v):
+ *   g_p = sqrt(sum k_j v_j / sum k_j) over the 3x3 neighbours j of p (step 1, in the image, valid, same material, p
+ *         included), k = [1,2,1] x [1,2,1], rows outer
+ *   taps q = p + s*(dy, dx), dy outer, dx inner, both -2..2, skipping those outside the image, invalid or of another
+ *   material:  h = h1(dy)*h1(dx) with h1(-2..2) = 1/16, 1/4, 3/8, 1/4, 1/16 ;
+ *              x = |l_p - l_q| / (sigma_l*g_p + 1e-6f) + |z_p - z_q| / ((sigma_z*s)*z_p) ;
+ *              w_n = max(0, N_p.N_q) squared 7 times ;  r = 1/(1 + x*0.125f) squared 3 times  ((1 + x/8)^-8 ~ exp(-x)) ;
+ *              w = (h*w_n)*r, except at q = p: w = 9/64 exactly (so sum w > 0)
+ *   c'_p = sum w*c_q / sum w per channel,  v'_p = sum (w*w)*v_q / (sum w * sum w), every sum in tap order from +0
+ * Output: the last level's c (levels = 0: c itself, the preview's mean bit for bit) and its RGB8 = rgbFloatToPixelRGB(c)
+ * (the preview's RGB8 at levels = 0).  A fixed shape, one thread per pixel, no atomics: the bits never depend on the
+ * device, the SM count or the group size.
+ * sqt_denoise            rank 0 gets rows*cols*3 RGB8 bytes and floats (either may be NULL); the preview is not touched.
+ *                        Stats: device_ms, reduce_ms (the feature reduce), d2h_ms / d2h_bytes, kernel_launches.
+ * sqt_download_features  rank 0: surface (tri_out numbering: orig_index, n_tris + k for sphere k, -1 for no hit), depth
+ *                        (t) and the camera-facing normal N (rows*cols*3) the filter uses -- AOVs for an external denoiser
+ *                        too.  Any pointer may be NULL.
+ * Errors: SQT_E_INVALID outside a frame, k < 2, levels outside 0..8, a sigma that is not positive and finite, non-zero
+ * reserved; SQT_E_UNSUPPORTED for a frame begun with SQT_F_NO_PRIMARY_REUSE (it keeps no primary hits).
+ * In a group every rank makes the same calls (sqt_download_features included); ranks that disagree on k, the target spp,
+ * levels or the sigmas fail on every rank before anything runs.  The features reach rank 0 once per frame by a sum over
+ * ranks (each value is non-zero on its owner only, so the sum is exact), and rank 0 filters the sums, moments and counts
+ * it holds: a group result is bit-identical to one GPU's.  Whatever ends a frame drops its features. */
+typedef struct sqt_denoise_params {
+    int32_t levels;                      /* 0..8; 0 = the preview itself */
+    float sigma_l, sigma_z;              /* > 0, finite: luminance (in units of the prefiltered standard error) and depth */
+    uint32_t reserved;                   /* 0 */
+} sqt_denoise_params;                    /* 16 B */
+int sqt_denoise(sqt_ctx *ctx, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats_or_null);
+int sqt_denoise_group(sqt_ctx **ctxs, int n, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats_or_null);
+int sqt_download_features(sqt_ctx *ctx, int32_t *surface_out, float *depth_out, float *normal_out);
+
 /* measured roofline denominators on this device (microbenchmarks; see DESIGN.md) ------------- */
 int sqt_measure_fp32_peak(sqt_ctx *ctx, double *gops_per_s);     /* non-fused FADD/FMUL issue rate, Gop/s */
 int sqt_measure_l2_bandwidth(sqt_ctx *ctx, double *gb_per_s);    /* L2-resident 128-bit read bandwidth */

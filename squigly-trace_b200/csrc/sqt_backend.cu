@@ -86,6 +86,12 @@ struct sqt_ctx {
     long long prog_total = 0;           // active pixels of the whole frame after the last retire
     int *d_counts = nullptr, *d_redc = nullptr, *d_list2 = nullptr; uint8_t *d_keep = nullptr; long long *d_tile = nullptr;
     long long *d_active = nullptr, *h_active = nullptr;          // all-reduced active total; pinned (local, total)
+    long long prog_frame = 0;           // numbers the progressive frames of this context (sqt_render_begin)
+    // denoiser (sqt_denoise / sqt_download_features): features (N, z) and (surface + 1, key) -- on rank 0 of a group the sum
+    // over ranks --, the filter's ping-pong (c, v) buffers, the denoised mean and its RGB8
+    float4 *d_feat = nullptr, *d_dn[2] = {nullptr, nullptr}; int2 *d_sk = nullptr; float *d_dn_mean = nullptr; uint8_t *d_dn_rgb8 = nullptr;
+    long long cap_dn = 0;
+    long long dn_frame = -1;            // the progressive frame whose features d_feat / d_sk hold (-1: none)
     // group
     int rank = 0, world = 1;
     ncclComm_t comm = nullptr;
@@ -185,6 +191,7 @@ extern "C" int sqt_destroy(sqt_ctx *c) {
     cudaFree(c->d_org); cudaFree(c->d_dir); cudaFree(c->d_dist); cudaFree(c->d_point); cudaFree(c->d_tri);
     cudaFree(c->d_m2); cudaFree(c->d_red1); cudaFree(c->d_red2); cudaFree(c->d_noise);
     cudaFree(c->d_counts); cudaFree(c->d_redc); cudaFree(c->d_list2); cudaFree(c->d_keep); cudaFree(c->d_tile); cudaFree(c->d_active);
+    cudaFree(c->d_feat); cudaFree(c->d_sk); cudaFree(c->d_dn[0]); cudaFree(c->d_dn[1]); cudaFree(c->d_dn_mean); cudaFree(c->d_dn_rgb8);
     if (c->h_noise) cudaFreeHost(c->h_noise);
     if (c->h_active) cudaFreeHost(c->h_active);
     if (c->h_stats) cudaFreeHost(c->h_stats);
@@ -948,7 +955,7 @@ extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_r
     };
     rc = enqueue(); if (rc) return group_abort(ctx, rc);
     fill_stats(ctx, stats, nl);
-    ctx->prog = true; ctx->prog_k = 0; ctx->prog_count = count; ctx->prog_d = d; ctx->prog_pl = pl;
+    ctx->prog = true; ctx->prog_k = 0; ctx->prog_count = count; ctx->prog_d = d; ctx->prog_pl = pl; ctx->prog_frame++;
     ctx->prog_adaptive = false; ctx->prog_n = (long long)ctx->h_stats->n_hit; ctx->prog_total = 0;
     return SQT_OK;
 }
@@ -1094,6 +1101,149 @@ extern "C" int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out) {
     return SQT_OK;
 }
 
+// ------------------------------------------------------------------------------ denoiser
+// The denoiser reads the frame and writes only its own buffers: sums, moments, counts, the preview and the pixel list stay
+// as they are.  Its buffers are made on first use, before the group agreement, as ensure_progressive does.
+static int ensure_denoise(sqt_ctx *ctx, long long npix) {
+    if (npix <= ctx->cap_dn) return SQT_OK;
+    cudaFree(ctx->d_feat); cudaFree(ctx->d_sk); cudaFree(ctx->d_dn[0]); cudaFree(ctx->d_dn[1]); cudaFree(ctx->d_dn_mean); cudaFree(ctx->d_dn_rgb8);
+    ctx->d_feat = ctx->d_dn[0] = ctx->d_dn[1] = nullptr; ctx->d_sk = nullptr; ctx->d_dn_mean = nullptr; ctx->d_dn_rgb8 = nullptr;
+    ctx->cap_dn = 0; ctx->dn_frame = -1;
+    CU(cudaMalloc(&ctx->d_feat, (size_t)npix * sizeof(float4)));
+    CU(cudaMalloc(&ctx->d_sk, (size_t)npix * sizeof(int2)));
+    CU(cudaMalloc(&ctx->d_dn[0], (size_t)npix * sizeof(float4)));
+    CU(cudaMalloc(&ctx->d_dn[1], (size_t)npix * sizeof(float4)));
+    CU(cudaMalloc(&ctx->d_dn_mean, (size_t)npix * 12));
+    CU(cudaMalloc(&ctx->d_dn_rgb8, (size_t)npix * 3));
+    ctx->cap_dn = npix;
+    return SQT_OK;
+}
+
+// the checks every denoiser call shares, then the group agreement on (k, spp, levels, sigma bits); sqt_download_features
+// (download) agrees on levels = -1
+static int denoise_enter(sqt_ctx *ctx, bool download, int levels, float sigma_l, float sigma_z, uint32_t reserved, const char *what) {
+    if (download) { levels = -1; sigma_l = sigma_z = 0.0f; reserved = 0; }
+    int rc = SQT_OK;
+    if (!ctx->prog) rc = fail(ctx, SQT_E_INVALID, "%s: no progressive frame in progress", what);
+    else if (!ctx->prog_d.primary_reuse) rc = fail(ctx, SQT_E_UNSUPPORTED, "%s needs primary reuse (not SQT_F_NO_PRIMARY_REUSE)", what);
+    else if (ctx->prog_k < 2) rc = fail(ctx, SQT_E_INVALID, "%s needs at least 2 samples per pixel (samples done: %d)", what, ctx->prog_k);
+    else if (!download && (levels > 8 || levels < 0)) rc = fail(ctx, SQT_E_INVALID, "%s: levels must be in 0..8", what);
+    else if (!download && (!(sigma_l > 0.0f) || !(sigma_l < INFINITY) || !(sigma_z > 0.0f) || !(sigma_z < INFINITY)))
+        rc = fail(ctx, SQT_E_INVALID, "%s: sigma_l and sigma_z must be positive and finite", what);
+    else if (reserved) rc = fail(ctx, SQT_E_INVALID, "%s: reserved must be 0", what);
+    if (!rc) rc = ensure_denoise(ctx, (long long)ctx->prog_d.rows * ctx->prog_d.cols);
+    const int32_t keys[5] = {rc ? 0 : ctx->prog_k, rc ? 0 : ctx->prog_d.spp, rc ? 0 : levels, rc ? 0 : (int32_t)float_bits(sigma_l),
+                             rc ? 0 : (int32_t)float_bits(sigma_z)};
+    return group_agree(ctx, rc, keys, 5);
+}
+
+// enqueue the features of this frame unless they are there already: k_features on every rank, then (groups) their sum
+// onto rank 0 -- every value is non-zero on its owner only, so the sum is exact.  Events 0 .. 2 bracket it.
+static int enqueue_features(sqt_ctx *ctx, uint32_t &nl) {
+    cudaStream_t st = ctx->stream;
+    const RenderParams &d = ctx->prog_d;
+    const long long npix = (long long)d.rows * d.cols;
+    CU(cudaEventRecord(ctx->ev[0], st));
+    const bool need = ctx->dn_frame != ctx->prog_frame;
+    if (need) {
+        CU(cudaMemsetAsync(ctx->d_feat, 0, (size_t)npix * sizeof(float4), st));
+        CU(cudaMemsetAsync(ctx->d_sk, 0, (size_t)npix * sizeof(int2), st));
+        const long long nwork = ctx->prog_pl.nwork;
+        k_features<<<(int)((nwork + 255) / 256), 256, 0, st>>>(ctx->sc, d, ctx->d_prim, nwork, ctx->d_feat, ctx->d_sk);
+        CU(cudaGetLastError()); nl++;
+    }
+    CU(cudaEventRecord(ctx->ev[1], st));
+    if (need && ctx->world > 1 && ctx->comm) {
+        NcclApi *na = nccl_api();
+        ncclResult_t r = na->Reduce(ctx->d_sk, ctx->d_sk, (size_t)npix * 2, kNcclInt32, kNcclSum, 0, ctx->comm, st);
+        // (N, z) as int32 bit patterns: adding +0 to an owner's -0.0 in f32 would give +0.0, adding the integer 0 keeps every bit
+        if (r == 0) r = na->Reduce(ctx->d_feat, ctx->d_feat, (size_t)npix * 4, kNcclInt32, kNcclSum, 0, ctx->comm, st);
+        if (r != 0) return fail(ctx, SQT_E_NCCL, "ncclReduce failed: %s", na->GetErrorString(r));
+        nl += 2;
+    }
+    CU(cudaEventRecord(ctx->ev[2], st));
+    return SQT_OK;
+}
+
+static void denoise_stats(sqt_ctx *ctx, sqt_stats *s, uint32_t nl, uint64_t d2h_bytes) {
+    if (!s) return;
+    s->device_ms = ev_ms(ctx->ev[0], ctx->ev[3]);
+    s->reduce_ms = ev_ms(ctx->ev[1], ctx->ev[2]);
+    s->d2h_ms = ev_ms(ctx->ev[3], ctx->ev[4]);
+    s->d2h_bytes = d2h_bytes;
+    s->kernel_launches = nl;
+}
+
+extern "C" int sqt_denoise(sqt_ctx *ctx, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats) {
+    if (!ctx) return SQT_E_INVALID;
+    if (stats) memset(stats, 0, sizeof *stats);
+    cudaSetDevice(ctx->device);
+    int rc = dp ? denoise_enter(ctx, false, dp->levels, dp->sigma_l, dp->sigma_z, dp->reserved, "sqt_denoise")
+                : group_agree(ctx, fail(ctx, SQT_E_INVALID, "sqt_denoise: params are NULL"));
+    if (rc) return rc;
+    const RenderParams &d = ctx->prog_d;
+    const long long npix = (long long)d.rows * d.cols;
+    const bool root = ctx->rank == 0;
+    cudaStream_t st = ctx->stream;
+    uint32_t nl = 0;
+    auto enqueue = [&]() -> int {
+        int r = enqueue_features(ctx, nl); if (r) return r;
+        if (root) {
+            k_denoise_prep<<<(int)((npix + 255) / 256), 256, 0, st>>>(frame_sums(ctx, false), frame_sums(ctx, true), npix, ctx->prog_k,
+                                                                     frame_counts(ctx), ctx->d_dn[0], ctx->d_dn_mean);
+            CU(cudaGetLastError()); nl++;
+            const dim3 grid((unsigned)((d.cols + 15) / 16), (unsigned)((d.rows + 15) / 16));
+            for (int i = 0; i < dp->levels; ++i) {
+                k_denoise_level<<<grid, 256, 0, st>>>(ctx->d_dn[i & 1], ctx->d_feat, ctx->d_sk, d.rows, d.cols, 1 << i, dp->sigma_l, dp->sigma_z,
+                                                      ctx->d_dn[(i + 1) & 1], i + 1 == dp->levels ? ctx->d_dn_mean : nullptr);
+                CU(cudaGetLastError()); nl++;
+            }
+            k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(ctx->d_dn_mean, npix, 1.0f, ctx->d_dn_rgb8, nullptr);
+            CU(cudaGetLastError()); nl++;
+        }
+        CU(cudaEventRecord(ctx->ev[3], st));
+        if (root && rgb8_out) CU(cudaMemcpyAsync(rgb8_out, ctx->d_dn_rgb8, (size_t)npix * 3, cudaMemcpyDeviceToHost, st));
+        if (root && mean_out) CU(cudaMemcpyAsync(mean_out, ctx->d_dn_mean, (size_t)npix * 12, cudaMemcpyDeviceToHost, st));
+        CU(cudaEventRecord(ctx->ev[4], st));
+        CU(cudaStreamSynchronize(st));
+        return SQT_OK;
+    };
+    rc = enqueue();
+    if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+    ctx->dn_frame = ctx->prog_frame;
+    denoise_stats(ctx, stats, nl, root ? (uint64_t)npix * ((rgb8_out ? 3 : 0) + (mean_out ? 12 : 0)) : 0);
+    return SQT_OK;
+}
+
+extern "C" int sqt_download_features(sqt_ctx *ctx, int32_t *surface_out, float *depth_out, float *normal_out) {
+    if (!ctx) return SQT_E_INVALID;
+    cudaSetDevice(ctx->device);
+    int rc = denoise_enter(ctx, true, 0, 0.0f, 0.0f, 0u, "sqt_download_features");
+    if (rc) return rc;
+    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    uint32_t nl = 0;
+    auto enqueue = [&]() -> int {
+        int r = enqueue_features(ctx, nl); if (r) return r;
+        CU(cudaEventRecord(ctx->ev[3], ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        return SQT_OK;
+    };
+    rc = enqueue();
+    if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+    ctx->dn_frame = ctx->prog_frame;
+    if (ctx->rank != 0 || (!surface_out && !depth_out && !normal_out)) return SQT_OK;
+    std::vector<float4> f((size_t)npix);
+    std::vector<int2> sk((size_t)npix);
+    CU(cudaMemcpy(f.data(), ctx->d_feat, (size_t)npix * sizeof(float4), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(sk.data(), ctx->d_sk, (size_t)npix * sizeof(int2), cudaMemcpyDeviceToHost));
+    for (long long i = 0; i < npix; ++i) {
+        if (surface_out) surface_out[i] = sk[i].x - 1;
+        if (depth_out) depth_out[i] = f[i].w;
+        if (normal_out) { normal_out[3 * i] = f[i].x; normal_out[3 * i + 1] = f[i].y; normal_out[3 * i + 2] = f[i].z; }
+    }
+    return SQT_OK;
+}
+
 // ------------------------------------------------------------------------------ group (NCCL)
 extern "C" int sqt_comm_unique_id(uint8_t id_out[SQT_COMM_ID_BYTES]) {
     NcclApi *na = nccl_api();
@@ -1183,6 +1333,19 @@ extern "C" int sqt_render_retire_group(sqt_ctx **ctxs, int n, const sqt_retire_p
     std::vector<std::thread> th;
     for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_retire(ctxs[i], rp, nullptr); });
     rcs[0] = sqt_render_retire(ctxs[0], rp, active_out);
+    for (auto &t : th) t.join();
+    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
+    return SQT_OK;
+}
+
+extern "C" int sqt_denoise_group(sqt_ctx **ctxs, int n, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats) {
+    if (!ctxs || n < 1) return SQT_E_INVALID;
+    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
+    if (n == 1) return sqt_denoise(ctxs[0], dp, rgb8_out, mean_out, stats);
+    std::vector<int> rcs(n, 0);
+    std::vector<std::thread> th;
+    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_denoise(ctxs[i], dp, nullptr, nullptr, nullptr); });
+    rcs[0] = sqt_denoise(ctxs[0], dp, rgb8_out, mean_out, stats);
     for (auto &t : th) t.join();
     for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
     return SQT_OK;

@@ -9,6 +9,7 @@
 //   k_accumulate_m2    : the same plus the per-pixel second moment (progressive frames)
 //   k_frame_noise_part, k_frame_noise : deterministic fp64 noise estimate of a progressive frame
 //   k_retire_mark, k_retire_scan, k_retire_compact : adaptive frames: convergence test + stable compaction of the pixel list
+//   k_features, k_denoise_prep, k_denoise_level : sqt_denoise: primary-hit features, the filter's inputs, one a-trous level
 //   k_raycast          : --cast mode (Lib.hs:141-151)
 //   k_tonemap          : mean + rgbFloatToPixelRGB (Lib.hs:88-104)
 //   k_leaf_records, k_check_materials, k_branch_tight, k_child_slabs, k_flag_slabs : scene upload (leaf records from the triangles; material
@@ -19,7 +20,7 @@
 #include <cooperative_groups.h>
 #include <type_traits>
 
-#include "sqt_paths.cuh"
+#include "sqt_denoise.cuh"
 
 namespace cg = cooperative_groups;
 using namespace sqt;
@@ -740,6 +741,45 @@ __global__ void __launch_bounds__(256) k_retire_compact(const int *__restrict__ 
     long long o = tile_off[blockIdx.x] + block_excl_scan(kept, sh, total);
     for (int j = 0; j < 4; ++j)
         if (f[j]) out[o++] = list[base + j];
+}
+
+// sqt_denoise (sqt_denoise.cuh): the features of this rank's pixels (ownership as work_to_pixel defines it) from the
+// primary hits; the caller zero-fills both buffers, so a pixel owned elsewhere stays 0 and a sum over ranks is exact.
+// sk = (tri_out numbering of the surface + 1, denoise_key), 0 for no hit.
+__global__ void __launch_bounds__(256) k_features(SceneView sc, RenderParams p, const int2 *__restrict__ prim, long long nwork,
+                                                  float4 *__restrict__ feat, int2 *__restrict__ sk) {
+    const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= nwork) return;
+    const long long pix = work_to_pixel(p, w);
+    if (pix < 0) return;
+    const int2 h = prim[pix];
+    if (h.x < 0) return;
+    const Ray r = make_ray(p, (int)(pix / p.cols), (int)(pix % p.cols));
+    feat[pix] = primary_feature(sc, r, h.x, __uint_as_float((uint32_t)h.y));
+    const int orig = (uint32_t)h.x >= sc.n_tris ? h.x : (int)__float_as_uint(sc.tris[3 * (size_t)h.x + 2].z);
+    sk[pix] = make_int2(orig + 1, denoise_key(sc, h.x));
+}
+// the filter's input (c, v) per pixel after k samples (counts: an adaptive frame's n_p, 0 = k; nullptr = k everywhere),
+// also written packed as the mean of level 0
+__global__ void __launch_bounds__(256) k_denoise_prep(const float *__restrict__ s1, const float *__restrict__ s2, long long npix, int k,
+                                                      const int *__restrict__ counts, float4 *__restrict__ cv, float *__restrict__ mean) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= npix) return;
+    const int c = counts ? counts[i] : 0;
+    const float4 o = denoise_input(s1 + 3 * i, s2 + 3 * i, c ? c : k);
+    cv[i] = o;
+    mean[3 * i] = o.x; mean[3 * i + 1] = o.y; mean[3 * i + 2] = o.z;
+}
+// one level, step s: one thread per pixel in 16 x 16 tiles.  mean (last level only): the packed c'
+__global__ void __launch_bounds__(256) k_denoise_level(const float4 *__restrict__ cv_in, const float4 *__restrict__ feat, const int2 *__restrict__ sk,
+                                                       int rows, int cols, int s, float sigma_l, float sigma_z,
+                                                       float4 *__restrict__ cv_out, float *__restrict__ mean) {
+    const int x = blockIdx.x * 16 + (threadIdx.x & 15), y = blockIdx.y * 16 + (threadIdx.x >> 4);
+    if (x >= cols || y >= rows) return;
+    const float4 o = denoise_level_pixel(cv_in, feat, sk, rows, cols, y, x, s, sigma_l, sigma_z);
+    const long long p = (long long)y * cols + x;
+    cv_out[p] = o;
+    if (mean) { mean[3 * p] = o.x; mean[3 * p + 1] = o.y; mean[3 * p + 2] = o.z; }
 }
 
 template <bool COUNT>

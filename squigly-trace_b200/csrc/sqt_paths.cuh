@@ -287,9 +287,10 @@ SQT_HD void accumulate_m2_slot(const RenderParams &p, const RoundInfo &rd, long 
     accum[3 * pixel] = sr; accum[3 * pixel + 1] = sg; accum[3 * pixel + 2] = sb;
     m2[3 * pixel] = qr; m2[3 * pixel + 1] = qg; m2[3 * pixel + 2] = qb;
 }
-// the convergence test of an adaptive frame (sqt_render_retire, include/sqt.h) for one pixel with sums s1 and second
-// moments s2 after n >= 2 samples, in fp64 and in the header's order; false whenever a NaN turns up on the way
-SQT_HD bool retire_test(const float *s1, const float *s2, int n, double rel_tol, double abs_tol) {
+// the per-pixel error terms of include/sqt.h for sums s1 and second moments s2 after n >= 2 samples, in fp64 and in the
+// header's order: e2 (the squared standard error) and m (the mean's channel sum); returns true when a channel's variance
+// is NaN.  Shared by the convergence test and the denoiser's variance.
+SQT_HD bool pixel_error(const float *s1, const float *s2, int n, double &e2, double &m) {
     const double dn = (double)n;
     double mu[3], v[3];
     bool nan = false;
@@ -300,7 +301,14 @@ SQT_HD bool retire_test(const float *s1, const float *s2, int n, double rel_tol,
         nan = nan || vc != vc;
         v[c] = vc > 0.0 ? vc : 0.0;
     }
-    const double e2 = (v[0] + v[1] + v[2]) / dn, m = mu[0] + mu[1] + mu[2];
+    e2 = (v[0] + v[1] + v[2]) / dn; m = mu[0] + mu[1] + mu[2];
+    return nan;
+}
+// the convergence test of an adaptive frame (sqt_render_retire, include/sqt.h) for one pixel; false whenever a NaN turns
+// up on the way
+SQT_HD bool retire_test(const float *s1, const float *s2, int n, double rel_tol, double abs_tol) {
+    double e2, m;
+    bool nan = pixel_error(s1, s2, n, e2, m);
     const double tr = rel_tol * m;
     const double t = tr > abs_tol ? tr : abs_tol;
     nan = nan || m != m || tr != tr;

@@ -1,7 +1,7 @@
 // main.cpp -- the squigly-trace command line (app/Main.hs:13-75) driving the B200 backend.
 // Flags follow the cmdargs record of the reference: -s/--samples, -d/--dimensions W,H, -p/--savepath,
 // --objpath, -c/--camerapath, --debug, --debugpath, --cast ; plus --bounces, --gpus, --corrected, --seed, --progress,
-// --adaptive.
+// --adaptive, --denoise.
 #include <cctype>
 #include <chrono>
 #include <climits>
@@ -34,6 +34,8 @@ static void usage() {
                  "     --progress=INT      Render in chunks of INT samples, saving a preview after each\n"
                  "     --adaptive=REL[,ABS[,MIN]]  With --progress: after each chunk stop sampling the pixels whose\n"
                  "                         standard error is below max(REL * mean, ABS) (after at least MIN samples, default 16)\n"
+                 "     --denoise[=LEVELS]  With --progress: also save <savepath stem>-denoised.png after each chunk, filtered\n"
+                 "                         with LEVELS (0..8, default 5) levels of the edge-aware denoiser\n"
                  "  -? --help              Display help message\n";
 }
 
@@ -104,10 +106,19 @@ int main(int argc, char **argv) {
             else if (a == "--seed") st.seed = std::stoull(need());
             else if (a == "--progress") { st.progress = std::stoi(need()); if (st.progress < 1) throw std::runtime_error("--progress must be at least 1"); }
             else if (a == "--adaptive") parseAdaptive(need(), st);
+            else if (a == "--denoise") {
+                st.denoise = 5;
+                if (has_val) {
+                    if (val.empty() || val.size() > 1 || !std::isdigit((unsigned char)val[0]) || val[0] > '8')
+                        throw std::runtime_error("Could not parse --denoise=" + val + ", expected LEVELS in 0..8");
+                    st.denoise = val[0] - '0';
+                }
+            }
             else if (a == "-?" || a == "--help") { usage(); return 0; }
             else throw std::runtime_error("Unknown flag: " + a);
         }
         if (st.adaptive && st.progress < 1) throw std::runtime_error("--adaptive needs --progress=N");
+        if (st.denoise >= 0 && st.progress < 1) throw std::runtime_error("--denoise needs --progress=N");
         // main (Main.hs:35-47)
         const Camera cam = loadCamera(st.cameraPath);
         // loadBIH (Main.hs:63-75)

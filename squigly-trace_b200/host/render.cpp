@@ -97,7 +97,14 @@ RenderReport renderToBuffer(const SceneBIH &scene, const Camera &cam, const Sett
 // overwrites the save path and one line reports samples done, the noise estimate and the elapsed time.  The last image
 // is the one-shot frame bit for bit.  --adaptive: after every chunk of at least 2 samples the converged pixels retire
 // (sqt_render_retire) and the line also reports the pixels still active; with zero tolerances nothing retires and the
-// image is the one-shot frame as well.
+// image is the one-shot frame as well.  --denoise: after every chunk of at least 2 samples the denoised preview
+// (sqt_denoise) also goes to <savepath stem>-denoised.png; the plain preview is not affected.
+static std::string denoisedPath(const std::string &path) {
+    const size_t slash = path.find_last_of('/'), dot = path.find_last_of('.');
+    const size_t stem = dot != std::string::npos && (slash == std::string::npos || dot > slash) ? dot : path.size();
+    return path.substr(0, stem) + "-denoised" + path.substr(stem);
+}
+
 static RenderReport renderProgressive(const SceneBIH &scene, const Camera &cam, const Settings &settings) {
     const sqt_render_params p = paramsFromSettings(settings);
     if (p.mode != 0) throw std::runtime_error("--progress needs path tracing (not --cast)");
@@ -120,6 +127,11 @@ static RenderReport renderProgressive(const SceneBIH &scene, const Camera &cam, 
             g.check(0, sqt_render_retire_group(g.ctxs(), g.gpus(), &rp, &active), "sqt_render_retire");
         g.check(0, sqt_download_image(g.ctx(0), img.data(), nullptr), "sqt_download_image");
         writeImage(settings.savePath, img.data(), rep.rows, rep.cols);
+        if (settings.denoise >= 0 && pr.samples_done >= 2) {
+            const sqt_denoise_params dp{settings.denoise, 4.0f, 0.05f, 0u};
+            g.check(0, sqt_denoise_group(g.ctxs(), g.gpus(), &dp, img.data(), nullptr, nullptr), "sqt_denoise");
+            writeImage(denoisedPath(settings.savePath), img.data(), rep.rows, rep.cols);
+        }
         const double sec = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         if (settings.adaptive && active >= 0)
             std::printf("%d/%d samples  noise %.6g  active %lld  %.3fs\n", pr.samples_done, pr.samples_total, pr.noise, (long long)active, sec);

@@ -106,6 +106,7 @@ struct Settings {
     bool adaptive = false;      // with progress: retire converged pixels after every chunk (sqt_render_retire)
     float adaptiveRel = 0.0f, adaptiveAbs = 0.0f;
     int adaptiveMin = 16;
+    int denoise = -1;           // with progress: >= 0 also writes <stem>-denoised.png after every chunk (sqt_denoise levels)
 };
 struct RenderReport { sqt_stats stats{}; int rows = 0, cols = 0; };
 // render :: Scene a -> Camera -> Settings -> IO ()   (Lib.hs:68-75): computes the image on the device(s) and writes it

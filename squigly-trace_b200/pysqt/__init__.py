@@ -30,7 +30,7 @@ ABI_SYMBOLS = [
     "sqt_comm_init_all", "sqt_render_group", "sqt_measure_fp32_peak", "sqt_measure_l2_bandwidth", "sqt_device_info", "sqt_set_option", "sqt_upload_spheres",
     "sqt_upload_scene_group", "sqt_last_upload", "sqt_render_begin", "sqt_render_advance", "sqt_render_begin_group",
     "sqt_render_advance_group", "sqt_download_moments", "sqt_render_retire", "sqt_render_retire_group",
-    "sqt_download_sample_counts",
+    "sqt_download_sample_counts", "sqt_denoise", "sqt_denoise_group", "sqt_download_features",
 ]
 
 
@@ -89,6 +89,13 @@ class RetireParams(C.Structure):
 MIN_SAMPLES = 16       # default min_samples of render_retire and of the CLI's --adaptive
 
 
+class DenoiseParams(C.Structure):
+    _fields_ = [("levels", C.c_int32), ("sigma_l", C.c_float), ("sigma_z", C.c_float), ("reserved", C.c_uint32)]
+
+
+DENOISE_LEVELS, DENOISE_SIGMA_L, DENOISE_SIGMA_Z = 5, 4.0, 0.05     # defaults of denoise and of the CLI's --denoise
+
+
 NODE_DT = np.dtype([("lmax", "<f4"), ("rmin", "<f4"), ("a", "<u4"), ("b", "<u4")])
 TRI_DT = np.dtype([("v0", "<f4", 3), ("e1", "<f4", 3), ("e2", "<f4", 3), ("material", "<u4"), ("orig_index", "<u4"), ("pad", "<u4")])
 SPHERE_DT = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4"), ("pad", "<u4", 3)])
@@ -140,6 +147,9 @@ def b200():
         L.sqt_render_retire.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqt_render_retire_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         L.sqt_download_sample_counts.argtypes = [C.c_void_p, C.c_void_p]
+        L.sqt_denoise.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sqt_denoise_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sqt_download_features.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqt_device_info.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p]
         for name in ABI_SYMBOLS:
             if name not in ("sqt_last_error",):
@@ -266,6 +276,7 @@ class Context:
             raise SqtError("sqt_create failed (%d): %s" % (rc, L.sqt_last_error(None).decode()))
         self.h = h
         self.L = L
+        self._shape = (0, 0)        # rows, cols of the progressive frame begun last
 
     def close(self):
         if self.h:
@@ -341,6 +352,7 @@ class Context:
         """Start a progressive frame (include/sqt.h): checks, allocations and the primary pass; returns the stats."""
         cam = camera_struct(cam12)
         st = Stats()
+        self._shape = (params.rows, params.cols)
         self._ck(self.L.sqt_render_begin(self.h, C.byref(cam), C.byref(params), C.byref(st)), "sqt_render_begin")
         return st.as_dict()
 
@@ -366,6 +378,23 @@ class Context:
         n = np.zeros((rows, cols), np.int32)
         self._ck(self.L.sqt_download_sample_counts(self.h, _p(n)), "sqt_download_sample_counts")
         return n
+
+    def denoise(self, levels=DENOISE_LEVELS, sigma_l=DENOISE_SIGMA_L, sigma_z=DENOISE_SIGMA_Z):
+        """Denoised preview of the progressive frame (include/sqt.h): returns rgb8, mean and stats.  The frame is unchanged."""
+        rows, cols = self._shape
+        dp, st = DenoiseParams(levels, sigma_l, sigma_z, 0), Stats()
+        rgb8 = np.zeros((rows, cols, 3), np.uint8)
+        mean = np.zeros((rows, cols, 3), np.float32)
+        self._ck(self.L.sqt_denoise(self.h, C.byref(dp), _p(rgb8), _p(mean), C.byref(st)), "sqt_denoise")
+        return dict(rgb8=rgb8, mean=mean, stats=st.as_dict())
+
+    def download_features(self, rows, cols):
+        """Primary-hit AOVs of the progressive frame: surface (tri_out numbering, -1 = no hit), depth t, camera-facing normal."""
+        surface = np.zeros((rows, cols), np.int32)
+        depth = np.zeros((rows, cols), np.float32)
+        normal = np.zeros((rows, cols, 3), np.float32)
+        self._ck(self.L.sqt_download_features(self.h, _p(surface), _p(depth), _p(normal)), "sqt_download_features")
+        return dict(surface=surface, depth=depth, normal=normal)
 
     def tone_map(self, mean_rgb):
         mean_rgb = np.ascontiguousarray(mean_rgb, np.float32)
@@ -409,6 +438,7 @@ class Group:
         if rc:
             raise SqtError("sqt_comm_init_all failed (%d): %s" % (rc, self.ctxs[0].last_error()))
         self.L = L
+        self._shape = (0, 0)
 
     def upload(self, scene):
         d = scene.desc() if hasattr(scene, "desc") else scene
@@ -430,6 +460,7 @@ class Group:
     def render_begin(self, cam12, params):
         cam = camera_struct(cam12)
         st = Stats()
+        self._shape = (params.rows, params.cols)
         rc = self.L.sqt_render_begin_group(self.arr, len(self.ctxs), C.byref(cam), C.byref(params), C.byref(st))
         if rc:
             raise SqtError("sqt_render_begin_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
@@ -451,6 +482,36 @@ class Group:
 
     def download_sample_counts(self, rows, cols):
         return self.ctxs[0].download_sample_counts(rows, cols)
+
+    def denoise(self, levels=DENOISE_LEVELS, sigma_l=DENOISE_SIGMA_L, sigma_z=DENOISE_SIGMA_Z):
+        rows, cols = self._shape
+        dp, st = DenoiseParams(levels, sigma_l, sigma_z, 0), Stats()
+        rgb8 = np.zeros((rows, cols, 3), np.uint8)
+        mean = np.zeros((rows, cols, 3), np.float32)
+        rc = self.L.sqt_denoise_group(self.arr, len(self.ctxs), C.byref(dp), _p(rgb8), _p(mean), C.byref(st))
+        if rc:
+            raise SqtError("sqt_denoise_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        return dict(rgb8=rgb8, mean=mean, stats=st.as_dict())
+
+    def download_features(self, rows, cols):
+        """Every rank takes part (the first call of a frame sums the features onto rank 0); rank 0's result is returned."""
+        import threading
+        res, errs = [None] * len(self.ctxs), []
+
+        def run(i):
+            try:
+                res[i] = self.ctxs[i].download_features(rows, cols)
+            except SqtError as e:
+                errs.append(e)
+        th = [threading.Thread(target=run, args=(i,)) for i in range(1, len(self.ctxs))]
+        for t in th:
+            t.start()
+        run(0)
+        for t in th:
+            t.join()
+        if errs:
+            raise errs[0]
+        return res[0]
 
     def close(self):
         for c in self.ctxs:

@@ -1,5 +1,5 @@
 """Smallest end-to-end exercise of every kernel, for compute-sanitizer (one tool per gpurun call):
-intersect batch, render with both path schedulers, cast mode, spheres, tone map, multi-round accumulation, a progressive frame."""
+intersect batch, render with both path schedulers, cast mode, spheres, tone map, multi-round accumulation, a progressive frame, the denoiser."""
 import os
 import sys
 
@@ -30,5 +30,7 @@ for pool in ("2", "0"):
     for n in (1, 2, 3):
         ctx.render_advance(n)
     ctx.download_moments(48, 64)
+    ctx.denoise(3)                              # k_features, k_denoise_prep, k_denoise_level
+    ctx.download_features(48, 64)
     print("pool", pool, "ok", int((tri >= 0).sum()), out["stats"]["rays_traced"], out3["stats"]["rays_traced"])
     ctx.close()
