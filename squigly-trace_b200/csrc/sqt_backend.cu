@@ -14,6 +14,7 @@
 #include <chrono>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/sqt.h"
@@ -22,8 +23,46 @@
 #include "sqt_nccl.hpp"
 
 // ============================================================================== context
+// A grow-only allocation of `cap` elements of T in device memory or, PINNED, in page-locked host memory; the destructor
+// frees it.  ensure(n) reallocates only when n exceeds the capacity, reset(n) always, at exactly n (0: free only).  The
+// contents are never kept.  On a failed allocation the buffer is empty, so the next ensure tries again.
+template <class T, bool PINNED = false>
+struct Buffer {
+    T *p = nullptr;
+    size_t cap = 0;
+    Buffer() = default;
+    Buffer(Buffer &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    Buffer &operator=(Buffer &&o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+    ~Buffer() { reset(0); }
+    operator T *() const { return p; }
+    T *operator->() const { return p; }
+    cudaError_t ensure(size_t n) { return n <= cap ? cudaSuccess : reset(n); }
+    cudaError_t reset(size_t n) {
+        if (p) { if (PINNED) cudaFreeHost(p); else cudaFree(p); }
+        p = nullptr; cap = 0;
+        if (n == 0) return cudaSuccess;
+        void *q = nullptr;
+        const cudaError_t e = PINNED ? cudaMallocHost(&q, n * sizeof(T)) : cudaMalloc(&q, n * sizeof(T));
+        if (e == cudaSuccess) { p = (T *)q; cap = n; }
+        return e;
+    }
+};
+template <class T> using Pinned = Buffer<T, true>;
+
 // launch shape of a frame's sample rounds (prepare_render): work items, this rank's sample range, S = 1 << log2_s
 struct RenderPlan { long long nwork = 0; int k0 = 0, k1 = 0, log2_s = 0; long long sbytes = 0; };
+
+// a progressive frame (sqt_render_begin until whatever ends it, include/sqt.h): what the frame needs between two calls
+struct ProgFrame {
+    bool on = false;                    // a progressive frame is in progress
+    int k = 0;                          // samples [0, k) are in the sums
+    bool count = false;
+    RenderParams d = {};
+    RenderPlan pl;
+    bool adaptive = false;              // retire has run in this frame: d_pixel_list / n_hit hold the active pixels
+    long long n = 0;                    // this rank's active slots (the primary pass's hit count until the first retire)
+    long long total = 0;                // active pixels of the whole frame after the last retire
+};
 
 struct sqt_ctx {
     int device = 0, sm_count = 0, cc_major = 0, cc_minor = 0;
@@ -34,34 +73,31 @@ struct sqt_ctx {
     // scene
     bool has_scene = false;
     SceneView sc = {};
-    float4 *d_slabs = nullptr, *d_tight = nullptr; uint32_t *d_levels = nullptr;          // subtree slabs (+ upload scratch)
-    float4 *d_nodes = nullptr, *d_boxes = nullptr, *d_tris = nullptr, *d_mats = nullptr, *d_leaves = nullptr, *d_spheres = nullptr;
-    float4 *d_sph_nodes = nullptr; uint32_t *d_sph_order = nullptr; int sphere_bvh = 1;      // extension: hierarchy over the spheres
-    uint2 *d_ranges = nullptr;          // (first, count) per leaf, input of k_leaf_records
-    uint32_t *d_flag = nullptr;         // material check result
-    size_t cap_branches = 0, cap_leaves = 0, cap_tris = 0, cap_mats = 0;     // allocation sizes (records), reused across uploads
+    Buffer<float4> d_slabs, d_tight; Buffer<uint32_t> d_levels;                   // subtree slabs (+ upload scratch)
+    Buffer<float4> d_nodes, d_boxes, d_tris, d_mats, d_leaves, d_spheres;
+    Buffer<float4> d_sph_nodes; Buffer<uint32_t> d_sph_order; int sphere_bvh = 1;  // extension: hierarchy over the spheres
+    Buffer<uint2> d_ranges;             // (first, count) per leaf, input of k_leaf_records
+    Buffer<uint32_t> d_flag;            // material check result
     uint64_t upload_bytes = 0; double upload_ms = 0, upload_layout_ms = 0;   // last sqt_upload_scene
     int leaf_cull = 1;
     int terminate_on_black_ok = 0;
     uint32_t tree_height = 0;
     // image buffers
-    long long cap_pixels = 0;
-    int2 *d_prim = nullptr;
-    int *d_pixel_list = nullptr;
-    float *d_sbuf = nullptr; long long cap_sbuf = 0;     // sample buffer of one round (bytes)
+    Buffer<int2> d_prim;
+    Buffer<int> d_pixel_list;
+    Buffer<float> d_sbuf;               // sample buffer of one round
     long long sbuf_budget = 2ll << 30;
-    float *d_accum = nullptr;
-    uint8_t *d_rgb8 = nullptr;
+    Buffer<float> d_accum;
+    Buffer<uint8_t> d_rgb8;
     long long img_pixels = 0;
     int img_spp = 0;
-    DeviceStats *d_stats = nullptr;
-    DeviceStats *h_stats = nullptr;     // pinned
+    Buffer<DeviceStats> d_stats;
+    Pinned<DeviceStats> h_stats;
     // batch staging
-    long long cap_rays = 0;
-    float *d_org = nullptr, *d_dir = nullptr, *d_dist = nullptr, *d_point = nullptr;
-    int *d_tri = nullptr;
+    Buffer<float> d_org, d_dir, d_dist, d_point;
+    Buffer<int> d_tri;
     // pinned host staging for image I/O
-    uint8_t *h_rgb8 = nullptr; float *h_accum = nullptr; long long cap_host_pixels = 0;
+    Pinned<uint8_t> h_rgb8; Pinned<float> h_accum;
     Tune tune = {12, 0, 12};
     int pool_k = 2;                     // 0: one ray per lane (k_paths) ; K > 0: ray pools of 32*K rays per warp (k_paths_pool)
     PoolTune pool_tune = {4, 10, 16};
@@ -69,28 +105,19 @@ struct sqt_ctx {
     float slab_ratio = kSlabRatioMax, slab_ratio_leaf = kSlabRatioMaxLeaf;   // subtree / leaf slabs: test a slab when it is at most this
                                                                              // fraction of the clipped box (SQT_SLAB_RATIO=branch[,leaf], 0 = never)
     int pool_carveout = 0;              // shared-memory carve-out of k_paths_pool in percent of 228 KB (0 = the driver's choice)
-    float4 *d_gstack = nullptr; uint16_t *d_gpm = nullptr; uint4 *d_gpath = nullptr; long long cap_pool_slots = 0, cap_stack_entries = 0;
+    Buffer<float4> d_gstack; Buffer<uint16_t> d_gpm; Buffer<uint4> d_gpath;     // per pool slot: stack, materials, path state
     bool comm_broken = false;           // the communicator was aborted after a rank failed
-    // progressive frame (sqt_render_begin / sqt_render_advance): what the frame needs between two calls
-    bool prog = false;                  // a progressive frame is in progress
-    int prog_k = 0;                     // samples [0, prog_k) are in the sums
-    bool prog_count = false;
-    RenderParams prog_d = {};
-    RenderPlan prog_pl;
-    float *d_m2 = nullptr; long long cap_m2 = 0;                 // per-pixel second moment (npix * 3 floats)
-    float *d_red1 = nullptr, *d_red2 = nullptr; long long cap_red = 0;   // rank 0 of a group: sums and moments of all ranks
-    double *d_noise = nullptr, *h_noise = nullptr;               // partial sums of k_frame_noise_part + the result (pinned copy)
+    ProgFrame prog;
+    long long prog_frame = 0;           // numbers the progressive frames of this context (sqt_render_begin); never reset
+    Buffer<float> d_m2;                 // per-pixel second moment (npix * 3 floats)
+    Buffer<float> d_red1, d_red2;       // rank 0 of a group: sums and moments of all ranks
+    Buffer<double> d_noise; Pinned<double> h_noise;              // partial sums of k_frame_noise_part + the result (pinned copy)
     // adaptive frame (sqt_render_retire): per-pixel sample counts (0 = active) and the scratch of the list compaction
-    bool prog_adaptive = false;         // retire has run in this frame: d_pixel_list / n_hit hold the active pixels
-    long long prog_n = 0;               // this rank's active slots (the primary pass's hit count until the first retire)
-    long long prog_total = 0;           // active pixels of the whole frame after the last retire
-    int *d_counts = nullptr, *d_redc = nullptr, *d_list2 = nullptr; uint8_t *d_keep = nullptr; long long *d_tile = nullptr;
-    long long *d_active = nullptr, *h_active = nullptr;          // all-reduced active total; pinned (local, total)
-    long long prog_frame = 0;           // numbers the progressive frames of this context (sqt_render_begin)
+    Buffer<int> d_counts, d_redc, d_list2; Buffer<uint8_t> d_keep; Buffer<long long> d_tile;
+    Buffer<long long> d_active; Pinned<long long> h_active;      // all-reduced active total; pinned (local, total)
     // denoiser (sqt_denoise / sqt_download_features): features (N, z) and (surface + 1, key) -- on rank 0 of a group the sum
     // over ranks --, the filter's ping-pong (c, v) buffers, the denoised mean and its RGB8
-    float4 *d_feat = nullptr, *d_dn[2] = {nullptr, nullptr}; int2 *d_sk = nullptr; float *d_dn_mean = nullptr; uint8_t *d_dn_rgb8 = nullptr;
-    long long cap_dn = 0;
+    Buffer<float4> d_feat, d_dn[2]; Buffer<int2> d_sk; Buffer<float> d_dn_mean; Buffer<uint8_t> d_dn_rgb8;
     long long dn_frame = -1;            // the progressive frame whose features d_feat / d_sk hold (-1: none)
     // group
     int rank = 0, world = 1;
@@ -163,9 +190,9 @@ extern "C" int sqt_create(int device, sqt_ctx **out) {
         sqt_ctx *ctx = c;
         CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
         for (auto &ev : c->ev) CU(cudaEventCreate(&ev));
-        CU(cudaMalloc(&c->d_stats, sizeof(DeviceStats)));
-        CU(cudaMalloc(&c->d_flag, kFlagWords * sizeof(uint32_t)));
-        CU(cudaMallocHost(&c->h_stats, sizeof(DeviceStats)));
+        CU(c->d_stats.ensure(1));
+        CU(c->d_flag.ensure(kFlagWords));
+        CU(c->h_stats.ensure(1));
         return SQT_OK;
     };
     const int rc = init();
@@ -175,31 +202,13 @@ extern "C" int sqt_create(int device, sqt_ctx **out) {
     return SQT_OK;
 }
 
-static void free_scene(sqt_ctx *c) {
-    cudaFree(c->d_slabs); cudaFree(c->d_tight); cudaFree(c->d_levels); c->d_slabs = c->d_tight = nullptr; c->d_levels = nullptr;
-    cudaFree(c->d_nodes); cudaFree(c->d_boxes); cudaFree(c->d_tris); cudaFree(c->d_mats); cudaFree(c->d_leaves); cudaFree(c->d_spheres); cudaFree(c->d_sph_nodes); cudaFree(c->d_sph_order); cudaFree(c->d_ranges);
-    c->d_nodes = c->d_boxes = c->d_tris = c->d_mats = c->d_leaves = c->d_spheres = c->d_sph_nodes = nullptr; c->d_sph_order = nullptr; c->d_ranges = nullptr; c->has_scene = false;
-    c->cap_branches = c->cap_leaves = c->cap_tris = c->cap_mats = 0;
-}
-
 extern "C" int sqt_destroy(sqt_ctx *c) {
     if (!c) return SQT_OK;
     cudaSetDevice(c->device);
     if (c->comm && nccl_api()->lib && !c->comm_broken) nccl_api()->CommDestroy(c->comm);
-    free_scene(c);
-    cudaFree(c->d_prim); cudaFree(c->d_accum); cudaFree(c->d_rgb8); cudaFree(c->d_stats); cudaFree(c->d_flag); cudaFree(c->d_pixel_list); cudaFree(c->d_sbuf); cudaFree(c->d_gstack); cudaFree(c->d_gpm); cudaFree(c->d_gpath);
-    cudaFree(c->d_org); cudaFree(c->d_dir); cudaFree(c->d_dist); cudaFree(c->d_point); cudaFree(c->d_tri);
-    cudaFree(c->d_m2); cudaFree(c->d_red1); cudaFree(c->d_red2); cudaFree(c->d_noise);
-    cudaFree(c->d_counts); cudaFree(c->d_redc); cudaFree(c->d_list2); cudaFree(c->d_keep); cudaFree(c->d_tile); cudaFree(c->d_active);
-    cudaFree(c->d_feat); cudaFree(c->d_sk); cudaFree(c->d_dn[0]); cudaFree(c->d_dn[1]); cudaFree(c->d_dn_mean); cudaFree(c->d_dn_rgb8);
-    if (c->h_noise) cudaFreeHost(c->h_noise);
-    if (c->h_active) cudaFreeHost(c->h_active);
-    if (c->h_stats) cudaFreeHost(c->h_stats);
-    if (c->h_rgb8) cudaFreeHost(c->h_rgb8);
-    if (c->h_accum) cudaFreeHost(c->h_accum);
     for (auto &ev : c->ev) if (ev) cudaEventDestroy(ev);
     if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;                           // the buffers free themselves, on c->device
     return SQT_OK;
 }
 
@@ -220,37 +229,21 @@ extern "C" int sqt_device_info(sqt_ctx *c, int *sm_count, int *cc_major, int *cc
 // Device allocations are kept and reused while the new scene fits them.
 static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
+// branches, leaves, triangles (48 bytes each) and materials (three float4 each)
 static int ensure_scene_capacity(sqt_ctx *ctx, size_t n_br, size_t n_lf, size_t n_tris, size_t n_mats) {
-    if (n_br > ctx->cap_branches) {
-        cudaFree(ctx->d_nodes); cudaFree(ctx->d_boxes); cudaFree(ctx->d_slabs); cudaFree(ctx->d_tight); cudaFree(ctx->d_levels);
-        ctx->d_nodes = ctx->d_boxes = ctx->d_slabs = ctx->d_tight = nullptr; ctx->d_levels = nullptr; ctx->cap_branches = 0;
-        CU(cudaMalloc(&ctx->d_nodes, n_br * sizeof(float4))); CU(cudaMalloc(&ctx->d_boxes, 2 * n_br * sizeof(float4)));
-        CU(cudaMalloc(&ctx->d_slabs, n_br * sizeof(float4))); CU(cudaMalloc(&ctx->d_tight, 2 * n_br * sizeof(float4)));
-        CU(cudaMalloc(&ctx->d_levels, n_br * sizeof(uint32_t)));
-        ctx->cap_branches = n_br;
-    }
-    if (n_lf > ctx->cap_leaves) {
-        cudaFree(ctx->d_leaves); cudaFree(ctx->d_ranges); ctx->d_leaves = nullptr; ctx->d_ranges = nullptr; ctx->cap_leaves = 0;
-        CU(cudaMalloc(&ctx->d_leaves, 2 * n_lf * sizeof(float4))); CU(cudaMalloc(&ctx->d_ranges, n_lf * sizeof(uint2)));
-        ctx->cap_leaves = n_lf;
-    }
-    if (n_tris > ctx->cap_tris) {
-        cudaFree(ctx->d_tris); ctx->d_tris = nullptr; ctx->cap_tris = 0;
-        CU(cudaMalloc(&ctx->d_tris, n_tris * 48));
-        ctx->cap_tris = n_tris;
-    }
-    if (n_mats > ctx->cap_mats) {
-        cudaFree(ctx->d_mats); ctx->d_mats = nullptr; ctx->cap_mats = 0;
-        CU(cudaMalloc(&ctx->d_mats, 3 * n_mats * sizeof(float4)));
-        ctx->cap_mats = n_mats;
-    }
+    CU(ctx->d_nodes.ensure(n_br)); CU(ctx->d_boxes.ensure(2 * n_br));
+    CU(ctx->d_slabs.ensure(n_br)); CU(ctx->d_tight.ensure(2 * n_br));
+    CU(ctx->d_levels.ensure(n_br));
+    CU(ctx->d_leaves.ensure(2 * n_lf)); CU(ctx->d_ranges.ensure(n_lf));
+    CU(ctx->d_tris.ensure(3 * n_tris));
+    CU(ctx->d_mats.ensure(3 * n_mats));
     return SQT_OK;
 }
 
 // triangles -> every context, chunk by chunk through two pinned buffers (runs on a helper thread)
 static void stream_tris(sqt_ctx **ctxs, int n, const sqt_tri *tris, size_t n_tris, std::atomic<int> *status, std::string *err) {
     const size_t CH = (size_t)32 << 20, bytes = n_tris * 48;
-    void *pin[2] = {nullptr, nullptr};
+    Pinned<char> pin[2];
     std::vector<cudaEvent_t> done(2 * (size_t)n);
     auto bail = [&](cudaError_t e, const char *what) { *err = std::string(what) + ": " + cudaGetErrorString(e); status->store(SQT_E_CUDA); };
     cudaError_t e = cudaSuccess;
@@ -259,7 +252,7 @@ static void stream_tris(sqt_ctx **ctxs, int n, const sqt_tri *tris, size_t n_tri
         if (bytes == 0) break;
         const size_t buf = bytes < CH ? bytes : CH;
         if ((e = cudaSetDevice(ctxs[0]->device)) != cudaSuccess) { bail(e, "cudaSetDevice"); break; }
-        if ((e = cudaMallocHost(&pin[0], buf)) != cudaSuccess || (bytes > CH && (e = cudaMallocHost(&pin[1], buf)) != cudaSuccess)) { bail(e, "cudaMallocHost (staging)"); break; }
+        if ((e = pin[0].ensure(buf)) != cudaSuccess || (bytes > CH && (e = pin[1].ensure(buf)) != cudaSuccess)) { bail(e, "cudaMallocHost (staging)"); break; }
         for (int g = 0; g < n && e == cudaSuccess; ++g) { cudaSetDevice(ctxs[g]->device); for (int b = 0; b < 2 && e == cudaSuccess; ++b) e = cudaEventCreateWithFlags(&done[2 * g + b], cudaEventDisableTiming); }
         if (e != cudaSuccess) { bail(e, "cudaEventCreate"); break; }
         have_ev = true;
@@ -272,7 +265,7 @@ static void stream_tris(sqt_ctx **ctxs, int n, const sqt_tri *tris, size_t n_tri
             memcpy(pin[b], (const char *)tris + off, len);
             for (int g = 0; g < n; ++g) {
                 cudaSetDevice(ctxs[g]->device);
-                if ((e = cudaMemcpyAsync((char *)ctxs[g]->d_tris + off, pin[b], len, cudaMemcpyHostToDevice, ctxs[g]->stream)) != cudaSuccess) break;
+                if ((e = cudaMemcpyAsync((char *)ctxs[g]->d_tris.p + off, pin[b], len, cudaMemcpyHostToDevice, ctxs[g]->stream)) != cudaSuccess) break;
                 if ((e = cudaEventRecord(done[2 * g + b], ctxs[g]->stream)) != cudaSuccess) break;
             }
             if (e != cudaSuccess) { bail(e, "cudaMemcpyAsync (triangles)"); break; }
@@ -281,13 +274,12 @@ static void stream_tris(sqt_ctx **ctxs, int n, const sqt_tri *tris, size_t n_tri
         for (int g = 0; g < n; ++g) { cudaSetDevice(ctxs[g]->device); cudaStreamSynchronize(ctxs[g]->stream); }
     } while (false);
     if (have_ev) for (int g = 0; g < n; ++g) { cudaSetDevice(ctxs[g]->device); for (int b = 0; b < 2; ++b) cudaEventDestroy(done[2 * g + b]); }
-    for (void *p : pin) if (p) cudaFreeHost(p);
 }
 
 static int upload_scene_to(sqt_ctx **ctxs, int n, const sqt_scene_desc *s) {
     sqt_ctx *ctx = ctxs[0];
     const double t0 = now_ms();
-    for (int g = 0; g < n; ++g) ctxs[g]->prog = false;          // a new scene ends a progressive frame
+    for (int g = 0; g < n; ++g) ctxs[g]->prog.on = false;       // a new scene ends a progressive frame
     if (!s->nodes || s->n_nodes == 0) return fail(ctx, SQT_E_INVALID, "scene has no BIH nodes");
     if (s->n_tris && !s->tris) return fail(ctx, SQT_E_INVALID, "tris is NULL");
     if (s->n_tris >= (1u << 27) || s->n_nodes >= (1u << 27)) return fail(ctx, SQT_E_UNSUPPORTED, "scene too large for the 27-bit indices");
@@ -384,11 +376,17 @@ extern "C" int sqt_upload_scene(sqt_ctx *ctx, const sqt_scene_desc *s) {
     return upload_scene_to(&ctx, 1, s);
 }
 
+// a group call's context array: n >= 1 contexts, none of them NULL
+static bool valid_group(sqt_ctx **ctxs, int n) {
+    if (!ctxs || n < 1) return false;
+    for (int i = 0; i < n; ++i) if (!ctxs[i]) return false;
+    return true;
+}
+
 // the same scene onto every context of a single-process group: the tree is walked once, every staged chunk of
 // triangles goes to all devices
 extern "C" int sqt_upload_scene_group(sqt_ctx **ctxs, int n, const sqt_scene_desc *s) {
-    if (!ctxs || n < 1 || !s) return SQT_E_INVALID;
-    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
+    if (!valid_group(ctxs, n) || !s) return SQT_E_INVALID;
     return upload_scene_to(ctxs, n, s);
 }
 
@@ -403,7 +401,7 @@ extern "C" int sqt_last_upload(const sqt_ctx *ctx, uint64_t *h2d_bytes, double *
 // extension: analytic spheres (include/sqt.h)
 extern "C" int sqt_upload_spheres(sqt_ctx *ctx, const sqt_sphere *sp, uint32_t n) {
     if (!ctx) return SQT_E_INVALID;
-    ctx->prog = false;
+    ctx->prog.on = false;
     if (!ctx->has_scene) return fail(ctx, SQT_E_NO_SCENE, "sqt_upload_spheres before sqt_upload_scene");
     if (n && !sp) return fail(ctx, SQT_E_INVALID, "spheres is NULL");
     if ((uint64_t)ctx->sc.n_tris + n >= (1u << 27)) return fail(ctx, SQT_E_UNSUPPORTED, "too many surfaces");
@@ -415,11 +413,10 @@ extern "C" int sqt_upload_spheres(sqt_ctx *ctx, const sqt_sphere *sp, uint32_t n
         ds[2 * k] = make_float4(sp[k].center[0], sp[k].center[1], sp[k].center[2], sp[k].radius);
         ds[2 * k + 1] = make_float4(u2f(sp[k].material), 0.0f, 0.0f, 0.0f);
     }
-    cudaFree(ctx->d_spheres); cudaFree(ctx->d_sph_nodes); cudaFree(ctx->d_sph_order);
-    ctx->d_spheres = nullptr; ctx->d_sph_nodes = nullptr; ctx->d_sph_order = nullptr;
+    ctx->d_spheres.reset(0); ctx->d_sph_nodes.reset(0); ctx->d_sph_order.reset(0);
     ctx->sc.spheres = nullptr; ctx->sc.sph_nodes = nullptr; ctx->sc.sph_order = nullptr; ctx->sc.n_spheres = 0;
     if (n == 0) return SQT_OK;
-    CU(cudaMalloc(&ctx->d_spheres, ds.size() * sizeof(float4)));
+    CU(ctx->d_spheres.reset(ds.size()));
     CU(cudaMemcpy(ctx->d_spheres, ds.data(), ds.size() * sizeof(float4), cudaMemcpyHostToDevice));
     ctx->sc.spheres = ctx->d_spheres; ctx->sc.n_spheres = n;
     // a hierarchy over the spheres (sphere_step): only for finite, moderate coordinates -- the culling bound assumes no overflow
@@ -429,8 +426,8 @@ extern "C" int sqt_upload_spheres(sqt_ctx *ctx, const sqt_sphere *sp, uint32_t n
     if (tame) {
         SphereBvh bvh;
         build_sphere_bvh(sp, n, bvh);
-        CU(cudaMalloc(&ctx->d_sph_nodes, bvh.nodes.size() * sizeof(float4)));
-        CU(cudaMalloc(&ctx->d_sph_order, bvh.order.size() * sizeof(uint32_t)));
+        CU(ctx->d_sph_nodes.reset(bvh.nodes.size()));
+        CU(ctx->d_sph_order.reset(bvh.order.size()));
         CU(cudaMemcpy(ctx->d_sph_nodes, bvh.nodes.data(), bvh.nodes.size() * sizeof(float4), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(ctx->d_sph_order, bvh.order.data(), bvh.order.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
         ctx->sc.sph_nodes = ctx->d_sph_nodes; ctx->sc.sph_order = ctx->d_sph_order;
@@ -450,40 +447,18 @@ extern "C" int sqt_set_option(sqt_ctx *ctx, int option, int value) {
 }
 
 // ------------------------------------------------------------------------------ helpers
+// the device buffers of an image of npix pixels (the pixel list has 32 entries of slack)
 static int ensure_image(sqt_ctx *ctx, long long npix) {
-    if (npix <= ctx->cap_pixels) return SQT_OK;
-    cudaFree(ctx->d_prim); cudaFree(ctx->d_accum); cudaFree(ctx->d_rgb8); cudaFree(ctx->d_pixel_list);
-    ctx->d_prim = nullptr; ctx->d_accum = nullptr; ctx->d_rgb8 = nullptr; ctx->d_pixel_list = nullptr; ctx->cap_pixels = 0;
-    CU(cudaMalloc(&ctx->d_prim, (size_t)npix * sizeof(int2)));
-    CU(cudaMalloc(&ctx->d_pixel_list, (size_t)(npix + 32) * sizeof(int)));
-    CU(cudaMalloc(&ctx->d_accum, (size_t)npix * 3 * sizeof(float)));
-    CU(cudaMalloc(&ctx->d_rgb8, (size_t)npix * 3));
-    ctx->cap_pixels = npix;
+    CU(ctx->d_prim.ensure(npix));
+    CU(ctx->d_pixel_list.ensure(npix + 32));
+    CU(ctx->d_accum.ensure(npix * 3));
+    CU(ctx->d_rgb8.ensure(npix * 3));
     return SQT_OK;
 }
-static int ensure_sbuf(sqt_ctx *ctx, long long bytes) {
-    if (bytes <= ctx->cap_sbuf) return SQT_OK;
-    cudaFree(ctx->d_sbuf); ctx->d_sbuf = nullptr; ctx->cap_sbuf = 0;
-    CU(cudaMalloc(&ctx->d_sbuf, (size_t)bytes));
-    ctx->cap_sbuf = bytes;
-    return SQT_OK;
-}
+// the pinned staging of an image's RGB8 and sums (also of the moments and the sample counts)
 static int ensure_host_image(sqt_ctx *ctx, long long npix) {
-    if (npix <= ctx->cap_host_pixels) return SQT_OK;
-    cudaFreeHost(ctx->h_rgb8); cudaFreeHost(ctx->h_accum); ctx->h_rgb8 = nullptr; ctx->h_accum = nullptr; ctx->cap_host_pixels = 0;
-    CU(cudaMallocHost(&ctx->h_rgb8, (size_t)npix * 3));
-    CU(cudaMallocHost(&ctx->h_accum, (size_t)npix * 3 * sizeof(float)));
-    ctx->cap_host_pixels = npix;
-    return SQT_OK;
-}
-static int ensure_rays(sqt_ctx *ctx, long long n) {
-    if (n <= ctx->cap_rays) return SQT_OK;
-    cudaFree(ctx->d_org); cudaFree(ctx->d_dir); cudaFree(ctx->d_dist); cudaFree(ctx->d_point); cudaFree(ctx->d_tri);
-    ctx->d_org = ctx->d_dir = ctx->d_dist = ctx->d_point = nullptr; ctx->d_tri = nullptr; ctx->cap_rays = 0;
-    CU(cudaMalloc(&ctx->d_org, (size_t)n * 12)); CU(cudaMalloc(&ctx->d_dir, (size_t)n * 12));
-    CU(cudaMalloc(&ctx->d_dist, (size_t)n * 4)); CU(cudaMalloc(&ctx->d_point, (size_t)n * 12));
-    CU(cudaMalloc(&ctx->d_tri, (size_t)n * 4));
-    ctx->cap_rays = n;
+    CU(ctx->h_rgb8.ensure(npix * 3));
+    CU(ctx->h_accum.ensure(npix * 3));
     return SQT_OK;
 }
 // persistent launch: as many 128-lane CTAs as stay resident on the 148 SMs (never more than the work needs)
@@ -524,14 +499,14 @@ static int pool_step(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, i
     // the per-path material list of a slot: max_depth entries, packed (16-byte granules) for the same reason
     int pm_stride = (d.max_depth + 7) & ~7;
     if (pm_stride > SQT_MAX_DEPTH) pm_stride = SQT_MAX_DEPTH;
-    if (slots > ctx->cap_pool_slots || slots * depth > ctx->cap_stack_entries) {
-        cudaFree(ctx->d_gstack); cudaFree(ctx->d_gpm); cudaFree(ctx->d_gpath);
-        ctx->d_gstack = nullptr; ctx->d_gpm = nullptr; ctx->d_gpath = nullptr; ctx->cap_pool_slots = 0; ctx->cap_stack_entries = 0;
+    // d_gpath holds two entries per slot, so its capacity tells the slot capacity; it is emptied first, so that after a
+    // failed allocation the next call allocates all three again
+    if (slots > (long long)ctx->d_gpath.cap / 2 || slots * depth > (long long)ctx->d_gstack.cap) {
         const long long cap = (long long)ctx->sm_count * 16 * 4 * 32 * K > slots ? (long long)ctx->sm_count * 16 * 4 * 32 * K : slots;
-        CU(cudaMalloc(&ctx->d_gstack, (size_t)cap * depth * sizeof(float4)));
-        CU(cudaMalloc(&ctx->d_gpm, (size_t)cap * SQT_MAX_DEPTH * sizeof(uint16_t)));
-        CU(cudaMalloc(&ctx->d_gpath, (size_t)cap * 2 * sizeof(uint4)));
-        ctx->cap_pool_slots = cap; ctx->cap_stack_entries = cap * depth;
+        ctx->d_gpath.reset(0);
+        CU(ctx->d_gstack.reset(cap * depth));
+        CU(ctx->d_gpm.reset(cap * SQT_MAX_DEPTH));
+        CU(ctx->d_gpath.reset(cap * 2));
     }
     if (!launch) return SQT_OK;
     kern<<<(int)grid, 128, smem, ctx->stream>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->pool_tune, ctx->d_gstack, ctx->d_gpm, ctx->d_gpath, depth, pm_stride);
@@ -557,7 +532,9 @@ extern "C" int sqt_intersect_batch(sqt_ctx *ctx, const float *org, const float *
     if (stats) memset(stats, 0, sizeof *stats);
     if (n == 0) return SQT_OK;
     CU(cudaSetDevice(ctx->device));
-    int rc = ensure_rays(ctx, n); if (rc) return rc;
+    CU(ctx->d_org.ensure(n * 3)); CU(ctx->d_dir.ensure(n * 3));
+    CU(ctx->d_dist.ensure(n)); CU(ctx->d_point.ensure(n * 3));
+    CU(ctx->d_tri.ensure(n));
     cudaStream_t st = ctx->stream;
     CU(cudaEventRecord(ctx->ev[0], st));
     CU(cudaMemcpyAsync(ctx->d_org, org, (size_t)n * 12, cudaMemcpyHostToDevice, st));
@@ -567,11 +544,11 @@ extern "C" int sqt_intersect_batch(sqt_ctx *ctx, const float *org, const float *
     CU(cudaEventRecord(ctx->ev[1], st));
     if (stats)      // instrumented variant: fills the visit/test counters
         k_intersect_batch<true><<<persistent_grid(ctx, k_intersect_batch<true>, n), 128, 0, st>>>(
-            ctx->sc, ctx->d_org, ctx->d_dir, n, ctx->d_tri, dist_out ? ctx->d_dist : nullptr, point_out ? ctx->d_point : nullptr,
+            ctx->sc, ctx->d_org, ctx->d_dir, n, ctx->d_tri, dist_out ? ctx->d_dist.p : nullptr, point_out ? ctx->d_point.p : nullptr,
             ctx->d_stats, ctx->tune);
     else
         k_intersect_batch<false><<<persistent_grid(ctx, k_intersect_batch<false>, n), 128, 0, st>>>(
-            ctx->sc, ctx->d_org, ctx->d_dir, n, ctx->d_tri, dist_out ? ctx->d_dist : nullptr, point_out ? ctx->d_point : nullptr,
+            ctx->sc, ctx->d_org, ctx->d_dir, n, ctx->d_tri, dist_out ? ctx->d_dist.p : nullptr, point_out ? ctx->d_point.p : nullptr,
             ctx->d_stats, ctx->tune);
     CU(cudaGetLastError());
     CU(cudaEventRecord(ctx->ev[2], st));
@@ -632,7 +609,7 @@ static int prepare_render(sqt_ctx *ctx, const RenderParams &d, bool count, bool 
     const int S = 1 << pl.log2_s;
     if ((pl.k1 - pl.k0 + S - 1) / S > 256) return fail(ctx, SQT_E_UNSUPPORTED, "more than 256 sample rounds (raise SQT_SBUF_MB)");
     pl.sbytes = pl.nwork * (long long)S * 12ll;
-    rc = ensure_sbuf(ctx, pl.sbytes > 0 ? pl.sbytes : 12); if (rc) return rc;
+    CU(ctx->d_sbuf.ensure((pl.sbytes > 0 ? pl.sbytes : 12) / sizeof(float)));
     if (ctx->pool_k > 0) {
         RoundInfo none = {};
         rc = count ? pool_step_k<true>(ctx, d, none, 0, pl.nwork << pl.log2_s, false) : pool_step_k<false>(ctx, d, none, 0, pl.nwork << pl.log2_s, false);
@@ -710,8 +687,8 @@ static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, long 
         return SQT_OK;
     }
     RoundInfo rd = {};
-    rd.pixel_list = d.primary_reuse ? ctx->d_pixel_list : nullptr;
-    rd.prim = d.primary_reuse ? ctx->d_prim : nullptr;
+    rd.pixel_list = d.primary_reuse ? ctx->d_pixel_list.p : nullptr;
+    rd.prim = d.primary_reuse ? ctx->d_prim.p : nullptr;
     rd.n_slots = nwork; rd.slot_stride = nwork;
     rd.log2_s = log2_s;
     const int S = 1 << rd.log2_s;
@@ -807,7 +784,7 @@ static void fill_stats(sqt_ctx *ctx, sqt_stats *s, uint32_t launches) {
 
 extern "C" int sqt_render_resident(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
     if (!ctx) return SQT_E_INVALID;
-    ctx->prog = false;
+    ctx->prog.on = false;
     if (stats) memset(stats, 0, sizeof *stats);
     cudaSetDevice(ctx->device);
     RenderParams d = {};
@@ -825,7 +802,7 @@ extern "C" int sqt_render_resident(sqt_ctx *ctx, const sqt_camera *cam, const sq
 // the sums (moments = false) or second moments of the frame: on rank 0 of a progressive group frame the reduced
 // copies, everywhere else the context's own buffers
 static float *frame_sums(sqt_ctx *ctx, bool moments) {
-    const bool reduced = ctx->prog && ctx->world > 1 && ctx->comm && ctx->rank == 0;
+    const bool reduced = ctx->prog.on && ctx->world > 1 && ctx->comm && ctx->rank == 0;
     if (moments) return reduced ? ctx->d_red2 : ctx->d_m2;
     return reduced ? ctx->d_red1 : ctx->d_accum;
 }
@@ -847,7 +824,7 @@ extern "C" int sqt_download_image(sqt_ctx *ctx, uint8_t *rgb8_out, float *accum_
 extern "C" int sqt_render(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, uint8_t *rgb8_out,
                           float *accum_out, sqt_stats *stats) {
     if (!ctx) return SQT_E_INVALID;
-    ctx->prog = false;
+    ctx->prog.on = false;
     if (stats) memset(stats, 0, sizeof *stats);
     cudaSetDevice(ctx->device);
     RenderParams d = {};
@@ -878,7 +855,7 @@ extern "C" int sqt_render(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_
 
 extern "C" int sqt_tone_map(sqt_ctx *ctx, const float *mean_rgb, int64_t npix, uint8_t *rgb8_out) {
     if (!ctx) return SQT_E_INVALID;
-    ctx->prog = false;                  // d_accum is its scratch
+    ctx->prog.on = false;               // d_accum is its scratch
     if (npix < 0 || (npix > 0 && (!mean_rgb || !rgb8_out))) return fail(ctx, SQT_E_INVALID, "bad tone_map arguments");
     if (npix == 0) return SQT_OK;
     CU(cudaSetDevice(ctx->device));
@@ -898,40 +875,46 @@ extern "C" int sqt_tone_map(sqt_ctx *ctx, const float *mean_rgb, int64_t npix, u
 // noise reduction's partial sums, what sqt_render_retire needs (sample counts, the compaction's scratch) and, on rank 0
 // of a group, the reduced sums, moments and counts.  Neither sqt_render_advance nor sqt_render_retire allocates.
 static int ensure_progressive(sqt_ctx *ctx, long long npix) {
-    if (!ctx->d_noise) CU(cudaMalloc(&ctx->d_noise, (2 * kNoiseBlocks + 1) * sizeof(double)));
-    if (!ctx->h_noise) CU(cudaMallocHost(&ctx->h_noise, sizeof(double)));
-    if (!ctx->d_active) CU(cudaMalloc(&ctx->d_active, sizeof(long long)));
-    if (!ctx->h_active) CU(cudaMallocHost(&ctx->h_active, 2 * sizeof(long long)));
-    if (npix > ctx->cap_m2) {
-        cudaFree(ctx->d_m2); cudaFree(ctx->d_counts); cudaFree(ctx->d_list2); cudaFree(ctx->d_keep); cudaFree(ctx->d_tile);
-        ctx->d_m2 = nullptr; ctx->d_counts = nullptr; ctx->d_list2 = nullptr; ctx->d_keep = nullptr; ctx->d_tile = nullptr; ctx->cap_m2 = 0;
-        CU(cudaMalloc(&ctx->d_m2, (size_t)npix * 12));
-        CU(cudaMalloc(&ctx->d_counts, (size_t)npix * sizeof(int)));
-        CU(cudaMalloc(&ctx->d_list2, (size_t)npix * sizeof(int)));
-        CU(cudaMalloc(&ctx->d_keep, (size_t)npix));
-        CU(cudaMalloc(&ctx->d_tile, (size_t)(npix / kRetireTile + 1) * sizeof(long long)));
-        ctx->cap_m2 = npix;
-    }
-    if (ctx->world > 1 && ctx->comm && ctx->rank == 0 && npix > ctx->cap_red) {
-        cudaFree(ctx->d_red1); cudaFree(ctx->d_red2); cudaFree(ctx->d_redc); ctx->d_red1 = ctx->d_red2 = nullptr; ctx->d_redc = nullptr; ctx->cap_red = 0;
-        CU(cudaMalloc(&ctx->d_red1, (size_t)npix * 12));
-        CU(cudaMalloc(&ctx->d_red2, (size_t)npix * 12));
-        CU(cudaMalloc(&ctx->d_redc, (size_t)npix * sizeof(int)));
-        ctx->cap_red = npix;
+    CU(ctx->d_noise.ensure(2 * kNoiseBlocks + 1));
+    CU(ctx->h_noise.ensure(1));
+    CU(ctx->d_active.ensure(1));
+    CU(ctx->h_active.ensure(2));
+    CU(ctx->d_m2.ensure(npix * 3));
+    CU(ctx->d_counts.ensure(npix));
+    CU(ctx->d_list2.ensure(npix));
+    CU(ctx->d_keep.ensure(npix));
+    CU(ctx->d_tile.ensure(npix / kRetireTile + 1));
+    if (ctx->world > 1 && ctx->comm && ctx->rank == 0) {
+        CU(ctx->d_red1.ensure(npix * 3));
+        CU(ctx->d_red2.ensure(npix * 3));
+        CU(ctx->d_redc.ensure(npix));
     }
     return SQT_OK;
 }
 // the sample counts of an adaptive frame (0 = samples_done): rank 0 of a group reads the sum over ranks
 static const int *frame_counts(sqt_ctx *ctx) {
-    if (!ctx->prog_adaptive) return nullptr;
+    if (!ctx->prog.adaptive) return nullptr;
     return ctx->world > 1 && ctx->comm && ctx->rank == 0 ? ctx->d_redc : ctx->d_counts;
+}
+// a failure after the group agreement of a progressive call ends the frame, leaving no image to download
+static int frame_abort(sqt_ctx *ctx, int rc) {
+    ctx->prog.on = false; ctx->img_pixels = 0;
+    return group_abort(ctx, rc);
+}
+// what retire and the denoiser read, the primary hits and the per-pixel variance, needs a frame in progress, begun with
+// primary reuse, with k >= 2 samples
+static int check_variance_frame(sqt_ctx *ctx, const char *what) {
+    if (!ctx->prog.on) return fail(ctx, SQT_E_INVALID, "%s: no progressive frame in progress", what);
+    if (!ctx->prog.d.primary_reuse) return fail(ctx, SQT_E_UNSUPPORTED, "%s needs primary reuse (not SQT_F_NO_PRIMARY_REUSE)", what);
+    if (ctx->prog.k < 2) return fail(ctx, SQT_E_INVALID, "%s needs at least 2 samples per pixel (samples done: %d)", what, ctx->prog.k);
+    return SQT_OK;
 }
 
 extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
     if (!ctx) return SQT_E_INVALID;
     if (stats) memset(stats, 0, sizeof *stats);
     cudaSetDevice(ctx->device);
-    ctx->prog = false; ctx->img_pixels = 0;
+    ctx->prog.on = false; ctx->img_pixels = 0;
     RenderParams d = {};
     RenderPlan pl;
     int rc = check_params(ctx, cam, p);
@@ -953,10 +936,10 @@ extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_r
         CU(cudaStreamSynchronize(st));
         return SQT_OK;
     };
-    rc = enqueue(); if (rc) return group_abort(ctx, rc);
+    rc = enqueue(); if (rc) return frame_abort(ctx, rc);
     fill_stats(ctx, stats, nl);
-    ctx->prog = true; ctx->prog_k = 0; ctx->prog_count = count; ctx->prog_d = d; ctx->prog_pl = pl; ctx->prog_frame++;
-    ctx->prog_adaptive = false; ctx->prog_n = (long long)ctx->h_stats->n_hit; ctx->prog_total = 0;
+    ctx->prog = ProgFrame{/*on*/ true, /*k*/ 0, count, d, pl, /*adaptive*/ false, /*n*/ (long long)ctx->h_stats->n_hit, /*total*/ 0};
+    ctx->prog_frame++;
     return SQT_OK;
 }
 
@@ -965,43 +948,44 @@ extern "C" int sqt_render_advance(sqt_ctx *ctx, int32_t n_samples, sqt_progress 
     if (stats) memset(stats, 0, sizeof *stats);
     cudaSetDevice(ctx->device);
     int rc = SQT_OK;
-    if (!ctx->prog) rc = fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    if (!ctx->prog.on) rc = fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
     else if (n_samples < 1) rc = fail(ctx, SQT_E_INVALID, "n_samples must be at least 1");
-    const RenderParams &d = ctx->prog_d;
-    const int k = ctx->prog_k, spp = d.spp;
+    ProgFrame &f = ctx->prog;
+    const RenderParams &d = f.d;
+    const int k = f.k, spp = d.spp;
     const int kb = rc ? 0 : (n_samples >= spp - k ? spp : k + n_samples);
     const int32_t keys[3] = {rc ? 0 : k, rc ? 0 : spp, kb};
     rc = group_agree(ctx, rc, keys, 3); if (rc) return rc;
     const bool root = ctx->rank == 0;
-    if (k < spp && ctx->prog_adaptive && ctx->prog_total == 0) {
-        ctx->prog_k = kb; ctx->img_spp = kb;            // every pixel has retired: nothing to trace, the image stays
+    if (k < spp && f.adaptive && f.total == 0) {
+        f.k = kb; ctx->img_spp = kb;                    // every pixel has retired: nothing to trace, the image stays
     } else if (k < spp) {
         const long long npix = (long long)d.rows * d.cols;
         // an adaptive frame traces its active slots only, in rounds as wide as the sample buffer allows for them (at
         // most the chunk: wider rounds would only skip items); results never depend on the round width
-        const long long nslots = ctx->prog_adaptive ? ctx->prog_n : ctx->prog_pl.nwork;
-        const int log2_s = ctx->prog_adaptive ? round_log2_s(nslots, kb - k, ctx->prog_pl.sbytes) : ctx->prog_pl.log2_s;
+        const long long nslots = f.adaptive ? f.n : f.pl.nwork;
+        const int log2_s = f.adaptive ? round_log2_s(nslots, kb - k, f.pl.sbytes) : f.pl.log2_s;
         cudaStream_t st = ctx->stream;
         uint32_t nl = 0;
         auto enqueue = [&]() -> int {
             // the counters of this call only; n_hit (the primary pass's pixel list) stays
             CU(cudaMemsetAsync(ctx->d_stats, 0, offsetof(DeviceStats, n_hit), st));
-            CU(cudaMemsetAsync((char *)ctx->d_stats + offsetof(DeviceStats, work_next), 0, sizeof(DeviceStats) - offsetof(DeviceStats, work_next), st));
+            CU(cudaMemsetAsync((char *)ctx->d_stats.p + offsetof(DeviceStats, work_next), 0, sizeof(DeviceStats) - offsetof(DeviceStats, work_next), st));
             CU(cudaEventRecord(ctx->ev[0], st));
             CU(cudaEventRecord(ctx->ev[1], st));
-            int r = enqueue_rounds(ctx, d, ctx->prog_count, nslots, log2_s, k, kb, ctx->d_m2, nl); if (r) return r;
+            int r = enqueue_rounds(ctx, d, f.count, nslots, log2_s, k, kb, ctx->d_m2, nl); if (r) return r;
             r = enqueue_finish(ctx, npix, 1.0f / (float)kb, frame_sums(ctx, false), frame_sums(ctx, true), kb, frame_counts(ctx), nl);
             if (r) return r;
             CU(cudaStreamSynchronize(st));
             return SQT_OK;
         };
         rc = enqueue();
-        if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+        if (rc) return frame_abort(ctx, rc);
         fill_stats(ctx, stats, nl);
-        ctx->prog_k = kb; ctx->img_pixels = npix; ctx->img_spp = kb;
+        f.k = kb; ctx->img_pixels = npix; ctx->img_spp = kb;
     }
     if (progress) {
-        progress->samples_done = ctx->prog_k; progress->samples_total = spp;
+        progress->samples_done = f.k; progress->samples_total = spp;
         progress->noise = root ? *ctx->h_noise : __builtin_nan("");
     }
     return SQT_OK;
@@ -1009,10 +993,10 @@ extern "C" int sqt_render_advance(sqt_ctx *ctx, int32_t n_samples, sqt_progress 
 
 extern "C" int sqt_download_moments(sqt_ctx *ctx, float *m2_out) {
     if (!ctx) return SQT_E_INVALID;
-    if (!ctx->prog) return fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    if (!ctx->prog.on) return fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
     if (!m2_out) return fail(ctx, SQT_E_INVALID, "m2_out is NULL");
     CU(cudaSetDevice(ctx->device));
-    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    const long long npix = (long long)ctx->prog.d.rows * ctx->prog.d.cols;
     int rc = ensure_host_image(ctx, npix); if (rc) return rc;
     CU(cudaMemcpyAsync(ctx->h_accum, frame_sums(ctx, true), (size_t)npix * 12, cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));
@@ -1026,27 +1010,24 @@ static uint32_t float_bits(float f) { uint32_t u; memcpy(&u, &f, 4); return u; }
 extern "C" int sqt_render_retire(sqt_ctx *ctx, const sqt_retire_params *rp, int64_t *active_out) {
     if (!ctx) return SQT_E_INVALID;
     cudaSetDevice(ctx->device);
-    int rc = SQT_OK;
-    if (!ctx->prog) rc = fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
-    else if (!rp) rc = fail(ctx, SQT_E_INVALID, "retire params are NULL");
-    else if (!ctx->prog_d.primary_reuse) rc = fail(ctx, SQT_E_UNSUPPORTED, "adaptive frames need primary reuse (not SQT_F_NO_PRIMARY_REUSE)");
-    else if (ctx->prog_k < 2) rc = fail(ctx, SQT_E_INVALID, "retire needs at least 2 samples per pixel (samples done: %d)", ctx->prog_k);
-    else if (rp->min_samples < 2) rc = fail(ctx, SQT_E_INVALID, "min_samples must be at least 2");
-    else if (!(rp->rel_tol >= 0.0f) || !(rp->abs_tol >= 0.0f)) rc = fail(ctx, SQT_E_INVALID, "tolerances must be non-negative numbers");
-    else if (rp->reserved) rc = fail(ctx, SQT_E_INVALID, "reserved must be 0");
-    const int k = ctx->prog_k, spp = ctx->prog_d.spp;
+    int rc = rp ? check_variance_frame(ctx, "sqt_render_retire") : fail(ctx, SQT_E_INVALID, "retire params are NULL");
+    if (!rc && rp->min_samples < 2) rc = fail(ctx, SQT_E_INVALID, "min_samples must be at least 2");
+    if (!rc && (!(rp->rel_tol >= 0.0f) || !(rp->abs_tol >= 0.0f))) rc = fail(ctx, SQT_E_INVALID, "tolerances must be non-negative numbers");
+    if (!rc && rp->reserved) rc = fail(ctx, SQT_E_INVALID, "reserved must be 0");
+    ProgFrame &f = ctx->prog;
+    const int k = f.k, spp = f.d.spp;
     const int32_t keys[5] = {rc ? 0 : k, rc ? 0 : spp, rc ? 0 : (int32_t)float_bits(rp->rel_tol), rc ? 0 : (int32_t)float_bits(rp->abs_tol),
                              rc ? 0 : rp->min_samples};
     rc = group_agree(ctx, rc, keys, 5); if (rc) return rc;
     const bool group = ctx->world > 1 && ctx->comm;
-    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    const long long npix = (long long)f.d.rows * f.d.cols;
     cudaStream_t st = ctx->stream;
     // at k = spp, and before min_samples, nothing can retire: only the active total is reported
     const bool test = k < spp && k >= rp->min_samples;
     auto enqueue = [&]() -> int {
-        const long long n = ctx->prog_n;
+        const long long n = f.n;
         if (test) {
-            if (!ctx->prog_adaptive) CU(cudaMemsetAsync(ctx->d_counts, 0, (size_t)npix * sizeof(int), st));
+            if (!f.adaptive) CU(cudaMemsetAsync(ctx->d_counts, 0, (size_t)npix * sizeof(int), st));
             if (n > 0) {
                 const long long tiles = (n + kRetireTile - 1) / kRetireTile;
                 k_retire_mark<<<(int)tiles, 256, 0, st>>>(ctx->d_pixel_list, n, ctx->d_accum, ctx->d_m2, k,
@@ -1074,21 +1055,21 @@ extern "C" int sqt_render_retire(sqt_ctx *ctx, const sqt_retire_params *rp, int6
         return SQT_OK;
     };
     rc = enqueue();
-    if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
-    ctx->prog_n = ctx->h_active[0];
-    ctx->prog_total = group ? ctx->h_active[1] : ctx->h_active[0];
-    if (test) ctx->prog_adaptive = true;
-    if (active_out) *active_out = ctx->prog_total;
+    if (rc) return frame_abort(ctx, rc);
+    f.n = ctx->h_active[0];
+    f.total = group ? ctx->h_active[1] : ctx->h_active[0];
+    if (test) f.adaptive = true;
+    if (active_out) *active_out = f.total;
     return SQT_OK;
 }
 
 extern "C" int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out) {
     if (!ctx) return SQT_E_INVALID;
-    if (!ctx->prog) return fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
+    if (!ctx->prog.on) return fail(ctx, SQT_E_INVALID, "no progressive frame in progress");
     if (!counts_out) return fail(ctx, SQT_E_INVALID, "counts_out is NULL");
     CU(cudaSetDevice(ctx->device));
-    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
-    const int k = ctx->prog_k;
+    const long long npix = (long long)ctx->prog.d.rows * ctx->prog.d.cols;
+    const int k = ctx->prog.k;
     if (const int *c = frame_counts(ctx)) {
         int rc = ensure_host_image(ctx, npix); if (rc) return rc;
         CU(cudaMemcpyAsync(ctx->h_accum, c, (size_t)npix * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1105,17 +1086,13 @@ extern "C" int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out) {
 // The denoiser reads the frame and writes only its own buffers: sums, moments, counts, the preview and the pixel list stay
 // as they are.  Its buffers are made on first use, before the group agreement, as ensure_progressive does.
 static int ensure_denoise(sqt_ctx *ctx, long long npix) {
-    if (npix <= ctx->cap_dn) return SQT_OK;
-    cudaFree(ctx->d_feat); cudaFree(ctx->d_sk); cudaFree(ctx->d_dn[0]); cudaFree(ctx->d_dn[1]); cudaFree(ctx->d_dn_mean); cudaFree(ctx->d_dn_rgb8);
-    ctx->d_feat = ctx->d_dn[0] = ctx->d_dn[1] = nullptr; ctx->d_sk = nullptr; ctx->d_dn_mean = nullptr; ctx->d_dn_rgb8 = nullptr;
-    ctx->cap_dn = 0; ctx->dn_frame = -1;
-    CU(cudaMalloc(&ctx->d_feat, (size_t)npix * sizeof(float4)));
-    CU(cudaMalloc(&ctx->d_sk, (size_t)npix * sizeof(int2)));
-    CU(cudaMalloc(&ctx->d_dn[0], (size_t)npix * sizeof(float4)));
-    CU(cudaMalloc(&ctx->d_dn[1], (size_t)npix * sizeof(float4)));
-    CU(cudaMalloc(&ctx->d_dn_mean, (size_t)npix * 12));
-    CU(cudaMalloc(&ctx->d_dn_rgb8, (size_t)npix * 3));
-    ctx->cap_dn = npix;
+    if ((size_t)npix > ctx->d_feat.cap || (size_t)npix > ctx->d_sk.cap) ctx->dn_frame = -1;     // new buffers hold no features
+    CU(ctx->d_feat.ensure(npix));
+    CU(ctx->d_sk.ensure(npix));
+    CU(ctx->d_dn[0].ensure(npix));
+    CU(ctx->d_dn[1].ensure(npix));
+    CU(ctx->d_dn_mean.ensure(npix * 3));
+    CU(ctx->d_dn_rgb8.ensure(npix * 3));
     return SQT_OK;
 }
 
@@ -1123,16 +1100,13 @@ static int ensure_denoise(sqt_ctx *ctx, long long npix) {
 // (download) agrees on levels = -1
 static int denoise_enter(sqt_ctx *ctx, bool download, int levels, float sigma_l, float sigma_z, uint32_t reserved, const char *what) {
     if (download) { levels = -1; sigma_l = sigma_z = 0.0f; reserved = 0; }
-    int rc = SQT_OK;
-    if (!ctx->prog) rc = fail(ctx, SQT_E_INVALID, "%s: no progressive frame in progress", what);
-    else if (!ctx->prog_d.primary_reuse) rc = fail(ctx, SQT_E_UNSUPPORTED, "%s needs primary reuse (not SQT_F_NO_PRIMARY_REUSE)", what);
-    else if (ctx->prog_k < 2) rc = fail(ctx, SQT_E_INVALID, "%s needs at least 2 samples per pixel (samples done: %d)", what, ctx->prog_k);
-    else if (!download && (levels > 8 || levels < 0)) rc = fail(ctx, SQT_E_INVALID, "%s: levels must be in 0..8", what);
-    else if (!download && (!(sigma_l > 0.0f) || !(sigma_l < INFINITY) || !(sigma_z > 0.0f) || !(sigma_z < INFINITY)))
+    int rc = check_variance_frame(ctx, what);
+    if (!rc && !download && (levels > 8 || levels < 0)) rc = fail(ctx, SQT_E_INVALID, "%s: levels must be in 0..8", what);
+    if (!rc && !download && (!(sigma_l > 0.0f) || !(sigma_l < INFINITY) || !(sigma_z > 0.0f) || !(sigma_z < INFINITY)))
         rc = fail(ctx, SQT_E_INVALID, "%s: sigma_l and sigma_z must be positive and finite", what);
-    else if (reserved) rc = fail(ctx, SQT_E_INVALID, "%s: reserved must be 0", what);
-    if (!rc) rc = ensure_denoise(ctx, (long long)ctx->prog_d.rows * ctx->prog_d.cols);
-    const int32_t keys[5] = {rc ? 0 : ctx->prog_k, rc ? 0 : ctx->prog_d.spp, rc ? 0 : levels, rc ? 0 : (int32_t)float_bits(sigma_l),
+    if (!rc && reserved) rc = fail(ctx, SQT_E_INVALID, "%s: reserved must be 0", what);
+    if (!rc) rc = ensure_denoise(ctx, (long long)ctx->prog.d.rows * ctx->prog.d.cols);
+    const int32_t keys[5] = {rc ? 0 : ctx->prog.k, rc ? 0 : ctx->prog.d.spp, rc ? 0 : levels, rc ? 0 : (int32_t)float_bits(sigma_l),
                              rc ? 0 : (int32_t)float_bits(sigma_z)};
     return group_agree(ctx, rc, keys, 5);
 }
@@ -1141,14 +1115,14 @@ static int denoise_enter(sqt_ctx *ctx, bool download, int levels, float sigma_l,
 // onto rank 0 -- every value is non-zero on its owner only, so the sum is exact.  Events 0 .. 2 bracket it.
 static int enqueue_features(sqt_ctx *ctx, uint32_t &nl) {
     cudaStream_t st = ctx->stream;
-    const RenderParams &d = ctx->prog_d;
+    const RenderParams &d = ctx->prog.d;
     const long long npix = (long long)d.rows * d.cols;
     CU(cudaEventRecord(ctx->ev[0], st));
     const bool need = ctx->dn_frame != ctx->prog_frame;
     if (need) {
         CU(cudaMemsetAsync(ctx->d_feat, 0, (size_t)npix * sizeof(float4), st));
         CU(cudaMemsetAsync(ctx->d_sk, 0, (size_t)npix * sizeof(int2), st));
-        const long long nwork = ctx->prog_pl.nwork;
+        const long long nwork = ctx->prog.pl.nwork;
         k_features<<<(int)((nwork + 255) / 256), 256, 0, st>>>(ctx->sc, d, ctx->d_prim, nwork, ctx->d_feat, ctx->d_sk);
         CU(cudaGetLastError()); nl++;
     }
@@ -1181,7 +1155,7 @@ extern "C" int sqt_denoise(sqt_ctx *ctx, const sqt_denoise_params *dp, uint8_t *
     int rc = dp ? denoise_enter(ctx, false, dp->levels, dp->sigma_l, dp->sigma_z, dp->reserved, "sqt_denoise")
                 : group_agree(ctx, fail(ctx, SQT_E_INVALID, "sqt_denoise: params are NULL"));
     if (rc) return rc;
-    const RenderParams &d = ctx->prog_d;
+    const RenderParams &d = ctx->prog.d;
     const long long npix = (long long)d.rows * d.cols;
     const bool root = ctx->rank == 0;
     cudaStream_t st = ctx->stream;
@@ -1189,13 +1163,13 @@ extern "C" int sqt_denoise(sqt_ctx *ctx, const sqt_denoise_params *dp, uint8_t *
     auto enqueue = [&]() -> int {
         int r = enqueue_features(ctx, nl); if (r) return r;
         if (root) {
-            k_denoise_prep<<<(int)((npix + 255) / 256), 256, 0, st>>>(frame_sums(ctx, false), frame_sums(ctx, true), npix, ctx->prog_k,
+            k_denoise_prep<<<(int)((npix + 255) / 256), 256, 0, st>>>(frame_sums(ctx, false), frame_sums(ctx, true), npix, ctx->prog.k,
                                                                      frame_counts(ctx), ctx->d_dn[0], ctx->d_dn_mean);
             CU(cudaGetLastError()); nl++;
             const dim3 grid((unsigned)((d.cols + 15) / 16), (unsigned)((d.rows + 15) / 16));
             for (int i = 0; i < dp->levels; ++i) {
                 k_denoise_level<<<grid, 256, 0, st>>>(ctx->d_dn[i & 1], ctx->d_feat, ctx->d_sk, d.rows, d.cols, 1 << i, dp->sigma_l, dp->sigma_z,
-                                                      ctx->d_dn[(i + 1) & 1], i + 1 == dp->levels ? ctx->d_dn_mean : nullptr);
+                                                      ctx->d_dn[(i + 1) & 1], i + 1 == dp->levels ? ctx->d_dn_mean.p : nullptr);
                 CU(cudaGetLastError()); nl++;
             }
             k_tonemap<<<(int)((npix + 255) / 256), 256, 0, st>>>(ctx->d_dn_mean, npix, 1.0f, ctx->d_dn_rgb8, nullptr);
@@ -1209,7 +1183,7 @@ extern "C" int sqt_denoise(sqt_ctx *ctx, const sqt_denoise_params *dp, uint8_t *
         return SQT_OK;
     };
     rc = enqueue();
-    if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+    if (rc) return frame_abort(ctx, rc);
     ctx->dn_frame = ctx->prog_frame;
     denoise_stats(ctx, stats, nl, root ? (uint64_t)npix * ((rgb8_out ? 3 : 0) + (mean_out ? 12 : 0)) : 0);
     return SQT_OK;
@@ -1220,7 +1194,7 @@ extern "C" int sqt_download_features(sqt_ctx *ctx, int32_t *surface_out, float *
     cudaSetDevice(ctx->device);
     int rc = denoise_enter(ctx, true, 0, 0.0f, 0.0f, 0u, "sqt_download_features");
     if (rc) return rc;
-    const long long npix = (long long)ctx->prog_d.rows * ctx->prog_d.cols;
+    const long long npix = (long long)ctx->prog.d.rows * ctx->prog.d.cols;
     uint32_t nl = 0;
     auto enqueue = [&]() -> int {
         int r = enqueue_features(ctx, nl); if (r) return r;
@@ -1229,7 +1203,7 @@ extern "C" int sqt_download_features(sqt_ctx *ctx, int32_t *surface_out, float *
         return SQT_OK;
     };
     rc = enqueue();
-    if (rc) { ctx->prog = false; ctx->img_pixels = 0; return group_abort(ctx, rc); }
+    if (rc) return frame_abort(ctx, rc);
     ctx->dn_frame = ctx->prog_frame;
     if (ctx->rank != 0 || (!surface_out && !depth_out && !normal_out)) return SQT_OK;
     std::vector<float4> f((size_t)npix);
@@ -1282,80 +1256,48 @@ extern "C" int sqt_comm_init_all(sqt_ctx **ctxs, int n) {
     return SQT_OK;
 }
 
-extern "C" int sqt_render_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const sqt_render_params *p,
-                                uint8_t *rgb8_out, float *accum_out, sqt_stats *stats) {
-    if (!ctxs || n < 1) return SQT_E_INVALID;
-    if (n == 1) return sqt_render(ctxs[0], cam, p, rgb8_out, accum_out, stats);
-    // one host thread per device: the ncclReduce calls of a single-process group must be issued concurrently
+// A call on every context of a single-process group, one host thread per device from ctxs[1] on (the collectives of such
+// a group must be issued concurrently) and ctxs[0] on the calling thread: call(ctx, root), root for ctxs[0] only, which
+// alone gets the outputs.  A failing rank's error is reported on ctxs[0].
+template <class F>
+static int fan_out(sqt_ctx **ctxs, int n, F call) {
+    if (!valid_group(ctxs, n)) return SQT_E_INVALID;
+    if (n == 1) return call(ctxs[0], true);
     std::vector<int> rcs(n, 0);
     std::vector<std::thread> th;
-    for (int i = 1; i < n; ++i)
-        th.emplace_back([&, i]() { rcs[i] = sqt_render(ctxs[i], cam, p, nullptr, nullptr, nullptr); });
-    rcs[0] = sqt_render(ctxs[0], cam, p, rgb8_out, accum_out, stats);
+    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = call(ctxs[i], false); });
+    rcs[0] = call(ctxs[0], true);
     for (auto &t : th) t.join();
     for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
     return SQT_OK;
 }
 
-// progressive frames on every context of a single-process group, one host thread per device like sqt_render_group
-// (rank 0 gets the progress and the stats)
+extern "C" int sqt_render_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const sqt_render_params *p,
+                                uint8_t *rgb8_out, float *accum_out, sqt_stats *stats) {
+    return fan_out(ctxs, n, [&](sqt_ctx *c, bool root) { return sqt_render(c, cam, p, root ? rgb8_out : nullptr, root ? accum_out : nullptr, root ? stats : nullptr); });
+}
+
 extern "C" int sqt_render_begin_group(sqt_ctx **ctxs, int n, const sqt_camera *cam, const sqt_render_params *p, sqt_stats *stats) {
-    if (!ctxs || n < 1) return SQT_E_INVALID;
-    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
-    if (n == 1) return sqt_render_begin(ctxs[0], cam, p, stats);
-    std::vector<int> rcs(n, 0);
-    std::vector<std::thread> th;
-    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_begin(ctxs[i], cam, p, nullptr); });
-    rcs[0] = sqt_render_begin(ctxs[0], cam, p, stats);
-    for (auto &t : th) t.join();
-    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
-    return SQT_OK;
+    return fan_out(ctxs, n, [&](sqt_ctx *c, bool root) { return sqt_render_begin(c, cam, p, root ? stats : nullptr); });
 }
 
 extern "C" int sqt_render_advance_group(sqt_ctx **ctxs, int n, int32_t n_samples, sqt_progress *progress, sqt_stats *stats) {
-    if (!ctxs || n < 1) return SQT_E_INVALID;
-    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
-    if (n == 1) return sqt_render_advance(ctxs[0], n_samples, progress, stats);
-    std::vector<int> rcs(n, 0);
-    std::vector<std::thread> th;
-    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_advance(ctxs[i], n_samples, nullptr, nullptr); });
-    rcs[0] = sqt_render_advance(ctxs[0], n_samples, progress, stats);
-    for (auto &t : th) t.join();
-    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
-    return SQT_OK;
+    return fan_out(ctxs, n, [&](sqt_ctx *c, bool root) { return sqt_render_advance(c, n_samples, root ? progress : nullptr, root ? stats : nullptr); });
 }
 
 extern "C" int sqt_render_retire_group(sqt_ctx **ctxs, int n, const sqt_retire_params *rp, int64_t *active_out) {
-    if (!ctxs || n < 1) return SQT_E_INVALID;
-    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
-    if (n == 1) return sqt_render_retire(ctxs[0], rp, active_out);
-    std::vector<int> rcs(n, 0);
-    std::vector<std::thread> th;
-    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_render_retire(ctxs[i], rp, nullptr); });
-    rcs[0] = sqt_render_retire(ctxs[0], rp, active_out);
-    for (auto &t : th) t.join();
-    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
-    return SQT_OK;
+    return fan_out(ctxs, n, [&](sqt_ctx *c, bool root) { return sqt_render_retire(c, rp, root ? active_out : nullptr); });
 }
 
 extern "C" int sqt_denoise_group(sqt_ctx **ctxs, int n, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats) {
-    if (!ctxs || n < 1) return SQT_E_INVALID;
-    for (int i = 0; i < n; ++i) if (!ctxs[i]) return SQT_E_INVALID;
-    if (n == 1) return sqt_denoise(ctxs[0], dp, rgb8_out, mean_out, stats);
-    std::vector<int> rcs(n, 0);
-    std::vector<std::thread> th;
-    for (int i = 1; i < n; ++i) th.emplace_back([&, i]() { rcs[i] = sqt_denoise(ctxs[i], dp, nullptr, nullptr, nullptr); });
-    rcs[0] = sqt_denoise(ctxs[0], dp, rgb8_out, mean_out, stats);
-    for (auto &t : th) t.join();
-    for (int i = 0; i < n; ++i) if (rcs[i]) { if (i) ctxs[0]->err = ctxs[i]->err; return rcs[i]; }
-    return SQT_OK;
+    return fan_out(ctxs, n, [&](sqt_ctx *c, bool root) { return sqt_denoise(c, dp, root ? rgb8_out : nullptr, root ? mean_out : nullptr, root ? stats : nullptr); });
 }
 
 // ------------------------------------------------------------------------------ roofline microbenchmarks
 extern "C" int sqt_measure_fp32_peak(sqt_ctx *ctx, double *gops) {
     if (!ctx || !gops) return SQT_E_INVALID;
     CU(cudaSetDevice(ctx->device));
-    float *d = nullptr; CU(cudaMalloc(&d, 16));
+    Buffer<float> d; CU(d.ensure(4));
     const int iters = 4096, grid = ctx->sm_count * 8, block = 256;
     cudaStream_t st = ctx->stream;
     double best = 0;
@@ -1369,7 +1311,6 @@ extern "C" int sqt_measure_fp32_peak(sqt_ctx *ctx, double *gops) {
         const double ops = (double)grid * block * iters * 32.0;
         if (rep > 0 && ops / ms * 1e-6 > best) best = ops / ms * 1e-6;
     }
-    cudaFree(d);
     *gops = best;
     return SQT_OK;
 }
@@ -1378,8 +1319,8 @@ extern "C" int sqt_measure_l2_bandwidth(sqt_ctx *ctx, double *gbs) {
     if (!ctx || !gbs) return SQT_E_INVALID;
     CU(cudaSetDevice(ctx->device));
     const long long bytes = 32ll << 20, n4 = bytes / 16;
-    float4 *buf = nullptr; float *out = nullptr;
-    CU(cudaMalloc(&buf, bytes)); CU(cudaMalloc(&out, 16));
+    Buffer<float4> buf; Buffer<float> out;
+    CU(buf.ensure(n4)); CU(out.ensure(4));
     CU(cudaMemset(buf, 0, bytes));
     cudaStream_t st = ctx->stream;
     const int grid = ctx->sm_count * 8, block = 256, reps = 16;
@@ -1394,7 +1335,6 @@ extern "C" int sqt_measure_l2_bandwidth(sqt_ctx *ctx, double *gbs) {
         const double gb = (double)bytes * reps / ms * 1e-6;
         if (rep > 0 && gb > best) best = gb;
     }
-    cudaFree(buf); cudaFree(out);
     *gbs = best;
     return SQT_OK;
 }

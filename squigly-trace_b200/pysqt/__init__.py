@@ -265,6 +265,23 @@ def camera_struct(cam12):
     return c
 
 
+def _advance(call):
+    """render_advance of a Context or a Group: call(progress, stats) makes the C call and checks it."""
+    pr, st = Progress(), Stats()
+    call(C.byref(pr), C.byref(st))
+    return dict(samples_done=pr.samples_done, samples_total=pr.samples_total, noise=pr.noise, stats=st.as_dict())
+
+
+def _denoise(shape, levels, sigma_l, sigma_z, call):
+    """denoise of a Context or a Group: call(params, rgb8, mean, stats) makes the C call and checks it."""
+    rows, cols = shape
+    dp, st = DenoiseParams(levels, sigma_l, sigma_z, 0), Stats()
+    rgb8 = np.zeros((rows, cols, 3), np.uint8)
+    mean = np.zeros((rows, cols, 3), np.float32)
+    call(C.byref(dp), _p(rgb8), _p(mean), C.byref(st))
+    return dict(rgb8=rgb8, mean=mean, stats=st.as_dict())
+
+
 class Context:
     """One sqt_ctx (one B200)."""
 
@@ -358,9 +375,7 @@ class Context:
 
     def render_advance(self, n_samples):
         """Trace the next n_samples samples per pixel of the progressive frame."""
-        pr, st = Progress(), Stats()
-        self._ck(self.L.sqt_render_advance(self.h, n_samples, C.byref(pr), C.byref(st)), "sqt_render_advance")
-        return dict(samples_done=pr.samples_done, samples_total=pr.samples_total, noise=pr.noise, stats=st.as_dict())
+        return _advance(lambda pr, st: self._ck(self.L.sqt_render_advance(self.h, n_samples, pr, st), "sqt_render_advance"))
 
     def download_moments(self, rows, cols):
         m2 = np.zeros((rows, cols, 3), np.float32)
@@ -381,12 +396,8 @@ class Context:
 
     def denoise(self, levels=DENOISE_LEVELS, sigma_l=DENOISE_SIGMA_L, sigma_z=DENOISE_SIGMA_Z):
         """Denoised preview of the progressive frame (include/sqt.h): returns rgb8, mean and stats.  The frame is unchanged."""
-        rows, cols = self._shape
-        dp, st = DenoiseParams(levels, sigma_l, sigma_z, 0), Stats()
-        rgb8 = np.zeros((rows, cols, 3), np.uint8)
-        mean = np.zeros((rows, cols, 3), np.float32)
-        self._ck(self.L.sqt_denoise(self.h, C.byref(dp), _p(rgb8), _p(mean), C.byref(st)), "sqt_denoise")
-        return dict(rgb8=rgb8, mean=mean, stats=st.as_dict())
+        return _denoise(self._shape, levels, sigma_l, sigma_z,
+                        lambda *a: self._ck(self.L.sqt_denoise(self.h, *a), "sqt_denoise"))
 
     def download_features(self, rows, cols):
         """Primary-hit AOVs of the progressive frame: surface (tri_out numbering, -1 = no hit), depth t, camera-facing normal."""
@@ -433,65 +444,51 @@ class Group:
     def __init__(self, devices):
         self.ctxs = [Context(d) for d in devices]
         self.arr = (C.c_void_p * len(self.ctxs))(*[c.h for c in self.ctxs])
-        L = b200()
-        rc = L.sqt_comm_init_all(self.arr, len(self.ctxs))
-        if rc:
-            raise SqtError("sqt_comm_init_all failed (%d): %s" % (rc, self.ctxs[0].last_error()))
-        self.L = L
+        self.L = b200()
+        self._ck(self.L.sqt_comm_init_all(self.arr, len(self.ctxs)), "sqt_comm_init_all")
         self._shape = (0, 0)
+
+    def _ck(self, rc, what):
+        if rc:
+            raise SqtError("%s failed (%d): %s" % (what, rc, self.ctxs[0].last_error()))
 
     def upload(self, scene):
         d = scene.desc() if hasattr(scene, "desc") else scene
         self._keep = scene
-        rc = self.L.sqt_upload_scene_group(self.arr, len(self.ctxs), C.byref(d))
-        if rc:
-            raise SqtError("sqt_upload_scene_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        self._ck(self.L.sqt_upload_scene_group(self.arr, len(self.ctxs), C.byref(d)), "sqt_upload_scene_group")
 
     def render(self, cam12, params, want_accum=True):
         cam = camera_struct(cam12)
         rgb8 = np.zeros((params.rows, params.cols, 3), np.uint8)
         accum = np.zeros((params.rows, params.cols, 3), np.float32) if want_accum else None
         st = Stats()
-        rc = self.L.sqt_render_group(self.arr, len(self.ctxs), C.byref(cam), C.byref(params), _p(rgb8), _p(accum), C.byref(st))
-        if rc:
-            raise SqtError("sqt_render_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        self._ck(self.L.sqt_render_group(self.arr, len(self.ctxs), C.byref(cam), C.byref(params), _p(rgb8), _p(accum), C.byref(st)),
+                 "sqt_render_group")
         return dict(rgb8=rgb8, accum=accum, stats=st.as_dict())
 
     def render_begin(self, cam12, params):
         cam = camera_struct(cam12)
         st = Stats()
         self._shape = (params.rows, params.cols)
-        rc = self.L.sqt_render_begin_group(self.arr, len(self.ctxs), C.byref(cam), C.byref(params), C.byref(st))
-        if rc:
-            raise SqtError("sqt_render_begin_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        self._ck(self.L.sqt_render_begin_group(self.arr, len(self.ctxs), C.byref(cam), C.byref(params), C.byref(st)),
+                 "sqt_render_begin_group")
         return st.as_dict()
 
     def render_advance(self, n_samples):
-        pr, st = Progress(), Stats()
-        rc = self.L.sqt_render_advance_group(self.arr, len(self.ctxs), n_samples, C.byref(pr), C.byref(st))
-        if rc:
-            raise SqtError("sqt_render_advance_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
-        return dict(samples_done=pr.samples_done, samples_total=pr.samples_total, noise=pr.noise, stats=st.as_dict())
+        return _advance(lambda pr, st: self._ck(self.L.sqt_render_advance_group(self.arr, len(self.ctxs), n_samples, pr, st),
+                                                "sqt_render_advance_group"))
 
     def render_retire(self, rel_tol, abs_tol=0.0, min_samples=MIN_SAMPLES):
         rp, act = RetireParams(rel_tol, abs_tol, min_samples, 0), C.c_int64()
-        rc = self.L.sqt_render_retire_group(self.arr, len(self.ctxs), C.byref(rp), C.byref(act))
-        if rc:
-            raise SqtError("sqt_render_retire_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
+        self._ck(self.L.sqt_render_retire_group(self.arr, len(self.ctxs), C.byref(rp), C.byref(act)), "sqt_render_retire_group")
         return act.value
 
     def download_sample_counts(self, rows, cols):
         return self.ctxs[0].download_sample_counts(rows, cols)
 
     def denoise(self, levels=DENOISE_LEVELS, sigma_l=DENOISE_SIGMA_L, sigma_z=DENOISE_SIGMA_Z):
-        rows, cols = self._shape
-        dp, st = DenoiseParams(levels, sigma_l, sigma_z, 0), Stats()
-        rgb8 = np.zeros((rows, cols, 3), np.uint8)
-        mean = np.zeros((rows, cols, 3), np.float32)
-        rc = self.L.sqt_denoise_group(self.arr, len(self.ctxs), C.byref(dp), _p(rgb8), _p(mean), C.byref(st))
-        if rc:
-            raise SqtError("sqt_denoise_group failed (%d): %s" % (rc, self.ctxs[0].last_error()))
-        return dict(rgb8=rgb8, mean=mean, stats=st.as_dict())
+        return _denoise(self._shape, levels, sigma_l, sigma_z,
+                        lambda *a: self._ck(self.L.sqt_denoise_group(self.arr, len(self.ctxs), *a), "sqt_denoise_group"))
 
     def download_features(self, rows, cols):
         """Every rank takes part (the first call of a frame sums the features onto rank 0); rank 0's result is returned."""
