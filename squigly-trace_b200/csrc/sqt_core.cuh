@@ -247,6 +247,45 @@ SQT_HD bool moller_trumbore_au(const float4 &a0, const float4 &a1, const float4 
     return pass_a && !neg && !big;
 }
 
+// ------------------------------------------------------------------------- exact culling margin
+// A-priori error bound of moller_trumbore (derivation: DESIGN.md section 5).  If the test accepts a triangle with edges
+// |e1|, |e2| <= E for a ray (o, d), the half-line o + t d, t >= 0, passes within
+//   delta = N E^2 (cS S + cE E) (1 + 2 krho N E^2)
+// of the triangle, where N >= |d|_2, S >= |o - v0|_1 and also >= |o_k - plane_k| for every plane of the box tested, and the
+// constants come from gamma_n bounds of the operation sequence (cS = 3 gamma_6 / 1e-4, cE = 2 sqrt3 gamma_5 / 1e-4,
+// krho = sqrt3 gamma_5 / 1e-4; the last factor covers the error of `a` itself).  cull_margin returns delta plus what the
+// rounding of the slab test needs, 2^-19 (|o|_inf + S) + kCullAbs, with n2 = 2N, P2 = n2 E^2 = 2 N E^2 and
+//   kCullC0 = cS / 2, kCullKappa = cE / cS, kCullC1 = kCullC0 krho,
+// all rounded up and C0 enlarged by (1 + 2^-19) so that the rounding of the margin's own 21 operations (all on
+// non-negative values) never leaves it below the bound.
+constexpr float kCullC0 = 0x1.5f9038p-8f, kCullC1 = 0x1.d092d0p-16f, kCullKappa = 0x1.ecac14p-1f;
+constexpr float kCullAbs = 1.0e-4f;
+SQT_HD float cull_margin(float n2, float E, float S, float omax) {
+    const float P2 = n2 * (E * E);
+    return P2 * (S + kCullKappa * E) * (kCullC0 + kCullC1 * P2) + (kCullAbs + 1.9073486328125e-6f * (omax + S));
+}
+// The margin of the leaf record (b0, b1) for ray r: N = (1 + |d|^2) / 2 >= |d| (exact for unit directions),
+// S = sum_k max(|o_k - lo_k|, |o_k - hi_k|) >= |o - v0|_1 for every v0 in the box.
+SQT_HD float leaf_margin(const float4 &b0, const float4 &b1, const Ray &r) {
+    const float S = fmaxf(fabsf(r.ox - b0.x), fabsf(r.ox - b0.w)) + fmaxf(fabsf(r.oy - b0.y), fabsf(r.oy - b1.x)) +
+                    fmaxf(fabsf(r.oz - b0.z), fabsf(r.oz - b1.y));
+    const float omax = fmaxf(fmaxf(fabsf(r.ox), fabsf(r.oy)), fabsf(r.oz));
+    const float n2 = 1.0f + (r.dx * r.dx + r.dy * r.dy + r.dz * r.dz);
+    return cull_margin(n2, b1.z, S, omax);
+}
+// Leaf culling: true if the ray provably misses the tight box (b0, b1) of a leaf record enlarged by leaf_margin, i.e. no
+// triangle of the leaf can be accepted.  Only for rays with finite direction components and reciprocals and finite
+// origins (`safe`); a NaN or infinite margin keeps the leaf.
+SQT_HD bool leaf_box_culled(const float4 &b0, const float4 &b1, const Ray &r, float dfx, float dfy, float dfz) {
+    const float m = leaf_margin(b0, b1, r);
+    const float lx = (b0.x - m - r.ox) * dfx, hx = (b0.w + m - r.ox) * dfx;
+    const float ly = (b0.y - m - r.oy) * dfy, hy = (b1.x + m - r.oy) * dfy;
+    const float lz = (b0.z - m - r.oz) * dfz, hz = (b1.y + m - r.oz) * dfz;
+    const float tmin = SQT_FMAX(SQT_FMAX(SQT_FMIN(lx, hx), SQT_FMIN(ly, hy)), SQT_FMIN(lz, hz));
+    const float tmax = SQT_FMIN(SQT_FMIN(SQT_FMAX(lx, hx), SQT_FMAX(ly, hy)), SQT_FMAX(lz, hz));
+    return tmax < 0.0f || tmin > tmax;          // a NaN anywhere keeps the leaf
+}
+
 // ------------------------------------------------------------------------------ leaf records
 // Leaf record (see "device records") of the leaf tris[first .. first + cnt): the tight box of the triangles as
 // Moller-Trumbore sees them (v0, v0 + e1, v0 + e2), rounded outwards, and their longest edge, rounded up.  Used only by
@@ -293,14 +332,13 @@ SQT_HD TightRec tight_union(const TightRec &a, const TightRec &b) {
     r.t1.z = fmaxf(a.t1.z, b.t1.z); r.t1.w = u2f(0u);
     return r;
 }
-// Margin: the leaf-culling bound (enter_step) with its per-ray quantities replaced by their maxima over tame rays --
-// |d|_1 (1 + |d|_1) <= 6, |origin - v0|_1 <= s_max = 3 x the root's 1-norm half extent, |coordinates| <= c_max:
-//   m = 0.03 * (s_max + E) * 6 * E^2 + 1e-4 + 2^-20 * (c_max + s_max), rounded up.
+// Margin: the leaf-culling margin (cull_margin) with its per-ray quantities replaced by their maxima over tame rays --
+// |d|_2 <= |d|_1 <= 2 (N = 2, n2 = 4), |origin - plane| and |origin - v0|_1 <= s_max = 3 x the root's 1-norm half extent,
+// |origin|_inf <= c_max + s_max (c_max = largest root coordinate).
 // The axis is the one on which the enlarged tight extent is the smallest fraction of the Branch's clipped box (c0, c1: the
 // box intersectBIH' passes down, BIH.hs:130-141); the slab is worth a test (return true) if that fraction is below ratio_max.
 SQT_HD bool make_slab(const TightRec &t, const float4 &c0, const float4 &c1, float s_max, float c_max, float ratio_max, float4 &slab) {
-    const float E = t.t1.z;
-    const float m = 1.001f * (0.03f * (s_max + E) * 6.0f * (E * E) + (1.0e-4f + 9.5367431640625e-7f * (c_max + s_max)));
+    const float m = cull_margin(4.0f, t.t1.z, s_max, c_max + s_max);
     const float tlo[3] = {t.t0.x, t.t0.y, t.t0.z}, thi[3] = {t.t0.w, t.t1.x, t.t1.y};
     const float clo[3] = {c0.x, c0.y, c0.z}, chi[3] = {c0.w, c1.x, c1.y};
     float best = 2.0f;
@@ -543,14 +581,10 @@ SQT_HD void start_ray(const SceneView &sc, TravLane &L, Counters *cn) {
 //
 // Conservative leaf culling (not in the reference; exact by a forward error bound, derivation in DESIGN.md section 5).
 // A triangle test can only return Just if |a| >= 1e-4 and the computed u, v, u+v pass their guards and t > 1e-4
-// (Geometry.hs:117-142).  With eps = 2^-24, E the longest edge in the leaf and s = origin - v0, every numerator is
-// a 3-term dot of a 2-term cross and is off by at most 12*eps*|d|*E*(|s|_1 + E); after the division by |a| >= 1e-4
-// an accepted hit lies, in exact arithmetic, within 0.0143*|d|*E^2*(|s|_1+E) of the triangle (origin at most that
-// far behind it).  The leaf is skipped only if the ray misses the leaf's tight box enlarged by
-// 0.03*|d|_1*(1+|d|_1)*E^2*(|s|_1+E)  (>= 2x the bound, 1-norm over-estimates)  +  1e-4 + 2^-20*(max|coord| + |s|_1):
-// no skipped triangle could have been accepted, so the traversal result is bit-identical (tests: culling on/off
-// agree on every ray; both agree with the oracle).  Rays with a zero/denormal/non-finite direction component
-// (`safe` false) are never culled.
+// (Geometry.hs:117-142); then the ray passes within the bound of cull_margin of the triangle.  The leaf is skipped only
+// if the ray misses the leaf's tight box enlarged by that margin (leaf_box_culled): no skipped triangle could have been
+// accepted, so the traversal result is bit-identical (tests: culling on/off agree on every ray; both agree with the
+// oracle).  Rays with a zero/non-finite direction component or reciprocal (`safe` false) are never culled.
 template <bool COUNT, class RA>
 SQT_HD void enter_step(const SceneView &sc, TravLane &L, const RA &ra, Counters *cn) {
     const float4 *lp = sc.leaves + 2 * (size_t)L.child;
@@ -560,22 +594,9 @@ SQT_HD void enter_step(const SceneView &sc, TravLane &L, const RA &ra, Counters 
     L.cur.tri = -1;
     if (count == 0u) { L.state = ST_RET; return; }                        // empty leaf -> Nothing (BIH.hs:107)
     if (sc.leaf_cull && !(L.rf & kRfUnsafe)) {
-        const Ray r = ra.ray();
         float dfx, dfy, dfz;
         ra.dfv(dfx, dfy, dfz);
-        const float d1 = fabsf(r.dx) + fabsf(r.dy) + fabsf(r.dz), dfac = d1 * (1.0f + d1);
-        const float E = b1.z;
-        const float s1 = fabsf(r.ox - 0.5f * (b0.x + b0.w)) + fabsf(r.oy - 0.5f * (b0.y + b1.x)) +
-                         fabsf(r.oz - 0.5f * (b0.z + b1.y)) + ((b0.w - b0.x) + (b1.x - b0.y) + (b1.y - b0.z));
-        const float cmax = fmaxf(fmaxf(fmaxf(fabsf(b0.x), fabsf(b0.w)), fmaxf(fabsf(b0.y), fabsf(b1.x))), fmaxf(fabsf(b0.z), fabsf(b1.y)));
-        const float m = 0.03f * (s1 + E) * dfac * (E * E) + (1.0e-4f + 9.5367431640625e-7f * (cmax + s1));
-        const float lx = (b0.x - m - r.ox) * dfx, hx = (b0.w + m - r.ox) * dfx;
-        const float ly = (b0.y - m - r.oy) * dfy, hy = (b1.x + m - r.oy) * dfy;
-        const float lz = (b0.z - m - r.oz) * dfz, hz = (b1.y + m - r.oz) * dfz;
-        const float tmin = SQT_FMAX(SQT_FMAX(SQT_FMIN(lx, hx), SQT_FMIN(ly, hy)), SQT_FMIN(lz, hz));
-        const float tmax = SQT_FMIN(SQT_FMIN(SQT_FMAX(lx, hx), SQT_FMAX(ly, hy)), SQT_FMAX(lz, hz));
-        // keep the leaf unless the ray clearly misses; a NaN (cannot happen for safe rays) keeps it too
-        if (tmax < 0.0f || tmin > tmax) {
+        if (leaf_box_culled(b0, b1, ra.ray(), dfx, dfy, dfz)) {
             if (COUNT) cn->leaves_culled += 1;
             L.state = ST_RET;
             return;
