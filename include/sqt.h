@@ -246,7 +246,7 @@ int sqt_download_moments(sqt_ctx *ctx, float *m2_out);   /* rows*cols*3 floats: 
  * sqt_render_advance   traces the active pixels only: stats.samples = active pixels * samples in the chunk.  With no
  *                      active pixel left it launches nothing (samples_done still moves on).
  * Errors: SQT_E_INVALID outside a frame, before k >= 2, for min_samples < 2, negative or NaN tolerances or non-zero
- * reserved; SQT_E_UNSUPPORTED for a frame begun with SQT_F_NO_PRIMARY_REUSE.  Whatever ends a frame ends its adaptive
+ * reserved; SQT_E_UNSUPPORTED for a frame begun with SQT_F_NO_PRIMARY_REUSE and without a lens (sqt_set_lens).  Whatever ends a frame ends its adaptive
  * state.  In a group every rank retires its own pixels from its own sums; ranks that disagree on k, the target spp or
  * any of the three criteria fail on every rank before anything runs.  The counts reach rank 0 by a sum over ranks, and
  * a group frame is bit-identical to one GPU's. */
@@ -294,7 +294,7 @@ int sqt_download_sample_counts(sqt_ctx *ctx, int32_t *counts_out);   /* rows*col
  *                        (t) and the camera-facing normal N (rows*cols*3) the filter uses -- AOVs for an external denoiser
  *                        too.  Any pointer may be NULL.
  * Errors: SQT_E_INVALID outside a frame, k < 2, levels outside 0..8, a sigma that is not positive and finite, non-zero
- * reserved; SQT_E_UNSUPPORTED for a frame begun with SQT_F_NO_PRIMARY_REUSE (it keeps no primary hits).
+ * reserved; SQT_E_UNSUPPORTED for a frame begun with SQT_F_NO_PRIMARY_REUSE or with a lens (it keeps no primary hits).
  * In a group every rank makes the same calls (sqt_download_features included); ranks that disagree on k, the target spp,
  * levels or the sigmas fail on every rank before anything runs.  The features reach rank 0 once per frame by a sum over
  * ranks (each value is non-zero on its owner only, so the sum is exact), and rank 0 filters the sums, moments and counts
@@ -307,6 +307,43 @@ typedef struct sqt_denoise_params {
 int sqt_denoise(sqt_ctx *ctx, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats_or_null);
 int sqt_denoise_group(sqt_ctx **ctxs, int n, const sqt_denoise_params *dp, uint8_t *rgb8_out, float *mean_out, sqt_stats *stats_or_null);
 int sqt_download_features(sqt_ctx *ctx, int32_t *surface_out, float *depth_out, float *normal_out);
+
+/* camera sampling (extension: the reference's makeRay, Lib.hs:107-114, sends every sample of a pixel along one ray
+ * through one point of the pixel): box-filtered pixels (anti-aliasing) and a thin lens (depth of field) ----------------
+ *
+ * sqt_set_lens sets the context's camera model; NULL restores the reference's pinhole (the default).  Invalid fields
+ * (jitter not 0 or 1, a negative or non-finite aperture, a non-positive or non-finite focus distance, non-zero reserved)
+ * are SQT_E_INVALID and leave the lens unchanged.  sqt_render, sqt_render_resident, sqt_render_group and
+ * sqt_render_begin[_group] read the lens when the frame starts; a progressive frame keeps the lens it began with.
+ * sqt_intersect_batch ignores it (it takes the caller's rays).
+ * The primary ray of sample k of pixel (y, x) in a frame with a lens set, s = spp*(x + y*seed_stride) + k the sample's
+ * stream, every operation one binary32 rounding in exactly this order, no contraction:
+ *   w0..w3 = Philox4x32-10(counter (s lo, s hi, 0, "SQTL" = 0x4C545153), key seed);  u_i = random_r01(w_i) (Lib.hs:183-188)
+ *     (the bounce draws use counter word "SQTR": they are untouched)
+ *   jx = jitter ? u0 - 0.5f : 0 ;  jy = jitter ? u1 - 0.5f : 0 ;  fx = (float)x + jx ;  fy = (float)y + jy
+ *   xo = (fx - ww/2) / ww ;  yo = (hh/2 - fy) / hh        with ww = (float)xdiv, hh = (float)ydiv (jx = 0: makeRay's bits)
+ *   o = position ;  d_i = ((0 + 1*R[i]) + xo*R[3+i]) + yo*R[6+i]          (rotVert, R = rotation, row-major)
+ *   aperture A == 0: the ray is (o, d).  Otherwise, with f = focus_distance:
+ *     r = A * sqrt(u2) ;  th = 6.2831855f * u3 ;  (sn, cs) = sqt_sincos(th)  (DESIGN.md section 6) ;  a = r*cs ;  b = r*sn
+ *     off_i = a*R[3+i] + b*R[6+i] ;  inv_f = 1/f ;  o'_i = o_i + off_i ;  d'_i = d_i - off_i*inv_f
+ *   so that o' + f*d' = o + f*d: every lens sample of an image point meets at ray parameter t = f (along the unnormalised
+ *   camera ray), the plane in focus.  The footprint of a jittered pixel is [x - 1/2, x + 1/2] x [y - 1/2, y + 1/2] around
+ *   the reference's sample point, so an anti-aliased frame stays registered with the pinhole frame.
+ * A frame with a lens set traces every owned pixel's primary ray for every sample: there is no primary pass and no primary
+ * reuse (SQT_F_NO_PRIMARY_REUSE changes nothing), and a pixel whose centre ray misses is sampled too.  rays_reference
+ * equals rays_traced.  Seeds stay keyed to the target spp, so a progressive lens frame's preview after k samples is the
+ * exact k-sample prefix and its final frame equals the one-shot lens frame bit for bit; sqt_render_retire works (every
+ * owned pixel starts active); a group frame is bit-identical to one GPU's.  SQT_E_UNSUPPORTED: cast mode (mode 1) with a
+ * lens, and sqt_denoise[_group] / sqt_download_features on a lens frame (they need the primary hits, which a lens frame
+ * does not trace; denoising lens frames is not supported).  In a group every rank must have the same lens (or none):
+ * ranks that disagree fail on every rank before anything is enqueued. */
+typedef struct sqt_lens {
+    uint32_t jitter;                     /* 0 or 1: box-filtered pixels */
+    float aperture_radius;               /* >= 0, finite, world units; 0 = pinhole */
+    float focus_distance;                /* > 0, finite: ray parameter t of the sharp plane along the unnormalised camera ray */
+    uint32_t reserved;                   /* 0 */
+} sqt_lens;                              /* 16 B */
+int sqt_set_lens(sqt_ctx *ctx, const sqt_lens *lens_or_null);
 
 /* measured roofline denominators on this device (microbenchmarks; see DESIGN.md) ------------- */
 int sqt_measure_fp32_peak(sqt_ctx *ctx, double *gops_per_s);     /* non-fused FADD/FMUL issue rate, Gop/s */

@@ -109,6 +109,7 @@ struct sqt_ctx {
     bool comm_broken = false;           // the communicator was aborted after a rank failed
     ProgFrame prog;
     long long prog_frame = 0;           // numbers the progressive frames of this context (sqt_render_begin); never reset
+    bool lens_set = false; sqt_lens lens = {};      // camera model of the frames this context starts (sqt_set_lens)
     Buffer<float> d_m2;                 // per-pixel second moment (npix * 3 floats)
     Buffer<float> d_red1, d_red2;       // rank 0 of a group: sums and moments of all ranks
     Buffer<double> d_noise; Pinned<double> h_noise;              // partial sums of k_frame_noise_part + the result (pinned copy)
@@ -124,7 +125,8 @@ struct sqt_ctx {
     ncclComm_t comm = nullptr;
 };
 
-// d_flag: word 0 the material check of an upload, words 1.. the group agreement (flag + up to seven keys as (v, -v))
+// d_flag: word 0 the material check of an upload, words 1.. the group agreement (flag + up to seven keys as (v, -v): the
+// lens and, for sqt_render_begin, samples done / target spp / chunk)
 constexpr int kFlagWords = 16;
 
 static thread_local std::string g_create_err;
@@ -446,6 +448,17 @@ extern "C" int sqt_set_option(sqt_ctx *ctx, int option, int value) {
     return fail(ctx, SQT_E_INVALID, "unknown option %d", option);
 }
 
+extern "C" int sqt_set_lens(sqt_ctx *ctx, const sqt_lens *l) {
+    if (!ctx) return SQT_E_INVALID;
+    if (!l) { ctx->lens_set = false; ctx->lens = sqt_lens{}; return SQT_OK; }
+    if (l->jitter > 1u) return fail(ctx, SQT_E_INVALID, "sqt_set_lens: jitter must be 0 or 1");
+    if (!(l->aperture_radius >= 0.0f) || !(l->aperture_radius < INFINITY)) return fail(ctx, SQT_E_INVALID, "sqt_set_lens: aperture_radius must be >= 0 and finite");
+    if (!(l->focus_distance > 0.0f) || !(l->focus_distance < INFINITY)) return fail(ctx, SQT_E_INVALID, "sqt_set_lens: focus_distance must be > 0 and finite");
+    if (l->reserved) return fail(ctx, SQT_E_INVALID, "sqt_set_lens: reserved must be 0");
+    ctx->lens = *l; ctx->lens_set = true;
+    return SQT_OK;
+}
+
 // ------------------------------------------------------------------------------ helpers
 // the device buffers of an image of npix pixels (the pixel list has 32 entries of slack)
 static int ensure_image(sqt_ctx *ctx, long long npix) {
@@ -473,10 +486,10 @@ static int persistent_grid(sqt_ctx *ctx, K kernel, long long nwork) {
 // k_paths_pool launch shape + the per-slot global state it needs.  `launch` false: only size the grid and make sure the
 // allocations exist (the pre-pass of a render, so that nothing can fail between the ranks' agreement and the collective).
 struct PoolPlan { int grid = 0; size_t smem = 0; int depth = 1, pm_stride = 8; };
-template <bool COUNT, int K>
+template <bool COUNT, int K, bool LENS>
 static int pool_step(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, int round, long long nitems, bool launch) {
     const size_t smem = (size_t)4 * (32 * K * PF_WORDS + 4 * (32 * K) / 4 + 64 + 8 + 8 + 32) * sizeof(uint32_t);
-    auto kern = k_paths_pool<COUNT, K>;
+    auto kern = k_paths_pool<COUNT, K, LENS>;
     if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
@@ -513,13 +526,18 @@ static int pool_step(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, i
     CU(cudaGetLastError());
     return SQT_OK;
 }
-template <bool COUNT>
+template <bool COUNT, bool LENS>
 static int pool_step_k(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, int round, long long nitems, bool launch) {
     switch (ctx->pool_k) {
-    case 1: return pool_step<COUNT, 1>(ctx, d, rd, round, nitems, launch);
-    case 2: return pool_step<COUNT, 2>(ctx, d, rd, round, nitems, launch);
-    default: return pool_step<COUNT, 4>(ctx, d, rd, round, nitems, launch);
+    case 1: return pool_step<COUNT, 1, LENS>(ctx, d, rd, round, nitems, launch);
+    case 2: return pool_step<COUNT, 2, LENS>(ctx, d, rd, round, nitems, launch);
+    default: return pool_step<COUNT, 4, LENS>(ctx, d, rd, round, nitems, launch);
     }
+}
+// the pool kernel of a frame: instrumented or not, lens frame (the sample's own primary ray) or pinhole
+static int pool_step_d(sqt_ctx *ctx, bool count, const RenderParams &d, const RoundInfo &rd, int round, long long nitems, bool launch) {
+    if (d.lens) return count ? pool_step_k<true, true>(ctx, d, rd, round, nitems, launch) : pool_step_k<false, true>(ctx, d, rd, round, nitems, launch);
+    return count ? pool_step_k<true, false>(ctx, d, rd, round, nitems, launch) : pool_step_k<false, false>(ctx, d, rd, round, nitems, launch);
 }
 static float ev_ms(cudaEvent_t a, cudaEvent_t b) { float ms = 0; cudaEventElapsedTime(&ms, a, b); return ms; }
 
@@ -581,6 +599,7 @@ static int check_params(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_pa
     if (p->max_depth < 1 || p->max_depth > SQT_MAX_DEPTH) return fail(ctx, SQT_E_UNSUPPORTED, "max_depth must be in 1..%d", SQT_MAX_DEPTH);
     if (p->mode != 0 && p->mode != 1) return fail(ctx, SQT_E_INVALID, "mode must be 0 (trace) or 1 (cast)");
     if ((long long)p->rows * p->cols > (1ll << 31)) return fail(ctx, SQT_E_UNSUPPORTED, "image too large");
+    if (ctx->lens_set && p->mode == 1) return fail(ctx, SQT_E_UNSUPPORTED, "cast mode (mode 1) has no lens: sqt_set_lens(ctx, NULL) first");
     return SQT_OK;
 }
 
@@ -593,6 +612,10 @@ static RenderParams to_device_params(const sqt_ctx *ctx, const sqt_camera *cam, 
     for (int k = 0; k < 3; ++k) d.cam_pos[k] = cam->position[k];
     for (int k = 0; k < 9; ++k) d.cam_rot[k] = cam->rotation[k];
     d.terminate_on_black = (ctx->terminate_on_black_ok && !(p->flags & SQT_F_NO_EARLY_TERMINATION)) ? 1 : 0;
+    if (ctx->lens_set) {                // every sample traces its own primary ray: no primary pass, no reuse
+        d.lens = 1; d.jitter = (int)ctx->lens.jitter; d.aperture = ctx->lens.aperture_radius; d.focus = ctx->lens.focus_distance;
+        d.primary_reuse = 0;
+    }
     return d;
 }
 
@@ -612,7 +635,7 @@ static int prepare_render(sqt_ctx *ctx, const RenderParams &d, bool count, bool 
     CU(ctx->d_sbuf.ensure((pl.sbytes > 0 ? pl.sbytes : 12) / sizeof(float)));
     if (ctx->pool_k > 0) {
         RoundInfo none = {};
-        rc = count ? pool_step_k<true>(ctx, d, none, 0, pl.nwork << pl.log2_s, false) : pool_step_k<false>(ctx, d, none, 0, pl.nwork << pl.log2_s, false);
+        rc = pool_step_d(ctx, count, d, none, 0, pl.nwork << pl.log2_s, false);
         if (rc) return rc;
     }
     return SQT_OK;
@@ -621,8 +644,8 @@ static int prepare_render(sqt_ctx *ctx, const RenderParams &d, bool count, bool 
 // Multi-rank contexts: all ranks learn whether every rank got through check_params + prepare_render, with a one-word
 // ncclAllReduce(max) -- a collective every rank reaches whatever happened to it locally.  Only if all agree is the
 // frame (and its ncclReduce) enqueued; otherwise every rank returns an error and nobody waits in a collective.
-// `keys` (progressive frames: samples done, target spp, end of the chunk) must be equal on every rank: each travels as
-// (v, -v) in the same all-reduce, so max(v) == -max(-v) holds exactly when all ranks agree.
+// `keys` (the lens; progressive frames: samples done, target spp, end of the chunk) must be equal on every rank: each
+// travels as (v, -v) in the same all-reduce, so max(v) == -max(-v) holds exactly when all ranks agree.
 static int group_agree(sqt_ctx *ctx, int rc_local, const int32_t *keys = nullptr, int n_keys = 0) {
     if (ctx->world <= 1 || !ctx->comm) return rc_local;
     if (ctx->comm_broken) return fail(ctx, SQT_E_NCCL, "the communicator of this group was aborted after an earlier failure");
@@ -645,10 +668,17 @@ static int group_agree(sqt_ctx *ctx, int rc_local, const int32_t *keys = nullptr
     if (out[0]) return fail(ctx, SQT_E_NCCL, "another rank of the group could not start this render; nothing was enqueued");
     for (int i = 0; i < n_keys; ++i)
         if ((int32_t)out[1 + 2 * i] != -(int32_t)out[2 + 2 * i])
-            return fail(ctx, SQT_E_INVALID, "the ranks of the group disagree on the progressive frame (samples done / target spp / chunk); nothing was enqueued");
+            return fail(ctx, SQT_E_INVALID, "the ranks of the group disagree on the frame (samples done / target spp / chunk / criteria / lens); nothing was enqueued");
     return SQT_OK;
 }
 // a failure after the agreement (a launch error) would leave the other ranks waiting in ncclReduce: abort the communicator
+// the lens as agreement keys: (set?, jitter, aperture bits, focus bits)
+static void lens_keys(const sqt_ctx *ctx, int32_t keys[4]) {
+    uint32_t a = 0, f = 0;
+    memcpy(&a, &ctx->lens.aperture_radius, 4); memcpy(&f, &ctx->lens.focus_distance, 4);
+    keys[0] = ctx->lens_set ? 1 : 0; keys[1] = ctx->lens_set ? (int32_t)ctx->lens.jitter : 0;
+    keys[2] = ctx->lens_set ? (int32_t)a : 0; keys[3] = ctx->lens_set ? (int32_t)f : 0;
+}
 static int group_abort(sqt_ctx *ctx, int rc) {
     if (rc && ctx->world > 1 && ctx->comm && !ctx->comm_broken) { nccl_api()->CommAbort(ctx->comm); ctx->comm_broken = true; }
     return rc;
@@ -658,7 +688,15 @@ static int group_abort(sqt_ctx *ctx, int rc) {
 // rounds, finish.  A one-shot frame is start + rounds [k0, k1) + finish; a progressive frame runs the start once and
 // rounds + finish once per chunk.  Events: 0 start, 1 after primary, 2 after paths, 3 after reduce, 4 after tonemap.
 
-// frame start: zero the stats and the sums, the primary pass
+// the pixels among the nwork work items of this rank: all but the padding of the last pixel group, which is their tail
+static long long owned_pixels(const RenderParams &d, long long nwork) {
+    const long long npix = (long long)d.rows * d.cols;
+    if (d.world <= 1 || d.split_samples) return npix;
+    const long long groups = (npix + 31) >> 5;
+    return (groups - 1) % d.world == d.rank ? nwork - (groups * 32 - npix) : nwork;
+}
+
+// frame start: zero the stats and the sums, the primary pass -- or, in a lens frame, the pixel list of every owned pixel
 static int enqueue_start(sqt_ctx *ctx, const RenderParams &d, bool count, const RenderPlan &pl, uint32_t &nl) {
     const long long npix = (long long)d.rows * d.cols;
     cudaStream_t st = ctx->stream;
@@ -668,6 +706,11 @@ static int enqueue_start(sqt_ctx *ctx, const RenderParams &d, bool count, const 
     if (d.mode == 0 && d.primary_reuse) {
         if (count) k_primary<true><<<persistent_grid(ctx, k_primary<true>, pl.nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_prim, ctx->d_pixel_list, ctx->d_stats, ctx->tune);
         else k_primary<false><<<persistent_grid(ctx, k_primary<false>, pl.nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_prim, ctx->d_pixel_list, ctx->d_stats, ctx->tune);
+        CU(cudaGetLastError()); nl++;
+    } else if (d.mode == 0 && d.lens) {
+        const long long n = owned_pixels(d, pl.nwork);
+        const long long blocks = (n + 255) / 256 < (long long)ctx->sm_count * 8 ? (n + 255) / 256 : (long long)ctx->sm_count * 8;
+        k_lens_list<<<blocks > 0 ? (int)blocks : 1, 256, 0, st>>>(d, n, ctx->d_pixel_list, ctx->d_stats);
         CU(cudaGetLastError()); nl++;
     }
     CU(cudaEventRecord(ctx->ev[1], st));
@@ -687,7 +730,7 @@ static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, long 
         return SQT_OK;
     }
     RoundInfo rd = {};
-    rd.pixel_list = d.primary_reuse ? ctx->d_pixel_list.p : nullptr;
+    rd.pixel_list = d.primary_reuse || d.lens ? ctx->d_pixel_list.p : nullptr;
     rd.prim = d.primary_reuse ? ctx->d_prim.p : nullptr;
     rd.n_slots = nwork; rd.slot_stride = nwork;
     rd.log2_s = log2_s;
@@ -699,9 +742,11 @@ static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, long 
         rd.k0 = k; rd.k1 = k + S < kb ? k + S : kb;
         CU(cudaMemsetAsync(ctx->d_sbuf, 0, (size_t)(nwork * (long long)(rd.k1 - rd.k0) * 12ll), st));
         if (ctx->pool_k > 0) {
-            rc = count ? pool_step_k<true>(ctx, d, rd, round, nwork << rd.log2_s, true) : pool_step_k<false>(ctx, d, rd, round, nwork << rd.log2_s, true);
+            rc = pool_step_d(ctx, count, d, rd, round, nwork << rd.log2_s, true);
             if (rc) return rc;
-        } else if (count) k_paths<true><<<persistent_grid(ctx, k_paths<true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
+        } else if (d.lens && count) k_paths<true, true><<<persistent_grid(ctx, k_paths<true, true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
+        else if (d.lens) k_paths<false, true><<<persistent_grid(ctx, k_paths<false, true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
+        else if (count) k_paths<true><<<persistent_grid(ctx, k_paths<true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
         else k_paths<false><<<persistent_grid(ctx, k_paths<false>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
         CU(cudaGetLastError()); nl++;
         if (m2) k_accumulate_m2<<<agrid > 0 ? agrid : 1, 256, 0, st>>>(d, rd, ctx->d_accum, m2, ctx->d_stats);
@@ -791,7 +836,9 @@ extern "C" int sqt_render_resident(sqt_ctx *ctx, const sqt_camera *cam, const sq
     RenderPlan pl;
     int rc = check_params(ctx, cam, p);
     if (!rc) { d = to_device_params(ctx, cam, p); rc = prepare_render(ctx, d, (p->flags & SQT_F_COUNT_WORK) != 0, false, pl); }
-    rc = group_agree(ctx, rc); if (rc) return rc;
+    int32_t keys[4];
+    lens_keys(ctx, keys);
+    rc = group_agree(ctx, rc, keys, 4); if (rc) return rc;
     uint32_t nl = 0;
     rc = enqueue_render(ctx, d, (p->flags & SQT_F_COUNT_WORK) != 0, pl, &nl); if (rc) return group_abort(ctx, rc);
     CU(cudaStreamSynchronize(ctx->stream));
@@ -831,7 +878,9 @@ extern "C" int sqt_render(sqt_ctx *ctx, const sqt_camera *cam, const sqt_render_
     RenderPlan pl;
     int rc = check_params(ctx, cam, p);
     if (!rc) { d = to_device_params(ctx, cam, p); rc = prepare_render(ctx, d, (p->flags & SQT_F_COUNT_WORK) != 0, true, pl); }
-    rc = group_agree(ctx, rc); if (rc) return rc;
+    int32_t keys[4];
+    lens_keys(ctx, keys);
+    rc = group_agree(ctx, rc, keys, 4); if (rc) return rc;
     const long long npix = (long long)d.rows * d.cols;
     uint32_t nl = 0;
     rc = enqueue_render(ctx, d, (p->flags & SQT_F_COUNT_WORK) != 0, pl, &nl); if (rc) return group_abort(ctx, rc);
@@ -901,11 +950,12 @@ static int frame_abort(sqt_ctx *ctx, int rc) {
     ctx->prog.on = false; ctx->img_pixels = 0;
     return group_abort(ctx, rc);
 }
-// what retire and the denoiser read, the primary hits and the per-pixel variance, needs a frame in progress, begun with
-// primary reuse, with k >= 2 samples
-static int check_variance_frame(sqt_ctx *ctx, const char *what) {
+// what retire and the denoiser read needs a frame in progress with k >= 2 samples and a pixel list (retire: primary reuse
+// or a lens frame) or the primary hits (the denoiser, `prim`: primary reuse, which a lens frame does not have)
+static int check_variance_frame(sqt_ctx *ctx, const char *what, bool prim) {
     if (!ctx->prog.on) return fail(ctx, SQT_E_INVALID, "%s: no progressive frame in progress", what);
-    if (!ctx->prog.d.primary_reuse) return fail(ctx, SQT_E_UNSUPPORTED, "%s needs primary reuse (not SQT_F_NO_PRIMARY_REUSE)", what);
+    if (prim && ctx->prog.d.lens) return fail(ctx, SQT_E_UNSUPPORTED, "%s needs primary hits, which a lens frame does not trace", what);
+    if (!ctx->prog.d.primary_reuse && !ctx->prog.d.lens) return fail(ctx, SQT_E_UNSUPPORTED, "%s needs primary reuse (not SQT_F_NO_PRIMARY_REUSE)", what);
     if (ctx->prog.k < 2) return fail(ctx, SQT_E_INVALID, "%s needs at least 2 samples per pixel (samples done: %d)", what, ctx->prog.k);
     return SQT_OK;
 }
@@ -924,8 +974,9 @@ extern "C" int sqt_render_begin(sqt_ctx *ctx, const sqt_camera *cam, const sqt_r
     if (!rc) { d = to_device_params(ctx, cam, p); rc = prepare_render(ctx, d, count, false, pl); }
     const long long npix = (long long)d.rows * d.cols;
     if (!rc) rc = ensure_progressive(ctx, npix);
-    const int32_t keys[3] = {0, rc ? 0 : p->spp, 0};
-    rc = group_agree(ctx, rc, keys, 3); if (rc) return rc;
+    int32_t keys[7] = {0, rc ? 0 : p->spp, 0};
+    lens_keys(ctx, keys + 3);
+    rc = group_agree(ctx, rc, keys, 7); if (rc) return rc;
     cudaStream_t st = ctx->stream;
     uint32_t nl = 0;
     auto enqueue = [&]() -> int {
@@ -1010,7 +1061,7 @@ static uint32_t float_bits(float f) { uint32_t u; memcpy(&u, &f, 4); return u; }
 extern "C" int sqt_render_retire(sqt_ctx *ctx, const sqt_retire_params *rp, int64_t *active_out) {
     if (!ctx) return SQT_E_INVALID;
     cudaSetDevice(ctx->device);
-    int rc = rp ? check_variance_frame(ctx, "sqt_render_retire") : fail(ctx, SQT_E_INVALID, "retire params are NULL");
+    int rc = rp ? check_variance_frame(ctx, "sqt_render_retire", false) : fail(ctx, SQT_E_INVALID, "retire params are NULL");
     if (!rc && rp->min_samples < 2) rc = fail(ctx, SQT_E_INVALID, "min_samples must be at least 2");
     if (!rc && (!(rp->rel_tol >= 0.0f) || !(rp->abs_tol >= 0.0f))) rc = fail(ctx, SQT_E_INVALID, "tolerances must be non-negative numbers");
     if (!rc && rp->reserved) rc = fail(ctx, SQT_E_INVALID, "reserved must be 0");
@@ -1100,7 +1151,7 @@ static int ensure_denoise(sqt_ctx *ctx, long long npix) {
 // (download) agrees on levels = -1
 static int denoise_enter(sqt_ctx *ctx, bool download, int levels, float sigma_l, float sigma_z, uint32_t reserved, const char *what) {
     if (download) { levels = -1; sigma_l = sigma_z = 0.0f; reserved = 0; }
-    int rc = check_variance_frame(ctx, what);
+    int rc = check_variance_frame(ctx, what, true);
     if (!rc && !download && (levels > 8 || levels < 0)) rc = fail(ctx, SQT_E_INVALID, "%s: levels must be in 0..8", what);
     if (!rc && !download && (!(sigma_l > 0.0f) || !(sigma_l < INFINITY) || !(sigma_z > 0.0f) || !(sigma_z < INFINITY)))
         rc = fail(ctx, SQT_E_INVALID, "%s: sigma_l and sigma_z must be positive and finite", what);

@@ -872,6 +872,8 @@ struct RenderParams {
     int rank, world, split_samples, primary_reuse;
     float cam_pos[3], cam_rot[9];
     int terminate_on_black;     // host proved C*L stays finite: a surface with surfColor == 0 ends the path exactly
+    int lens, jitter;           // camera sampling (sqt_set_lens): a lens is set; box-filtered pixels
+    float aperture, focus;      // lens radius (0 = pinhole) and focus distance
 };
 
 // makeRay (Lib.hs:107-114) + rotVert (Geometry.hs:104-107: row vector x matrix, sum = foldl (+) 0)
@@ -885,6 +887,38 @@ SQT_HD Ray make_ray(const RenderParams &p, int y, int x) {
     r.dx = XADD(XADD(XADD(0.0f, XMUL(1.0f, R[0])), XMUL(xo, R[3])), XMUL(yo, R[6]));
     r.dy = XADD(XADD(XADD(0.0f, XMUL(1.0f, R[1])), XMUL(xo, R[4])), XMUL(yo, R[7]));
     r.dz = XADD(XADD(XADD(0.0f, XMUL(1.0f, R[2])), XMUL(xo, R[5])), XMUL(yo, R[8]));
+    return r;
+}
+
+// the primary ray of the sample with generator seed `s` (spp*(x + y*seed_stride) + k) in a frame with a lens set: jittered
+// sample point, then a thin-lens offset, in the order include/sqt.h (sqt_set_lens) writes down
+SQT_HD Ray lens_ray(const RenderParams &p, int y, int x, unsigned long long s) {
+    uint32_t w[4];
+    philox4x32_10((uint32_t)s, (uint32_t)(s >> 32), 0u, 0x4C545153u, (uint32_t)p.seed, (uint32_t)(p.seed >> 32), w);
+    const float jx = p.jitter ? XSUB(random_r01(w[0]), 0.5f) : 0.0f;
+    const float jy = p.jitter ? XSUB(random_r01(w[1]), 0.5f) : 0.0f;
+    const float fx = XADD((float)x, jx), fy = XADD((float)y, jy);
+    const float ww = (float)p.xdiv, hh = (float)p.ydiv;
+    const float xo = XDIV(XSUB(fx, XDIV(ww, 2.0f)), ww);
+    const float yo = XDIV(XSUB(XDIV(hh, 2.0f), fy), hh);
+    const float *R = p.cam_rot;
+    Ray r;
+    r.ox = p.cam_pos[0]; r.oy = p.cam_pos[1]; r.oz = p.cam_pos[2];
+    r.dx = XADD(XADD(XADD(0.0f, XMUL(1.0f, R[0])), XMUL(xo, R[3])), XMUL(yo, R[6]));
+    r.dy = XADD(XADD(XADD(0.0f, XMUL(1.0f, R[1])), XMUL(xo, R[4])), XMUL(yo, R[7]));
+    r.dz = XADD(XADD(XADD(0.0f, XMUL(1.0f, R[2])), XMUL(xo, R[5])), XMUL(yo, R[8]));
+    if (p.aperture != 0.0f) {
+        const float rad = XMUL(p.aperture, XSQRT(random_r01(w[2])));
+        const float th = XMUL(6.2831855f, random_r01(w[3]));
+        float sn, cs;
+        sqt_sincos(th, sn, cs);
+        const float a = XMUL(rad, cs), b = XMUL(rad, sn), inv_f = XDIV(1.0f, p.focus);
+        const float offx = XADD(XMUL(a, R[3]), XMUL(b, R[6]));
+        const float offy = XADD(XMUL(a, R[4]), XMUL(b, R[7]));
+        const float offz = XADD(XMUL(a, R[5]), XMUL(b, R[8]));
+        r.ox = XADD(r.ox, offx); r.oy = XADD(r.oy, offy); r.oz = XADD(r.oz, offz);
+        r.dx = XSUB(r.dx, XMUL(offx, inv_f)); r.dy = XSUB(r.dy, XMUL(offy, inv_f)); r.dz = XSUB(r.dz, XMUL(offz, inv_f));
+    }
     return r;
 }
 

@@ -2,6 +2,7 @@
 //
 //   k_intersect_batch  : one lane per ray, grid-stride; batched Scene.intersect (Geometry.hs:64 / BIH.hs:101)
 //   k_primary          : one lane per pixel; makeRay (Lib.hs:107-114) + closest hit, cached per pixel
+//   k_lens_list        : the start of a lens frame: every owned pixel onto the pixel list (no primary pass)
 //   k_paths_pool       : the integrator: every warp owns a pool of 32*K rays in shared memory, keeps them in three
 //                        queues by the kind of step they need and serves one queue per round with all lanes (default)
 //   k_paths            : the integrator with one ray per lane and warp-synchronous phases (SQT_POOL=0)
@@ -232,6 +233,14 @@ __global__ void __launch_bounds__(128) k_primary(SceneView sc, RenderParams p, i
     flush_stats(ds, st, cn, COUNT);
 }
 
+// the start of a lens frame (no primary pass): every owned pixel, in work-item order, goes to the pixel list.  The padding
+// of the pixel-group partition is the tail of the work items, so the owned pixels are the first n_owned items.
+__global__ void __launch_bounds__(256) k_lens_list(RenderParams p, long long n_owned, int *__restrict__ pixel_list, DeviceStats *ds) {
+    for (long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x; w < n_owned; w += (long long)gridDim.x * blockDim.x)
+        pixel_list[w] = (int)work_to_pixel(p, w);
+    if (blockIdx.x == 0 && threadIdx.x == 0) ds->n_hit = (unsigned long long)n_owned;
+}
+
 struct DeviceFetch {
     unsigned long long *counter;
     long long n;
@@ -250,14 +259,14 @@ struct DeviceFetch {
 #define SQT_WL_MIN_BLOCKS 6
 #endif
 // One round of samples (sqt_paths.cuh): persistent lanes pull (pixel, sample) items from the round's counter.
-template <bool COUNT>
+template <bool COUNT, bool LENS = false>
 __global__ void __launch_bounds__(128, SQT_WL_MIN_BLOCKS) k_paths(SceneView sc, RenderParams p, RoundInfo rd, int round, DeviceStats *ds, Tune tn) {
     Counters cn = {};
     PathStats st = {0, 0, 0};
     if (rd.pixel_list) rd.n_slots = (long long)ds->n_hit;
     DeviceFetch fetch = {&ds->work_next[round], rd.n_slots << rd.log2_s};
     uint16_t pm[SQT_MAX_DEPTH];
-    PathPolicy<DeviceFetch> pol(p, rd, fetch, st, pm);
+    PathPolicy<DeviceFetch, LENS> pol(p, rd, fetch, st, pm);
     warp_loop<COUNT>(sc, pol, &cn, tn);
     flush_stats(ds, st, cn, COUNT);
 }
@@ -322,7 +331,7 @@ enum { PF_OX = 0, PF_OY, PF_OZ, PF_DX, PF_DY, PF_DZ, PF_DFX, PF_DFY, PF_DFZ, PF_
        PF_FLAGS, PF_WORDS };
 enum { KT = 0, KL = 1, KR = 2, KS = 3, KNONE = 4 };
 
-template <bool COUNT, int K>
+template <bool COUNT, int K, bool LENS = false>
 __global__ void __launch_bounds__(128, SQT_POOL_MIN_BLOCKS) k_paths_pool(SceneView sc, RenderParams p, RoundInfo rd, int round, DeviceStats *ds, PoolTune tn,
                                                     float4 *__restrict__ gstack, uint16_t *__restrict__ gpm, uint4 *__restrict__ gpath, int stack_depth, int pm_stride) {
     extern __shared__ uint32_t pool_smem[];
@@ -574,7 +583,7 @@ __global__ void __launch_bounds__(128, SQT_POOL_MIN_BLOCKS) k_paths_pool(SceneVi
                 q.saved_r = u2f(g1.x); q.saved_j = (int)(pf & 0xffffu) - 1;
                 q.any_emit = ((pf >> 16) & 1u) != 0u; q.in_flight = ((pf >> 17) & 1u) != 0u;
             }
-            path_regen_warp<COUNT>(sc, p, rd, fetch, st, q, gpm + (size_t)(gbase + slot) * (size_t)pm_stride, L, &cn, act);
+            path_regen_warp<COUNT, LENS>(sc, p, rd, fetch, st, q, gpm + (size_t)(gbase + slot) * (size_t)pm_stride, L, &cn, act);
             if (act) {
                 PW(PF_OX, slot) = f2u(L.r.ox); PW(PF_OY, slot) = f2u(L.r.oy); PW(PF_OZ, slot) = f2u(L.r.oz);
                 PW(PF_DX, slot) = f2u(L.r.dx); PW(PF_DY, slot) = f2u(L.r.dy); PW(PF_DZ, slot) = f2u(L.r.dz);

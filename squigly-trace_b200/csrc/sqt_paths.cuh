@@ -131,9 +131,10 @@ SQT_HD void path_finish(const SceneView &sc, const RoundInfo &rd, const uint16_t
     g.htri = -1;
 }
 // B2: next sample.  0 = the queue is empty, 1 = item skipped (padding / beyond the sample range) -- fetch again,
-//     2 = the primary hit is known (shade it), 3 = the primary ray has to be traced (primary reuse off)
+//     2 = the primary hit is known (shade it), 3 = the primary ray has to be traced (primary reuse off, or a lens frame:
+//     LENS, whose primary ray is the sample's own, lens_ray)
 enum : int { NS_EMPTY = 0, NS_SKIP = 1, NS_SHADE = 2, NS_TRACE = 3 };
-template <class Fetch>
+template <bool LENS, class Fetch>
 SQT_HD int path_next_sample(const RenderParams &p, const RoundInfo &rd, Fetch &fetch, PathStats &st, PathRay &q, TravLane &L, RegenLane &g) {
     const long long w = fetch();
     if (w < 0) return NS_EMPTY;
@@ -148,6 +149,11 @@ SQT_HD int path_next_sample(const RenderParams &p, const RoundInfo &rd, Fetch &f
                + (unsigned long long)k;
     q.sidx = (uint32_t)((long long)ks * rd.slot_stride + slot);
     q.any_emit = false; q.saved_j = -1;
+    if constexpr (LENS) {
+        L.r = lens_ray(p, py, px, q.stream);
+        q.j = -1; q.in_flight = true;
+        return NS_TRACE;
+    }
     L.r = make_ray(p, py, px);
     if (rd.prim) {
         // the primary ray is the same for every sample of a pixel (Lib.hs:81): its hit was traced once
@@ -183,7 +189,7 @@ SQT_HD void path_bounce(const SceneView &sc, const RenderParams &p, PathRay &q, 
 // called when L.state == ST_DONE: consume the hit (if a ray was in flight), then shade / start the next sample until
 // the slot has a ray to trace (-> start_ray) or the queue is empty (-> ST_EXIT).  pm: SQT_MAX_DEPTH entries of
 // ray-private memory holding the material of every shaded bounce of the current path.
-template <bool COUNT, class Fetch>
+template <bool COUNT, bool LENS, class Fetch>
 SQT_HD void path_regen(const SceneView &sc, const RenderParams &p, const RoundInfo &rd, Fetch &fetch, PathStats &st, PathRay &q,
                        uint16_t *pm, TravLane &L, Counters *cn) {
     RegenLane g;
@@ -191,7 +197,7 @@ SQT_HD void path_regen(const SceneView &sc, const RenderParams &p, const RoundIn
     for (;;) {
         if (path_over) { path_finish(sc, rd, pm, q, st, g); path_over = false; }
         if (g.htri < 0) {
-            const int ns = path_next_sample(p, rd, fetch, st, q, L, g);
+            const int ns = path_next_sample<LENS>(p, rd, fetch, st, q, L, g);
             if (ns == NS_EMPTY) { L.state = ST_EXIT; return; }
             if (ns == NS_SKIP) continue;
             if (ns == NS_TRACE) { start_ray<COUNT>(sc, L, cn); return; }
@@ -206,7 +212,7 @@ SQT_HD void path_regen(const SceneView &sc, const RenderParams &p, const RoundIn
 #if defined(__CUDACC__)
 // The same for all lanes of a warp at once (`mine`: this lane is ST_DONE): every stage is one convergent block, the
 // loop is closed by a warp vote.  Per lane the sequence of stage calls is exactly path_regen's.
-template <bool COUNT, class Fetch>
+template <bool COUNT, bool LENS, class Fetch>
 __device__ __forceinline__ void path_regen_warp(const SceneView &sc, const RenderParams &p, const RoundInfo &rd, Fetch &fetch, PathStats &st,
                                                 PathRay &q, uint16_t *pm, TravLane &L, Counters *cn, bool mine) {
     RegenLane g;
@@ -220,7 +226,7 @@ __device__ __forceinline__ void path_regen_warp(const SceneView &sc, const Rende
     for (;;) {
         if (fin) { path_finish(sc, rd, pm, q, st, g); fin = false; nxt = true; }
         if (nxt) {
-            const int ns = path_next_sample(p, rd, fetch, st, q, L, g);
+            const int ns = path_next_sample<LENS>(p, rd, fetch, st, q, L, g);
             if (ns == NS_EMPTY) { L.state = ST_EXIT; nxt = false; }
             else if (ns == NS_SHADE) { nxt = false; shd = true; }
             else if (ns == NS_TRACE) { nxt = false; trace = true; }
@@ -236,7 +242,8 @@ __device__ __forceinline__ void path_regen_warp(const SceneView &sc, const Rende
 }
 #endif
 
-template <class Fetch>
+// LENS: a frame with a lens set (sqt_set_lens) -- a compile-time choice, so that the pinhole kernels stay as they are
+template <class Fetch, bool LENS = false>
 struct PathPolicy {
     const RenderParams &p;
     const RoundInfo &rd;
@@ -247,12 +254,12 @@ struct PathPolicy {
     SQT_HD PathPolicy(const RenderParams &p_, const RoundInfo &rd_, Fetch &f_, PathStats &st_, uint16_t *pm_)
         : p(p_), rd(rd_), fetch(f_), st(st_), pm(pm_) { path_ray_init(q); }
     template <bool COUNT>
-    SQT_HD void regen(const SceneView &sc, TravLane &L, Counters *cn) { path_regen<COUNT>(sc, p, rd, fetch, st, q, pm, L, cn); }
+    SQT_HD void regen(const SceneView &sc, TravLane &L, Counters *cn) { path_regen<COUNT, LENS>(sc, p, rd, fetch, st, q, pm, L, cn); }
 #if defined(__CUDACC__)
     static constexpr bool kWarpRegen = true;
     template <bool COUNT>
     __device__ __forceinline__ void regen_warp(const SceneView &sc, TravLane &L, Counters *cn, bool mine) {
-        path_regen_warp<COUNT>(sc, p, rd, fetch, st, q, pm, L, cn, mine);
+        path_regen_warp<COUNT, LENS>(sc, p, rd, fetch, st, q, pm, L, cn, mine);
     }
 #endif
 };

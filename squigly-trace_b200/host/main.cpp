@@ -1,7 +1,7 @@
 // main.cpp -- the squigly-trace command line (app/Main.hs:13-75) driving the B200 backend.
 // Flags follow the cmdargs record of the reference: -s/--samples, -d/--dimensions W,H, -p/--savepath,
 // --objpath, -c/--camerapath, --debug, --debugpath, --cast ; plus --bounces, --gpus, --corrected, --seed, --progress,
-// --adaptive, --denoise.
+// --adaptive, --denoise, --aa, --lens.
 #include <cctype>
 #include <chrono>
 #include <climits>
@@ -36,6 +36,9 @@ static void usage() {
                  "                         standard error is below max(REL * mean, ABS) (after at least MIN samples, default 16)\n"
                  "     --denoise[=LEVELS]  With --progress: also save <savepath stem>-denoised.png after each chunk, filtered\n"
                  "                         with LEVELS (0..8, default 5) levels of the edge-aware denoiser\n"
+                 "     --aa                Anti-aliasing: jitter every sample over its pixel (box filter)\n"
+                 "     --lens=APERTURE,FOCUS  Depth of field: thin lens of radius APERTURE (>= 0) focused at ray parameter\n"
+                 "                         FOCUS (> 0) along the camera ray\n"
                  "  -? --help              Display help message\n";
 }
 
@@ -44,6 +47,23 @@ static std::string showTime() {      // formatTime defaultTimeLocale "%T%P UTC"
     char buf[64];
     std::strftime(buf, sizeof buf, "%T%P UTC", std::gmtime(&t));
     return buf;
+}
+
+// --lens=APERTURE,FOCUS: a finite aperture >= 0 and a finite focus distance > 0
+static void parseLens(const std::string &v, Settings &st) {
+    const std::runtime_error bad("Could not parse --lens=" + v + ", expected APERTURE,FOCUS with a number APERTURE >= 0 and a number FOCUS > 0");
+    const size_t c = v.find(',');
+    if (c == std::string::npos) throw bad;
+    auto num = [&](const std::string &s) {
+        if (s.empty() || !(std::isdigit((unsigned char)s[0]) || s[0] == '.')) throw bad;
+        char *e = nullptr;
+        const double d = std::strtod(s.c_str(), &e);
+        if (*e || !std::isfinite(d) || !std::isfinite((float)d)) throw bad;
+        return (float)d;
+    };
+    st.aperture = num(v.substr(0, c));
+    st.focus = num(v.substr(c + 1));
+    if (!(st.focus > 0.0f)) throw bad;
 }
 
 // --adaptive=REL[,ABS[,MIN]]: finite non-negative tolerances, MIN an integer >= 2
@@ -114,11 +134,16 @@ int main(int argc, char **argv) {
                     st.denoise = val[0] - '0';
                 }
             }
+            else if (a == "--aa") st.aa = true;
+            else if (a == "--lens") parseLens(need(), st);
             else if (a == "-?" || a == "--help") { usage(); return 0; }
             else throw std::runtime_error("Unknown flag: " + a);
         }
         if (st.adaptive && st.progress < 1) throw std::runtime_error("--adaptive needs --progress=N");
         if (st.denoise >= 0 && st.progress < 1) throw std::runtime_error("--denoise needs --progress=N");
+        if (st.denoise >= 0 && (st.aa || st.focus > 0.0f))
+            throw std::runtime_error("--denoise cannot be combined with --aa or --lens: the denoiser needs the primary hits, which such frames do not trace");
+        if (st.cast && (st.aa || st.focus > 0.0f)) throw std::runtime_error("--cast cannot be combined with --aa or --lens");
         // main (Main.hs:35-47)
         const Camera cam = loadCamera(st.cameraPath);
         // loadBIH (Main.hs:63-75)

@@ -79,6 +79,13 @@ sqt_render_params paramsFromSettings(const Settings &s) {
     return p;
 }
 
+// --aa / --lens: the same camera model on every GPU of the run (sqt_set_lens); without either, the reference's pinhole
+static void setLens(const DeviceBIH &g, const Settings &s) {
+    const bool on = s.aa || s.focus > 0.0f;
+    const sqt_lens l{s.aa ? 1u : 0u, s.aperture, s.focus > 0.0f ? s.focus : 1.0f, 0u};
+    for (int k = 0; k < g.gpus(); ++k) g.check(k, sqt_set_lens(g.ctx(k), on ? &l : nullptr), "sqt_set_lens");
+}
+
 RenderReport renderToBuffer(const SceneBIH &scene, const Camera &cam, const Settings &settings, std::vector<uint8_t> &rgb8,
                             std::vector<float> *accum) {
     const sqt_render_params p = paramsFromSettings(settings);
@@ -89,6 +96,7 @@ RenderReport renderToBuffer(const SceneBIH &scene, const Camera &cam, const Sett
     rgb8.assign((size_t)p.rows * p.cols * 3, 0);
     if (accum) accum->assign((size_t)p.rows * p.cols * 3, 0.0f);
     const DeviceBIH &g = *scene.geometry;
+    setLens(g, settings);
     g.check(0, sqt_render_group(g.ctxs(), g.gpus(), &c, &p, rgb8.data(), accum ? accum->data() : nullptr, &rep.stats), "sqt_render");
     return rep;
 }
@@ -115,6 +123,7 @@ static RenderReport renderProgressive(const SceneBIH &scene, const Camera &cam, 
     std::vector<uint8_t> img((size_t)p.rows * p.cols * 3, 0);
     const DeviceBIH &g = *scene.geometry;
     const auto t0 = std::chrono::steady_clock::now();
+    setLens(g, settings);
     g.check(0, sqt_render_begin_group(g.ctxs(), g.gpus(), &c, &p, &rep.stats), "sqt_render_begin");
     sqt_progress pr{0, p.spp, 0.0};
     const sqt_retire_params rp{settings.adaptiveRel, settings.adaptiveAbs, settings.adaptiveMin, 0u};

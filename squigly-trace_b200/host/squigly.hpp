@@ -107,6 +107,8 @@ struct Settings {
     float adaptiveRel = 0.0f, adaptiveAbs = 0.0f;
     int adaptiveMin = 16;
     int denoise = -1;           // with progress: >= 0 also writes <stem>-denoised.png after every chunk (sqt_denoise levels)
+    bool aa = false;            // box-filtered pixels (sqt_set_lens jitter)
+    float aperture = 0.0f, focus = 0.0f;    // --lens=APERTURE,FOCUS (focus > 0: a thin lens is set)
 };
 struct RenderReport { sqt_stats stats{}; int rows = 0, cols = 0; };
 // render :: Scene a -> Camera -> Settings -> IO ()   (Lib.hs:68-75): computes the image on the device(s) and writes it

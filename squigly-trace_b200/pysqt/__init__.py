@@ -30,7 +30,7 @@ ABI_SYMBOLS = [
     "sqt_comm_init_all", "sqt_render_group", "sqt_measure_fp32_peak", "sqt_measure_l2_bandwidth", "sqt_device_info", "sqt_set_option", "sqt_upload_spheres",
     "sqt_upload_scene_group", "sqt_last_upload", "sqt_render_begin", "sqt_render_advance", "sqt_render_begin_group",
     "sqt_render_advance_group", "sqt_download_moments", "sqt_render_retire", "sqt_render_retire_group",
-    "sqt_download_sample_counts", "sqt_denoise", "sqt_denoise_group", "sqt_download_features",
+    "sqt_download_sample_counts", "sqt_denoise", "sqt_denoise_group", "sqt_download_features", "sqt_set_lens",
 ]
 
 
@@ -96,6 +96,10 @@ class DenoiseParams(C.Structure):
 DENOISE_LEVELS, DENOISE_SIGMA_L, DENOISE_SIGMA_Z = 5, 4.0, 0.05     # defaults of denoise and of the CLI's --denoise
 
 
+class Lens(C.Structure):
+    _fields_ = [("jitter", C.c_uint32), ("aperture_radius", C.c_float), ("focus_distance", C.c_float), ("reserved", C.c_uint32)]
+
+
 NODE_DT = np.dtype([("lmax", "<f4"), ("rmin", "<f4"), ("a", "<u4"), ("b", "<u4")])
 TRI_DT = np.dtype([("v0", "<f4", 3), ("e1", "<f4", 3), ("e2", "<f4", 3), ("material", "<u4"), ("orig_index", "<u4"), ("pad", "<u4")])
 SPHERE_DT = np.dtype([("center", "<f4", 3), ("radius", "<f4"), ("material", "<u4"), ("pad", "<u4", 3)])
@@ -150,6 +154,7 @@ def b200():
         L.sqt_denoise.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqt_denoise_group.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.sqt_download_features.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.sqt_set_lens.argtypes = [C.c_void_p, C.c_void_p]
         L.sqt_device_info.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_char_p]
         for name in ABI_SYMBOLS:
             if name not in ("sqt_last_error",):
@@ -423,6 +428,12 @@ class Context:
     def set_leaf_cull(self, on):
         self._ck(self.L.sqt_set_option(self.h, 1, 1 if on else 0), "sqt_set_option")
 
+    def set_lens(self, jitter=False, aperture=0.0, focus=1.0):
+        """Camera sampling of the frames this context starts (include/sqt.h, sqt_set_lens): box-filtered pixels and a thin
+        lens of radius `aperture` focused at ray parameter `focus`.  set_lens(None) restores the reference's pinhole."""
+        lens = None if jitter is None else Lens(int(bool(jitter)), aperture, focus, 0)
+        self._ck(self.L.sqt_set_lens(self.h, C.byref(lens) if lens is not None else None), "sqt_set_lens")
+
     def comm_init(self, rank, world, uid):
         buf = (C.c_uint8 * SQT_COMM_ID_BYTES).from_buffer_copy(bytes(uid))
         self._ck(self.L.sqt_comm_init(self.h, rank, world, buf), "sqt_comm_init")
@@ -485,6 +496,11 @@ class Group:
 
     def download_sample_counts(self, rows, cols):
         return self.ctxs[0].download_sample_counts(rows, cols)
+
+    def set_lens(self, jitter=False, aperture=0.0, focus=1.0):
+        """The same lens on every context of the group (set_lens(None): the pinhole)."""
+        for c in self.ctxs:
+            c.set_lens(jitter, aperture, focus)
 
     def denoise(self, levels=DENOISE_LEVELS, sigma_l=DENOISE_SIGMA_L, sigma_z=DENOISE_SIGMA_Z):
         return _denoise(self._shape, levels, sigma_l, sigma_z,
