@@ -99,12 +99,9 @@ struct sqt_ctx {
     // pinned host staging for image I/O
     Pinned<uint8_t> h_rgb8; Pinned<float> h_accum;
     Tune tune = {12, 0, 12};
-    int pool_k = 2;                     // 0: one ray per lane (k_paths) ; K > 0: ray pools of 32*K rays per warp (k_paths_pool)
     PoolTune pool_tune = {4, 10, 16};
-    int pool_blocks = 0;                // cap on resident CTAs per SM for k_paths_pool (0 = occupancy limit); fewer CTAs leave more L1
     float slab_ratio = kSlabRatioMax, slab_ratio_leaf = kSlabRatioMaxLeaf;   // subtree / leaf slabs: test a slab when it is at most this
                                                                              // fraction of the clipped box (SQT_SLAB_RATIO=branch[,leaf], 0 = never)
-    int pool_carveout = 0;              // shared-memory carve-out of k_paths_pool in percent of 228 KB (0 = the driver's choice)
     Buffer<float4> d_gstack; Buffer<uint16_t> d_gpm; Buffer<uint4> d_gpath;     // per pool slot: stack, materials, path state
     bool comm_broken = false;           // the communicator was aborted after a rank failed
     ProgFrame prog;
@@ -148,8 +145,6 @@ static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v
 // Environment knobs (development only; they change scheduling, never a result).  Malformed values are ignored and every
 // value is clamped to a range in which the persistent kernels are guaranteed to make progress.
 static void read_env_tuning(sqt_ctx *c) {
-    if (const char *t = getenv("SQT_POOL")) { char *e = nullptr; long k = strtol(t, &e, 10); if (e != t && k >= 0 && k <= 4) c->pool_k = k == 3 ? 4 : (int)k; }      // rays per warp = 32 * K, K a power of two
-    if (const char *t = getenv("SQT_POOL_BLOCKS")) { char *e = nullptr; long k = strtol(t, &e, 10); if (e != t && k >= 0 && k <= 32) c->pool_blocks = (int)k; }
     if (const char *t = getenv("SQT_SLAB_RATIO")) {
         char *e = nullptr; double v = strtod(t, &e);
         if (e != t && v >= 0.0 && v <= 2.0) {
@@ -157,7 +152,6 @@ static void read_env_tuning(sqt_ctx *c) {
             if (*e == ',') { const char *u = e + 1; double w = strtod(u, &e); if (e != u && w >= 0.0 && w <= 2.0) c->slab_ratio_leaf = (float)w; }
         }
     }
-    if (const char *t = getenv("SQT_POOL_CARVEOUT")) { char *e = nullptr; long k = strtol(t, &e, 10); if (e != t && k >= 0 && k <= 100) c->pool_carveout = (int)k; }
     if (const char *t = getenv("SQT_POOL_TUNE")) {       // "burst_t,t_leave,c_min"
         int a, b, cm;
         if (sscanf(t, "%d,%d,%d", &a, &b, &cm) == 3) c->pool_tune = {clampi(a, 1, 64), clampi(b, 0, 31), clampi(cm, 1, 32)};
@@ -485,25 +479,16 @@ static int persistent_grid(sqt_ctx *ctx, K kernel, long long nwork) {
 }
 // k_paths_pool launch shape + the per-slot global state it needs.  `launch` false: only size the grid and make sure the
 // allocations exist (the pre-pass of a render, so that nothing can fail between the ranks' agreement and the collective).
-struct PoolPlan { int grid = 0; size_t smem = 0; int depth = 1, pm_stride = 8; };
-template <bool COUNT, int K, bool LENS>
+template <bool COUNT, bool LENS>
 static int pool_step(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, int round, long long nitems, bool launch) {
-    const size_t smem = (size_t)4 * (32 * K * PF_WORDS + 4 * (32 * K) / 4 + 64 + 8 + 8 + 32) * sizeof(uint32_t);
-    auto kern = k_paths_pool<COUNT, K, LENS>;
+    const size_t smem = kPoolSmemBytes;
+    auto kern = k_paths_pool<COUNT, LENS>;
     if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 128, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-    if (ctx->pool_blocks > 0 && ctx->pool_blocks < per_sm) {
-        // keep the rest of the 228 KB for L1: the triangle / node / stack working set lives there
-        per_sm = ctx->pool_blocks;
-        int pct = (int)((smem + 1024) * per_sm * 100 / (228 * 1024)) + 1;
-        if (pct > 100) pct = 100;
-        CU(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
-    }
-    if (ctx->pool_carveout > 0) CU(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, ctx->pool_carveout));
-    long long grid = (long long)ctx->sm_count * per_sm, want = (nitems + 128 * K - 1) / (128 * K);
+    long long grid = (long long)ctx->sm_count * per_sm, want = (nitems + kPoolSlots - 1) / kPoolSlots;
     if (want < grid) grid = want ? want : 1;
-    const long long slots = grid * 4 * 32 * K;
+    const long long slots = grid * kPoolSlots;
     // a ray's stack holds at most one 16-byte entry per branch on a root-to-leaf path; the stacks of a warp's slots are
     // interleaved entry by entry, so the few entries in use of all resident slots share cache lines and stay in L2
     int depth = (int)ctx->tree_height;
@@ -515,7 +500,7 @@ static int pool_step(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, i
     // d_gpath holds two entries per slot, so its capacity tells the slot capacity; it is emptied first, so that after a
     // failed allocation the next call allocates all three again
     if (slots > (long long)ctx->d_gpath.cap / 2 || slots * depth > (long long)ctx->d_gstack.cap) {
-        const long long cap = (long long)ctx->sm_count * 16 * 4 * 32 * K > slots ? (long long)ctx->sm_count * 16 * 4 * 32 * K : slots;
+        const long long cap = (long long)ctx->sm_count * 16 * kPoolSlots > slots ? (long long)ctx->sm_count * 16 * kPoolSlots : slots;
         ctx->d_gpath.reset(0);
         CU(ctx->d_gstack.reset(cap * depth));
         CU(ctx->d_gpm.reset(cap * SQT_MAX_DEPTH));
@@ -526,18 +511,10 @@ static int pool_step(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, i
     CU(cudaGetLastError());
     return SQT_OK;
 }
-template <bool COUNT, bool LENS>
-static int pool_step_k(sqt_ctx *ctx, const RenderParams &d, const RoundInfo &rd, int round, long long nitems, bool launch) {
-    switch (ctx->pool_k) {
-    case 1: return pool_step<COUNT, 1, LENS>(ctx, d, rd, round, nitems, launch);
-    case 2: return pool_step<COUNT, 2, LENS>(ctx, d, rd, round, nitems, launch);
-    default: return pool_step<COUNT, 4, LENS>(ctx, d, rd, round, nitems, launch);
-    }
-}
 // the pool kernel of a frame: instrumented or not, lens frame (the sample's own primary ray) or pinhole
 static int pool_step_d(sqt_ctx *ctx, bool count, const RenderParams &d, const RoundInfo &rd, int round, long long nitems, bool launch) {
-    if (d.lens) return count ? pool_step_k<true, true>(ctx, d, rd, round, nitems, launch) : pool_step_k<false, true>(ctx, d, rd, round, nitems, launch);
-    return count ? pool_step_k<true, false>(ctx, d, rd, round, nitems, launch) : pool_step_k<false, false>(ctx, d, rd, round, nitems, launch);
+    if (d.lens) return count ? pool_step<true, true>(ctx, d, rd, round, nitems, launch) : pool_step<false, true>(ctx, d, rd, round, nitems, launch);
+    return count ? pool_step<true, false>(ctx, d, rd, round, nitems, launch) : pool_step<false, false>(ctx, d, rd, round, nitems, launch);
 }
 static float ev_ms(cudaEvent_t a, cudaEvent_t b) { float ms = 0; cudaEventElapsedTime(&ms, a, b); return ms; }
 
@@ -633,12 +610,8 @@ static int prepare_render(sqt_ctx *ctx, const RenderParams &d, bool count, bool 
     if ((pl.k1 - pl.k0 + S - 1) / S > 256) return fail(ctx, SQT_E_UNSUPPORTED, "more than 256 sample rounds (raise SQT_SBUF_MB)");
     pl.sbytes = pl.nwork * (long long)S * 12ll;
     CU(ctx->d_sbuf.ensure((pl.sbytes > 0 ? pl.sbytes : 12) / sizeof(float)));
-    if (ctx->pool_k > 0) {
-        RoundInfo none = {};
-        rc = pool_step_d(ctx, count, d, none, 0, pl.nwork << pl.log2_s, false);
-        if (rc) return rc;
-    }
-    return SQT_OK;
+    RoundInfo none = {};
+    return pool_step_d(ctx, count, d, none, 0, pl.nwork << pl.log2_s, false);
 }
 
 // Multi-rank contexts: all ranks learn whether every rank got through check_params + prepare_render, with a one-word
@@ -721,7 +694,6 @@ static int enqueue_start(sqt_ctx *ctx, const RenderParams &d, bool count, const 
 // counter per round, numbered from 0 in every call), then add in sample order -- onto the sums alone (m2 == nullptr) or
 // the sums and the second moments.  nwork, log2_s: the plan's, or an adaptive frame's active slots (sqt_render_advance).
 static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, long long nwork, int log2_s, int ka, int kb, float *m2, uint32_t &nl) {
-    int rc = SQT_OK;
     cudaStream_t st = ctx->stream;
     if (d.mode == 1) {
         if (count) k_raycast<true><<<persistent_grid(ctx, k_raycast<true>, nwork), 128, 0, st>>>(ctx->sc, d, ctx->d_accum, ctx->d_stats, ctx->tune);
@@ -741,14 +713,9 @@ static int enqueue_rounds(sqt_ctx *ctx, const RenderParams &d, bool count, long 
     for (int k = ka; k < kb; k += S, ++round) {
         rd.k0 = k; rd.k1 = k + S < kb ? k + S : kb;
         CU(cudaMemsetAsync(ctx->d_sbuf, 0, (size_t)(nwork * (long long)(rd.k1 - rd.k0) * 12ll), st));
-        if (ctx->pool_k > 0) {
-            rc = pool_step_d(ctx, count, d, rd, round, nwork << rd.log2_s, true);
-            if (rc) return rc;
-        } else if (d.lens && count) k_paths<true, true><<<persistent_grid(ctx, k_paths<true, true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
-        else if (d.lens) k_paths<false, true><<<persistent_grid(ctx, k_paths<false, true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
-        else if (count) k_paths<true><<<persistent_grid(ctx, k_paths<true>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
-        else k_paths<false><<<persistent_grid(ctx, k_paths<false>, nwork << rd.log2_s), 128, 0, st>>>(ctx->sc, d, rd, round, ctx->d_stats, ctx->tune);
-        CU(cudaGetLastError()); nl++;
+        const int rc = pool_step_d(ctx, count, d, rd, round, nwork << rd.log2_s, true);
+        if (rc) return rc;
+        nl++;
         if (m2) k_accumulate_m2<<<agrid > 0 ? agrid : 1, 256, 0, st>>>(d, rd, ctx->d_accum, m2, ctx->d_stats);
         else k_accumulate<<<agrid > 0 ? agrid : 1, 256, 0, st>>>(d, rd, ctx->d_accum, ctx->d_stats);
         CU(cudaGetLastError()); nl++;

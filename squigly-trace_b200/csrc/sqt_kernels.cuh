@@ -3,9 +3,8 @@
 //   k_intersect_batch  : one lane per ray, grid-stride; batched Scene.intersect (Geometry.hs:64 / BIH.hs:101)
 //   k_primary          : one lane per pixel; makeRay (Lib.hs:107-114) + closest hit, cached per pixel
 //   k_lens_list        : the start of a lens frame: every owned pixel onto the pixel list (no primary pass)
-//   k_paths_pool       : the integrator: every warp owns a pool of 32*K rays in shared memory, keeps them in three
-//                        queues by the kind of step they need and serves one queue per round with all lanes (default)
-//   k_paths            : the integrator with one ray per lane and warp-synchronous phases (SQT_POOL=0)
+//   k_paths_pool       : the integrator: every warp owns a pool of 64 rays in shared memory, keeps them in queues by
+//                        the kind of step they need and serves one queue per round with all lanes
 //   k_accumulate       : adds a round's samples to the per-pixel sums in sample order (Lib.hs:88)
 //   k_accumulate_m2    : the same plus the per-pixel second moment (progressive frames)
 //   k_frame_noise_part, k_frame_noise : deterministic fp64 noise estimate of a progressive frame
@@ -19,7 +18,6 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cooperative_groups.h>
-#include <type_traits>
 
 #include "sqt_denoise.cuh"
 
@@ -131,9 +129,6 @@ __device__ __forceinline__ void leaf_pairs(const SceneView &sc, TravLane &L, Cou
 // (one Moller-Trumbore test).  The votes force the 32 lanes back together at every phase boundary; an ordinary
 // per-lane loop nest compiles to code where the lanes drift apart through the data-dependent traversal and
 // never reconverge (measured: 2.4 of 32 lanes active, profiles/r01_k_paths_v0_divergent.txt).
-template <class P, class = void> struct has_warp_regen : std::false_type {};
-template <class P> struct has_warp_regen<P, std::void_t<decltype(P::kWarpRegen)>> : std::true_type {};
-
 template <bool COUNT, class Policy>
 __device__ __forceinline__ void warp_loop(const SceneView &sc, Policy &pol, Counters *cn, const Tune tn) {
     const unsigned FULL = 0xffffffffu;
@@ -155,8 +150,7 @@ __device__ __forceinline__ void warp_loop(const SceneView &sc, Policy &pol, Coun
         const unsigned m_done = __ballot_sync(FULL, L.state == ST_DONE);
         const unsigned m_busy = __ballot_sync(FULL, L.state == ST_DESC || L.state == ST_RET || L.state == ST_LEAF || L.state == ST_ENTER);
         if (m_done != 0u && (__popc(m_done) >= tn.c_min || m_busy == 0u)) {
-            if constexpr (has_warp_regen<Policy>::value) pol.template regen_warp<COUNT>(sc, L, cn, L.state == ST_DONE);
-            else { if (L.state == ST_DONE) pol.template regen<COUNT>(sc, L, cn); }
+            if (L.state == ST_DONE) pol.template regen<COUNT>(sc, L, cn);
             __syncwarp(FULL);
         } else if (m_busy == 0u) break;                       // every lane is ST_EXIT
         // ---- traversal steps (stack pops + one branch visit) while more than a_leave lanes want one; then every
@@ -255,24 +249,9 @@ struct DeviceFetch {
     }
 };
 
-#ifndef SQT_WL_MIN_BLOCKS
-#define SQT_WL_MIN_BLOCKS 6
-#endif
-// One round of samples (sqt_paths.cuh): persistent lanes pull (pixel, sample) items from the round's counter.
-template <bool COUNT, bool LENS = false>
-__global__ void __launch_bounds__(128, SQT_WL_MIN_BLOCKS) k_paths(SceneView sc, RenderParams p, RoundInfo rd, int round, DeviceStats *ds, Tune tn) {
-    Counters cn = {};
-    PathStats st = {0, 0, 0};
-    if (rd.pixel_list) rd.n_slots = (long long)ds->n_hit;
-    DeviceFetch fetch = {&ds->work_next[round], rd.n_slots << rd.log2_s};
-    uint16_t pm[SQT_MAX_DEPTH];
-    PathPolicy<DeviceFetch, LENS> pol(p, rd, fetch, st, pm);
-    warp_loop<COUNT>(sc, pol, &cn, tn);
-    flush_stats(ds, st, cn, COUNT);
-}
-
 // ------------------------------------------------------------------------------ ray pools
-// k_paths_pool: the same per-ray logic as k_paths, scheduled differently.  Every warp owns a POOL of P = 32*K rays whose
+// k_paths_pool: one round of samples (sqt_paths.cuh), whose (pixel, sample) items are pulled from the round's counter and
+// traced with the per-ray unit steps of sqt_core.cuh.  Every warp owns a POOL of P = kPoolRays rays whose
 // state lives in shared memory (structure of arrays, 16 words per ray; traversal stacks, per-path material lists and the
 // integrator state of a slot in global memory, one region per pool slot).  A ray waits in one of four queues (byte rings of
 // slot ids in shared memory, heads and fills packed in two warp-uniform registers; a served ray is appended with one MATCH + one
@@ -291,9 +270,6 @@ __global__ void __launch_bounds__(128, SQT_WL_MIN_BLOCKS) k_paths(SceneView sc, 
 // Each round the warp serves the longest queue with up to 32 lanes.  With one ray per lane at most ~10 of 32 lanes share a
 // step kind at any time (tests/sched_sim.py); regrouping rays lifts that limit.  Scheduling never changes a result: every
 // ray runs the same unit steps of sqt_core.cuh in the same order (test_every_path_kernel_scheduler_is_bit_exact).
-#ifndef SQT_POOL_MIN_BLOCKS
-#define SQT_POOL_MIN_BLOCKS 8
-#endif
 // The pool is read and written by 32-bit shared-memory address.  A generic pointer into shared memory makes the compiler rebuild
 // the shared window base (S2UR SR_CgaCtaId, UMOV, ULEA, LEA) wherever it is short of registers -- inside the branch visit, in
 // every chunk of the leaf phase -- and that sequence sits in front of the LDS it feeds.  The base is taken once, passed through a
@@ -331,17 +307,25 @@ enum { PF_OX = 0, PF_OY, PF_OZ, PF_DX, PF_DY, PF_DZ, PF_DFX, PF_DFY, PF_DFZ, PF_
        PF_FLAGS, PF_WORDS };
 enum { KT = 0, KL = 1, KR = 2, KS = 3, KNONE = 4 };
 
-template <bool COUNT, int K, bool LENS = false>
-__global__ void __launch_bounds__(128, SQT_POOL_MIN_BLOCKS) k_paths_pool(SceneView sc, RenderParams p, RoundInfo rd, int round, DeviceStats *ds, PoolTune tn,
+// The pool of a CTA of 4 warps (128 lanes).  Dynamic shared memory: the kPoolSlots x PF_WORDS pool, then the scratch of
+// each warp (the four queue rings, 64 survivors, 32 + 32 bytes and 32 words of the leaf round).
+constexpr int kPoolRays = 64;                    // rays per warp (a power of two, at most 128: the queue fills are bytes)
+constexpr int kPoolSlots = 4 * kPoolRays;        // pool slots of the CTA
+constexpr int kPoolAuxWords = 4 * kPoolRays / 4 + 64 + 8 + 8 + 32;
+constexpr size_t kPoolSmemBytes = sizeof(uint32_t) * (kPoolSlots * PF_WORDS + 4 * kPoolAuxWords);
+constexpr int kPoolMinBlocks = 8;                // resident CTAs per SM: at most 64 registers per lane
+
+template <bool COUNT, bool LENS>
+__global__ void __launch_bounds__(128, kPoolMinBlocks) k_paths_pool(SceneView sc, RenderParams p, RoundInfo rd, int round, DeviceStats *ds, PoolTune tn,
                                                     float4 *__restrict__ gstack, uint16_t *__restrict__ gpm, uint4 *__restrict__ gpath, int stack_depth, int pm_stride) {
     extern __shared__ uint32_t pool_smem[];
-    constexpr int P = 32 * K;                     // rays per warp (a power of two)
-    constexpr int PT = 4 * P;                     // pool slots of the CTA: slot g = warp * P + s, and g is what the queues hold,
-                                                  // so the hot accesses index CTA-wide arrays by a value the lane already has
-                                                  // (one uniform base, see lds32)
+    constexpr int P = kPoolRays;
+    constexpr int PT = kPoolSlots;                // slot g = warp * P + s, and g is what the queues hold, so the hot accesses
+                                                  // index CTA-wide arrays by a value the lane already has (one uniform base,
+                                                  // see lds32)
     // per-warp scratch, kept small on purpose: 8 CTAs x (pool + scratch + 1 KB) must stay within the 164 KB shared-memory
     // carve-out, the next one (196 KB) would leave 32 KB instead of 64 KB of L1 for triangles, nodes and stacks
-    constexpr int AUX_WORDS = 4 * P / 4 + 64 + 8 + 8 + 32;
+    constexpr int AUX_WORDS = kPoolAuxWords;
     const unsigned FULL = 0xffffffffu;
     // (the warp index comes out of a REDUX, i.e. in a uniform register: the per-warp scratch addresses derived from it are then
     //  uniform too and are not rebuilt from SR_TID in every loop that is short of registers)
@@ -363,7 +347,7 @@ __global__ void __launch_bounds__(128, SQT_POOL_MIN_BLOCKS) k_paths_pool(SceneVi
     if (rd.pixel_list) rd.n_slots = (long long)ds->n_hit;
     DeviceFetch fetch = {&ds->work_next[round], rd.n_slots << rd.log2_s};
 #pragma unroll
-    for (int k = 0; k < K; ++k) {
+    for (int k = 0; k < P / 32; ++k) {
         const int slot = wbase + lane + 32 * k;
         PW(PF_FLAGS, slot) = (uint32_t)ST_DONE << 4;
         PW(PF_CTRI, slot) = 0xffffffffu;
@@ -376,7 +360,7 @@ __global__ void __launch_bounds__(128, SQT_POOL_MIN_BLOCKS) k_paths_pool(SceneVi
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(lt_mask));
     asm("mov.u32 %0, %%lanemask_le;" : "=r"(le_mask));
     // queue state, warp-uniform, one byte per kind: ring head (< P) and fill (<= P <= 128)
-    unsigned q_head = 0u, q_cnt = (unsigned)P << (8 * KR);     // (P = 128 fills its byte exactly: the top byte, KS, never holds more than P)
+    unsigned q_head = 0u, q_cnt = (unsigned)P << (8 * KR);
     unsigned long long dbg_rounds[3] = {0, 0, 0}, dbg_sel[3] = {0, 0, 0}, dbg_desc[8] = {}, dbg_ret[8] = {}, dbg_leaf[4] = {};
     for (;;) {
         // ---- pick the longest queue (regeneration only in batches, or when nothing else can run)

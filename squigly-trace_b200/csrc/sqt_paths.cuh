@@ -6,10 +6,11 @@
 //                        then put the lane's next ray into L.r and start it -- or set ST_EXIT when the lane
 //                        has no more work.
 //
-// The kernels in sqt_kernels.cuh run one warp-synchronous loop around these: regen for lanes that are done,
-// traversal steps for lanes that are descending/returning, triangle steps for lanes inside a leaf
-// (sqt_core.cuh).  Lanes are independent, so any schedule yields the same per-lane results; tests/emu runs
-// each lane to completion on the host with the same functions.
+// k_intersect_batch, k_primary and k_raycast (sqt_kernels.cuh) run one warp-synchronous loop around these: regen for
+// lanes that are done, traversal steps for lanes that are descending/returning, triangle tests for lanes inside a leaf
+// (sqt_core.cuh).  The integrator kernel, k_paths_pool, keeps its rays in shared-memory pools and regenerates them with
+// path_regen_warp.  Rays are independent, so any schedule yields the same per-ray results; tests/emu runs each lane to
+// completion on the host with the same functions (run_lane), the integrator as PathPolicy.
 //
 // Integrator layout: the work item is one SAMPLE of one pixel; a frame is rendered in rounds of S samples per pixel
 // whose radiances go to a sample buffer and are then added to the per-pixel sums strictly in sample order
@@ -242,6 +243,7 @@ __device__ __forceinline__ void path_regen_warp(const SceneView &sc, const Rende
 }
 #endif
 
+// The integrator as one lane's policy (run_lane in the host build, the reference schedule of k_paths_pool).
 // LENS: a frame with a lens set (sqt_set_lens) -- a compile-time choice, so that the pinhole kernels stay as they are
 template <class Fetch, bool LENS = false>
 struct PathPolicy {
@@ -255,13 +257,6 @@ struct PathPolicy {
         : p(p_), rd(rd_), fetch(f_), st(st_), pm(pm_) { path_ray_init(q); }
     template <bool COUNT>
     SQT_HD void regen(const SceneView &sc, TravLane &L, Counters *cn) { path_regen<COUNT, LENS>(sc, p, rd, fetch, st, q, pm, L, cn); }
-#if defined(__CUDACC__)
-    static constexpr bool kWarpRegen = true;
-    template <bool COUNT>
-    __device__ __forceinline__ void regen_warp(const SceneView &sc, TravLane &L, Counters *cn, bool mine) {
-        path_regen_warp<COUNT, LENS>(sc, p, rd, fetch, st, q, pm, L, cn, mine);
-    }
-#endif
 };
 
 // avg-in-order part of renderPixel (Lib.hs:87-88): add the round's samples of one slot to the pixel's running sum,

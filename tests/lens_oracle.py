@@ -94,7 +94,7 @@ def prefix_window(scene, cam12, params, lens, pix0, pix1, k_end):
 
 
 class EmuLens:
-    """Host build of the kernels' lens frames (same source as k_paths / k_paths_pool with LENS)."""
+    """Host build of the kernels' lens frames (the integrator source of k_paths_pool with LENS)."""
 
     def __init__(self, host_scene):
         L = _lib("libemu_lens.so")

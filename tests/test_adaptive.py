@@ -1,6 +1,6 @@
 """Adaptive frames on the B200 (include/sqt.h: sqt_render_retire): zero tolerances change nothing, every pixel is the exact
 n_p-sample prefix of the full frame, each call retires exactly the pixels the formula picks, results do not depend on the
-scheduler or the sample-buffer budget, work counts follow the active set, the noise estimate uses per-pixel counts, the
+sample-buffer budget, work counts follow the active set, the noise estimate uses per-pixel counts, the
 session rules hold, config 2 at full size, and the CLI."""
 import ctypes as C
 import os
@@ -53,15 +53,14 @@ def final(ctx, p):
     return rgb8, acc, ctx.download_moments(p.rows, p.cols), ctx.download_sample_counts(p.rows, p.cols)
 
 
-@pytest.mark.parametrize("pool", ["0", "1", "2", "4"])
-def test_zero_tolerances_change_nothing_and_results_do_not_depend_on_the_schedule(host_scene, camera, monkeypatch, pool):
+def test_zero_tolerances_change_nothing_and_results_do_not_depend_on_the_round_width(host_scene, camera, monkeypatch):
     """Zero tolerances retire nothing: the frame is sqt_render's bit for bit.  With a tolerance, the same call sequence gives
-    the same sums, moments, counts and RGB8 under every scheduler and sample-buffer budget."""
+    the same sums, moments, counts and RGB8 under every sample-buffer budget (samples per round)."""
     W, H, spp = 160, 120, 16
     p = pysqt.make_params(W, H, spp, max_depth=5, seed=9)
     results = []
     for sbuf in (None, "1"):
-        env = dict(SQT_POOL=pool) if sbuf is None else dict(SQT_POOL=pool, SQT_SBUF_MB=sbuf)
+        env = {} if sbuf is None else dict(SQT_SBUF_MB=sbuf)
         ctx = ctx_with(monkeypatch, host_scene, **env)
         ref = ctx.render(camera, p)
         outs, acts = adaptive_run(ctx, camera, p, [3, 5, 8], 0.0, 0.0, 2)
@@ -69,11 +68,11 @@ def test_zero_tolerances_change_nothing_and_results_do_not_depend_on_the_schedul
         assert acts == [hits] * 3
         rgb8, acc, _, counts = final(ctx, p)
         assert (counts == spp).all()
-        assert np.array_equal(bits(acc), bits(ref["accum"])) and np.array_equal(rgb8, ref["rgb8"]), (pool, sbuf)
+        assert np.array_equal(bits(acc), bits(ref["accum"])) and np.array_equal(rgb8, ref["rgb8"]), sbuf
         adaptive_run(ctx, camera, p, [2, 2, 1, 3, 8], 0.05, 0.0, 2)
         results.append(final(ctx, p))
         ctx.close()
-    # the reference for every pool value: the default scheduler at the default budget
+    # the reference: a fresh context at the default budget
     ctx = ctx_with(monkeypatch, host_scene)
     adaptive_run(ctx, camera, p, [2, 2, 1, 3, 8], 0.05, 0.0, 2)
     want = final(ctx, p)
@@ -81,7 +80,7 @@ def test_zero_tolerances_change_nothing_and_results_do_not_depend_on_the_schedul
     assert 0 < (want[3] < spp).sum() < H * W
     for got in results:
         for g, w in zip(got, want):
-            assert np.array_equal(g.view(np.uint8), w.view(np.uint8)), pool
+            assert np.array_equal(g.view(np.uint8), w.view(np.uint8))
 
 
 def _sphere_scene(host_scene):

@@ -39,12 +39,11 @@ def host_denoise(ctx, hs, p, levels, k):
     return mean, rgb8, s1, counts, feats
 
 
-@pytest.mark.parametrize("pool", ["0", "2"])
 @pytest.mark.parametrize("adaptive", [False, True])
-def test_device_matches_host_build(host_scene, camera, monkeypatch, pool, adaptive):
+def test_device_matches_host_build(host_scene, camera, monkeypatch, adaptive):
     """Levels 1, 3 and 5: the denoised mean bits equal the host build's, the RGB8 is the tone map of that mean; levels = 0
     is the preview's mean and RGB8; mirror pixels (material 5 of scene.obj) pass through bit for bit."""
-    ctx = ctx_with(monkeypatch, host_scene, SQT_POOL=pool)
+    ctx = ctx_with(monkeypatch, host_scene)
     p = pysqt.make_params(160, 120, 16, max_depth=8, seed=5)
     ctx.render_begin(camera, p)
     ctx.render_advance(6)

@@ -276,7 +276,7 @@ def test_resident_then_download_equals_render(gpu_ctx, host_scene, camera):
     st = gpu_ctx.render_resident(camera, p)
     rgb8, accum = gpu_ctx.download(p.rows, p.cols)
     assert np.array_equal(a["rgb8"], rgb8) and np.array_equal(bits(a["accum"]), bits(accum))
-    # k_primary + one (k_paths, k_accumulate) pair per sample round + k_tonemap
+    # k_primary + one (k_paths_pool, k_accumulate) pair per sample round + k_tonemap
     assert st["rays_traced"] == a["stats"]["rays_traced"] and st["kernel_launches"] == 4
 
 
@@ -297,11 +297,9 @@ def test_many_sample_rounds_are_bit_identical(host_scene, camera, monkeypatch):
     assert np.array_equal(bits(a["accum"]), bits(b["accum"])) and np.array_equal(a["rgb8"], b["rgb8"])
 
 
-@pytest.mark.parametrize("pool", ["0", "1", "2", "4"])
-def test_every_path_kernel_scheduler_is_bit_exact(host_scene, oracle_scene, camera, monkeypatch, pool):
-    """SQT_POOL selects how rays are scheduled onto lanes (0: one ray per lane, warp-synchronous phases; K: ray pools of
-    32*K rays per warp in shared memory).  Scheduling must never change a result."""
-    monkeypatch.setenv("SQT_POOL", pool)
+def test_every_path_kernel_scheduler_is_bit_exact(host_scene, oracle_scene, camera):
+    """The path kernel schedules rays onto lanes from pools of 64 rays per warp in shared memory; the oracle traces one
+    path after the other.  Scheduling must never change a result."""
     ctx = pysqt.Context(0)
     ctx.upload(host_scene)
     for w, h, spp, depth, flags in [(96, 64, 8, 8, 0), (64, 48, 5, 3, pysqt.SQT_F_NO_PRIMARY_REUSE | pysqt.SQT_F_NO_EARLY_TERMINATION),
@@ -339,15 +337,14 @@ def test_baseline_config2_at_full_size(gpu_ctx, host_scene, oracle_scene, camera
     assert np.array_equal(out["rgb8"], O.tone_map(acc, spp, trig=1))
 
 
-def test_schedulers_and_culling_agree_at_full_size(host_scene, camera, monkeypatch):
-    """The bench frame (1920x1080, depth 8) at 32 spp -- 170 M rays -- rendered four ways: ray pools (default), one ray per
-    lane, ray pools without the leaf culling, and ray pools without primary reuse / early termination.  All four
-    accumulation buffers must be bit-identical, and the last one must trace strictly more rays."""
+def test_schedulers_and_culling_agree_at_full_size(host_scene, camera):
+    """The bench frame (1920x1080, depth 8) at 32 spp -- 170 M rays -- rendered three ways: default, without the leaf
+    culling, and without primary reuse / early termination.  All three accumulation buffers must be bit-identical, and
+    the last one must trace strictly more rays."""
     p = pysqt.make_params(1920, 1080, 32, max_depth=8, seed=21)
     results = {}
-    for name, pool, cull, flags in [("pool", "2", True, 0), ("lane", "0", True, 0), ("pool-nocull", "2", False, 0),
-                                    ("pool-reference-work", "2", True, pysqt.SQT_F_NO_PRIMARY_REUSE | pysqt.SQT_F_NO_EARLY_TERMINATION)]:
-        monkeypatch.setenv("SQT_POOL", pool)
+    for name, cull, flags in [("pool", True, 0), ("pool-nocull", False, 0),
+                              ("pool-reference-work", True, pysqt.SQT_F_NO_PRIMARY_REUSE | pysqt.SQT_F_NO_EARLY_TERMINATION)]:
         ctx = pysqt.Context(0)
         ctx.upload(host_scene)
         ctx.set_leaf_cull(cull)
@@ -359,7 +356,7 @@ def test_schedulers_and_culling_agree_at_full_size(host_scene, camera, monkeypat
     for name, (acc, st) in results.items():
         assert np.array_equal(bits(acc), bits(base)), name
         assert st["samples"] == 1920 * 1080 * 32
-    assert results["pool"][1]["rays_traced"] == results["lane"][1]["rays_traced"] == results["pool-nocull"][1]["rays_traced"]
+    assert results["pool"][1]["rays_traced"] == results["pool-nocull"][1]["rays_traced"]
     assert results["pool-reference-work"][1]["rays_traced"] > results["pool"][1]["rays_traced"]
 
 

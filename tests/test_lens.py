@@ -1,5 +1,5 @@
 """Camera sampling on the B200 (include/sqt.h, sqt_set_lens): lens frames equal the oracle bit for bit under every
-scheduler; a pinhole lens (aperture 0, no jitter) gives the plain frame; progressive and adaptive lens frames are exact
+sample-buffer budget; a pinhole lens (aperture 0, no jitter) gives the plain frame; progressive and adaptive lens frames are exact
 prefixes; the error rules; and the optics -- anti-aliased edges converge to the pixel's analytic coverage and a thin lens
 blurs an edge by the analytic disk."""
 import os
@@ -35,12 +35,11 @@ def _sphere_oracle():
     return osc, spheres
 
 
-@pytest.mark.parametrize("pool", ["0", "1", "2", "4"])
-def test_lens_frames_match_oracle(host_scene, oracle_scene, camera, monkeypatch, pool):
+def test_lens_frames_match_oracle(host_scene, oracle_scene, camera, monkeypatch):
     W, H, spp, depth = 64, 48, 8, 5
     osc_s, spheres = _sphere_oracle()
     for sbuf in (None, "1"):
-        env = dict(SQT_POOL=pool) if sbuf is None else dict(SQT_POOL=pool, SQT_SBUF_MB=sbuf)
+        env = {} if sbuf is None else dict(SQT_SBUF_MB=sbuf)
         ctx = ctx_with(monkeypatch, host_scene, **env)
         for name, lens in LENSES.items():
             ctx.set_lens(*lens)
@@ -50,8 +49,8 @@ def test_lens_frames_match_oracle(host_scene, oracle_scene, camera, monkeypatch,
             for cull in (True, False):
                 ctx.set_leaf_cull(cull)
                 out = ctx.render(camera, p)
-                assert np.array_equal(bits(out["accum"]), bits(ref["accum"])), (pool, sbuf, name, cull)
-                assert np.array_equal(out["rgb8"], ref["rgb8"]), (pool, sbuf, name, cull)
+                assert np.array_equal(bits(out["accum"]), bits(ref["accum"])), (sbuf, name, cull)
+                assert np.array_equal(out["rgb8"], ref["rgb8"]), (sbuf, name, cull)
                 st = out["stats"]
                 assert st["samples"] == W * H * spp and st["rays_reference"] == st["rays_traced"]
             ctx.set_leaf_cull(True)
@@ -60,7 +59,7 @@ def test_lens_frames_match_oracle(host_scene, oracle_scene, camera, monkeypatch,
         ctx.set_lens(*lens)
         out = ctx.render(camera, pysqt.make_params(W, H, spp, max_depth=depth, seed=13))
         ref = LO.render(osc_s, camera, O.make_params(W, H, spp, max_depth=depth, seed=13, trig=1), lens)
-        assert np.array_equal(bits(out["accum"]), bits(ref["accum"])), (pool, sbuf, "spheres")
+        assert np.array_equal(bits(out["accum"]), bits(ref["accum"])), (sbuf, "spheres")
         ctx.close()
 
 

@@ -38,20 +38,19 @@ def run_chunks(ctx, cam, p, chunks):
     return outs
 
 
-@pytest.mark.parametrize("pool", ["0", "1", "2", "4"])
-def test_chunked_final_frame_equals_one_shot(host_scene, camera, monkeypatch, pool):
+def test_chunked_final_frame_equals_one_shot(host_scene, camera, monkeypatch):
     W, H, spp = 160, 120, 16
     p = pysqt.make_params(W, H, spp, max_depth=5, seed=9)
     for sbuf in (None, "1"):          # 1 MB: 4 samples per round, so chunks of 6 and 7 straddle round boundaries
-        env = dict(SQT_POOL=pool) if sbuf is None else dict(SQT_POOL=pool, SQT_SBUF_MB=sbuf)
+        env = {} if sbuf is None else dict(SQT_SBUF_MB=sbuf)
         ctx = ctx_with(monkeypatch, host_scene, **env)
         ref = ctx.render(camera, p)
         chunkings = [[spp], [1] * spp, [3, 5, spp - 8]] + ([[3, 6, 7], [5, 100]] if sbuf else [])
         for chunks in chunkings:
             run_chunks(ctx, camera, p, chunks)
             rgb8, acc = ctx.download(H, W)
-            assert np.array_equal(bits(acc), bits(ref["accum"])), (pool, sbuf, chunks)
-            assert np.array_equal(rgb8, ref["rgb8"]), (pool, sbuf, chunks)
+            assert np.array_equal(bits(acc), bits(ref["accum"])), (sbuf, chunks)
+            assert np.array_equal(rgb8, ref["rgb8"]), (sbuf, chunks)
         ctx.close()
 
 

@@ -1,4 +1,4 @@
-"""Small render used under ncu: data/scene.obj at a reduced frame so that one k_paths launch replays quickly.
+"""Small render used under ncu: data/scene.obj at a reduced frame so that one k_paths_pool launch replays quickly.
 usage: python tools/prof_render.py [W H SPP DEPTH]"""
 import os
 import sys
